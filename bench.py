@@ -4,15 +4,17 @@
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference --gpus N --steps K ...  # CPU arm: the oracle port on all host cores
     python bench.py --config car_gtg_pb | haul_push_point | haul_push_car   # the other BASELINE configs
+    python bench.py --steps K --dump-outputs DIR   # also write the last timed step's outputs to DIR/<name>.npy
 
 Workload (default, N=1): BASELINE.json configs[1] -- point go_to_goal, 65,536 environments per GPU, pseudo-lidar
 observation + hazard/vase/pillar cost, i.i.d. U(-1,1) actions, action_noise 0.01 (reference default), 1000-step
 episodes (tests/test_safety_gym.py:78).  A "step" = one env.step over the whole batch.
 
 The cost of a step depends on the episode phase (no robot is near anything right after a reset; ~10 % of them
-are late in the episode), so the K timed steps are STRATIFIED over one whole episode: S = min(K, 20) windows
-of K/S consecutive steps centred at (i + 1/2) * 1000 / S, the steps between the windows run untimed with the
-same kernels (fast-forward), and the episode's reset (layout rejection sampling, timed with events) is added
+are late in the episode), so the K timed steps are STRATIFIED over whole episodes: ceil(K / 1000) episodes share
+them as evenly as possible, and an episode that times Ke of them does so in S = min(Ke, 20) windows of Ke/S
+consecutive steps centred at (i + 1/2) * 1000 / S; the steps between the windows run untimed with the same kernels
+(fast-forward), and the episode's reset (layout rejection sampling, timed with events) is added
 amortised as t_reset / 1000 per step.  `value` is therefore the whole-episode average the reference arm
 measures by running whole episodes.
 
@@ -23,6 +25,11 @@ e2e          : same metric and strata through sag_step_host (C ABI, pinned HOST 
 roofline     : algorithmic bytes per env-step (SURVEY 8d) x envs / average step duration vs the measured HBM
                copy bandwidth.
 cpu_baseline : the oracle port (oracle/sag_oracle.c, pthreads) on the box's host cores, whole episodes.
+
+--dump-outputs DIR writes what the last timed step returned (rank 0's environments): obs.npy (float32 [n, obs_dim]),
+reward.npy (float64 [n]), cost.npy and done.npy (float32 [n]).  Seeds are fixed, so two builds run with the same
+arguments can be compared output for output.  Above DUMP_BYTES a fixed, seeded sample of rows is written instead,
+with their environment indices in env_index.npy.
 """
 import argparse
 import ctypes as C
@@ -35,9 +42,11 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the benchmark leaves the source tree as it found it (it may be read-only)
 
 EPISODE = 1000  # tests/test_safety_gym.py:78
 UNIT = "env-steps/s"
+DUMP_BYTES = 60_000_000  # data budget of --dump-outputs (all files together stay under 64 MB)
 # SURVEY.md 8(d): algorithmic bytes per env-step of the fused step
 CONFIGS = {
     "point_gtg": dict(robot="point", tasks=["go_to_goal"], envs=65536, b_alg=2582, metric="env_steps_per_sec_point_go_to_goal",
@@ -75,6 +84,23 @@ def strata(K):
         a = min(a, EPISODE - (K - used) - ln)
         out.append((a, ln))
     return out
+
+
+def dump_outputs(path, obs, rew, cost, done):
+    """DIR/<name>.npy of one step's outputs (device tensors, row = environment), float32 / float64, within DUMP_BYTES"""
+    import numpy as np
+    import torch
+    arrays = {"obs": obs.float(), "reward": rew.double(), "cost": cost.float(), "done": done.float()}
+    n = obs.shape[0]
+    row_bytes = sum(a.element_size() * a[0].numel() for a in arrays.values())
+    os.makedirs(path, exist_ok=True)
+    if n * row_bytes > DUMP_BYTES:
+        rows = np.sort(np.random.RandomState(0).choice(n, DUMP_BYTES // (row_bytes + 8), replace=False))
+        idx = torch.from_numpy(rows).to(obs.device)
+        arrays = {k: a[idx] for k, a in arrays.items()}
+        np.save(os.path.join(path, "env_index.npy"), rows.astype(np.float64))
+    for k, a in arrays.items():
+        np.save(os.path.join(path, k + ".npy"), a.cpu().numpy())
 
 
 class ClockSampler:
@@ -176,7 +202,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--stagger", action="store_true", help="extra: episodes staggered over all 1000 phases (auto-reset every step)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write obs / reward / cost / done of the last timed step to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs dumps the CUDA path's outputs (--impl b200)")
     cfg = CONFIGS[args.config]
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -207,8 +239,9 @@ def main():
     n = args.envs_per_gpu or cfg["envs"]
     K, W = args.steps, max(3, args.warmup)
     n_ep = (K + EPISODE - 1) // EPISODE
-    windows = strata((K + n_ep - 1) // n_ep)
-    K = n_ep * sum(ln for _, ln in windows)
+    # episode i times K*(i+1)//n_ep - K*i//n_ep steps: exactly K timed steps in all
+    ep_windows = [strata(K * (i + 1) // n_ep - K * i // n_ep) for i in range(n_ep)]
+    windows = ep_windows[0]
     task_objs = [TASKS[t]() for t in cfg["tasks"]]
 
     def make_env():
@@ -255,9 +288,10 @@ def main():
     t_wall0 = time.perf_counter()
     l0 = launches_now(h)
     timed_launches = 0
-    for _ep in range(n_ep):
+    last_out = None
+    for ep_win in ep_windows:
         t = 0
-        for (a, ln) in windows + [(EPISODE, 0)]:
+        for (a, ln) in ep_win + [(EPISODE, 0)]:
             if a > t:  # fast-forward (warm L2, timed as one block for the value_l2_warm extra)
                 e0, e1 = ev(), ev()
                 e0.record(stream)
@@ -275,6 +309,8 @@ def main():
                 e1.record(stream)
                 timed_launches += launches_now(h) - lc
                 timed.append((a + k, e0, e1))
+                if args.dump_outputs and len(timed) == K:  # the last timed step: keep its outputs before the reset
+                    last_out = [x.clone() for x in (obs, rew, cost, done)]
             t = a + ln
         e0, e1 = ev(), ev()
         flush.zero_()
@@ -305,12 +341,15 @@ def main():
     value_warm = world * n * ff_steps / (ff_ms * 1e-3) if ff_steps else None
     win_ms = []
     i = 0
-    for _ep in range(n_ep):
-        for (a, ln) in windows:
+    for ep_win in ep_windows:
+        for (a, ln) in ep_win:
             if ln:
                 w = [m for _, m in ms[i:i + ln]]
                 win_ms.append({"phase": a, "steps": ln, "ms_per_step": float(sum(w) / ln)})
             i += ln
+    if last_out is not None and rank == 0:
+        dump_outputs(args.dump_outputs, *last_out)
+        del last_out
 
     # ---- optional extra: episodes staggered over all 1000 phases (every step some envs auto-reset)
     stagger = None
@@ -340,7 +379,7 @@ def main():
                    "note": "warm L2, step + auto-reset of the ~n/1000 envs that expire every step"}
         env_s.close()
 
-    # ---- end to end through the C ABI with pinned host buffers, on a second handle, same strata
+    # ---- end to end through the C ABI with pinned host buffers, on a second handle: one episode, the first episode's strata
     e2e = None
     if not args.no_e2e:
         env2 = make_env()
@@ -416,7 +455,8 @@ def main():
                "host_ceiling_note": ("ceiling = sum of the ranks' copy rates while ALL ranks copy one step's outputs device -> pinned host back to "
                                      "back; with several ranks the e2e steps are not in lockstep, so their copies contend less than the probe's"),
                "binding": binding,
-               "api": "sag_step_host (C ABI; one pinned output block, a single D2H copy per step), same strata as `value`"}
+               "api": "sag_step_host (C ABI; one pinned output block, a single D2H copy per step); one episode, timed in the windows "
+                      "of `value`'s first episode"}
         L.L.sag_host_free(C.c_void_p(ptrs[0].value))
         env2.close()
 
@@ -444,8 +484,10 @@ def main():
             "dtype": "f64", "data": "synthetic",
             "config": {"workload": cfg["workload"], "envs_per_gpu": n, "global_envs": world * n, "parallelism": f"env-shard x{world}",
                        "l2": "flushed before every timed step (256 MiB memset outside the event pair)", "action_noise": 0.01,
-                       "episode_phase": (f"stratified over whole {EPISODE}-step episodes: {len(windows)} windows of "
-                                         f"{windows[0][1]}..{windows[-1][1]} steps at phases {[a for a, _ in windows]}, untimed fast-forward "
+                       "episode_phase": (f"stratified over {n_ep} whole {EPISODE}-step episode(s), {K} timed steps: per episode "
+                                         f"{len(windows)} windows of {min(ln for w in ep_windows for _, ln in w)}.."
+                                         f"{max(ln for w in ep_windows for _, ln in w)} steps at phases "
+                                         f"{[[a for a, _ in w] for w in ep_windows]} (one list per episode), untimed fast-forward "
                                          f"in between, + reset {reset_ms:.3f} ms amortised / {EPISODE}")},
             "ms_per_step_windows": win_ms, "reset_ms": reset_ms,
             "value_l2_warm": value_warm,

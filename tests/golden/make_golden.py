@@ -1,9 +1,9 @@
 #!/usr/bin/env python
 """Generate golden vectors by running the REFERENCE'S OWN PYTHON CODE.
 
-Run in the build container only (needs /root/reference):
+Run where the reference's sources are, SAG_REFERENCE naming their directory:
 
-    python tests/golden/make_golden.py
+    SAG_REFERENCE=<reference checkout> python tests/golden/make_golden.py
 
 The reference (lasgroup/safe-adaptation-gym) is pure Python on top of dm_control/MuJoCo, gym and
 xmltodict, none of which is installable here.  Everything the reference computes itself -- lidar
@@ -11,7 +11,7 @@ xmltodict, none of which is installable here.  Everything the reference computes
 task's reward / goal logic (tasks/*.py), layout rejection sampling (world.py:172-217,
 utils.py:28-70), yaw draw order (world.py:108-137), the step loop (safe_adaptation_gym.py:56-83) and
 the benchmark task sampler (benchmark/__init__.py, task_sampler.py) -- is executed UNMODIFIED from
-/root/reference.  Only the third-party layer is replaced:
+the directory SAG_REFERENCE names.  Only the third-party layer is replaced:
 
   * ``dm_control`` / ``gym`` / ``xmltodict`` are stub modules;
   * ``MujocoBridge`` (mujoco_bridge.py, the reference's one and only door to the simulator) is
@@ -34,7 +34,7 @@ import numpy as np
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
-REF = "/root/reference"
+REF = os.environ.get("SAG_REFERENCE", "")
 sys.path.insert(0, ROOT)
 
 import oracle as O  # noqa: E402
@@ -90,6 +90,9 @@ class _Elem:
 
 
 def install_stubs():
+    if not os.path.isdir(REF):  # otherwise "" would put the working directory on sys.path and the import fail late
+        sys.exit("SAG_REFERENCE must name the directory of the reference's sources (safe_adaptation_gym/ inside it); "
+                 "got %r" % REF)
     dm = types.ModuleType("dm_control")
     mujoco = types.ModuleType("dm_control.mujoco")
     def _quat2mat(m, q):  # mujoco.mju_quat2Mat [EXT]: row-major 3x3 of a unit quaternion (w, x, y, z)
