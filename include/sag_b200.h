@@ -85,7 +85,7 @@ void sag_default_config(SagConfig* cfg); /* world.py:17-34 defaults */
 
 /* lifetime.  replaces SafeAdaptationGym.__init__ + MujocoBridge.__init__ (safe_adaptation_gym.py:30-54).
  * Side effect on the device: cudaLimitStackSize is raised (never lowered) to the largest stack frame of the library's kernels
- * (about 1.75 KB), so that the driver does not re-size its local-memory pool -- a device-wide stall of tens to hundreds of
+ * (about 1.7 KB), so that the driver does not re-size its local-memory pool -- a device-wide stall of tens to hundreds of
  * milliseconds -- whenever an observation / auto-reset kernel follows a run of step kernels. */
 int sag_create(const SagConfig* cfg, int device, void** handle);
 int sag_destroy(void* handle);

@@ -32,11 +32,6 @@ extern long* sag_prof_ptr;  // tests/hostemu instrumentation: per-env work count
 #define SAG_PROF_MAX(e, i, n) do { } while (0)
 #endif
 
-// Phase alignment of the cooperative kernel's warps is on by default (coop_align below; -DSAG_COOP_NOALIGN for A/B runs)
-#if !defined(SAG_COOP_NOALIGN) && !defined(SAG_COOP_ALIGN)
-#define SAG_COOP_ALIGN 1
-#endif
-
 // SAG_TIMING (tuning builds only): the cooperative kernel accumulates clock64() intervals per section into D.dbg[16]
 #if defined(SAG_TIMING) && defined(__CUDA_ARCH__)
 #define SAG_CLK_DECL long long clk_ = clock64()
@@ -706,14 +701,15 @@ struct Scratch {
 #endif
 };
 
-// env_step / end_of_step modes: full scalar path (one thread = one environment, contact solver included), quiet-only
-// (no contact code), warp-cooperative (one warp = one environment, device only)
-// kStepNear: the contact-free path, with (run-time flag `pretest`) the exact overlap / tendon pre-test in front of every
-// substep and of the final forward pass -- for environments that have something within reach but (usually) touch
-// nothing; the step is abandoned (return 1, nothing written that the full path would not write identically) as soon as
-// a robot geom overlaps an object or the tendon is taut, and the environment is handed to the contact path.  With
-// pretest == false it is the quiet path.
-constexpr int kStepFull = 0, kStepQuiet = 1, kStepCoop = 2, kStepNear = 3;
+// env_step / end_of_step modes:
+// kStepFull: the full scalar path (one thread = one environment, contact solver included);
+// kStepCoop: warp-cooperative (one warp = one environment, device only);
+// kStepNear: the contact-free path (no contact code), with (run-time flag `pretest`) the exact overlap / tendon pre-test in
+// front of every substep and of the final forward pass -- for environments that have something within reach but
+// (usually) touch nothing; the step is abandoned (return 1, nothing written that the full path would not write
+// identically) as soon as a robot geom overlaps an object or the tendon is taut, and the environment is handed to the
+// contact path.  With pretest == false it is the quiet path.
+constexpr int kStepFull = 0, kStepCoop = 1, kStepNear = 2;
 
 struct Ctx {  // per-thread view of one environment
   const Dev& D;
@@ -846,17 +842,14 @@ SAG_HD void car_free_solve(const CarRobot& R, double sn, double cs, const PtCons
 // code at the same time and share its instruction-cache lines instead of evicting each other's.  A warp without an
 // environment executes the same number of barriers (coop_idle_step).
 __device__ __forceinline__ void coop_align() {
-#if defined(SAG_COOP_ALIGN) && defined(__CUDA_ARCH__)
+#if defined(__CUDA_ARCH__)
   asm volatile("bar.sync 0;" ::: "memory");
 #endif
 }
-#ifndef SAG_ALIGN_EVERY
-#define SAG_ALIGN_EVERY 1   // a barrier in front of every SAG_ALIGN_EVERY-th trip of the pass loop
-#endif
 template <class RB>
 __device__ __forceinline__ void coop_idle_step() {
 #pragma unroll 1
-  for (int k = 0; k <= RB::kNsub; ++k) if (k % SAG_ALIGN_EVERY == 0) coop_align();
+  for (int k = 0; k <= RB::kNsub; ++k) coop_align();
 }
 
 #endif
@@ -2011,7 +2004,7 @@ template <int Mode, class RB>
 SAG_HD void end_of_step(unsigned wmask, Scratch* S, const SolveConsts& Q, const Ctx& C, const RB& R, TaskState& T, const Rng& rng, const PtConst& K,
                         unsigned mov, bool phys_err, const double* qacc_err, bool with_reward, float* obs_s, int ostride, EndOut& O,
                         const Phys* Pfwd = nullptr, unsigned cand = 0xffffffffu, const double* mocap = nullptr) {
-  constexpr bool QuietOnly = Mode == kStepQuiet || Mode == kStepNear, Coop = Mode == kStepCoop, Near = Mode == kStepNear;
+  constexpr bool Coop = Mode == kStepCoop, Near = Mode == kStepNear;
   const Dev& D = C.D;
   const int e = C.e;
   O.bail = 0;
@@ -2091,7 +2084,7 @@ SAG_HD void end_of_step(unsigned wmask, Scratch* S, const SolveConsts& Q, const 
   if (Pfwd) {  // cooperative kernel: the forward pass has been evaluated as the last trip of env_step's pass loop
     P = *Pfwd;
   } else {
-  if (!QuietOnly && !skip_forward) {  // (a quiet step ends with positive clearance: no contact is possible)
+  if (!Near && !skip_forward) {  // (a quiet step ends with positive clearance: no contact is possible)
     const bool always = RB::kGremlins && C.sp.ng > 0;  // a welded gremlin is a constraint row in every pass
     const bool near_ = !(clear > 0.0 && mov == 0) || always;
     if constexpr (Coop) {
@@ -2112,7 +2105,7 @@ SAG_HD void end_of_step(unsigned wmask, Scratch* S, const SolveConsts& Q, const 
     SAG_CLK(7);
     if (need) contact_pass<RB, true>(C, R, sn, cs, K, fs, mov, false, 0.0, *S, Q, P, mocap);
     SAG_CLK_RESET;
-  } else if (!QuietOnly) {
+  } else if (!Near) {
     warp_contact_pass(wmask, need, C, R, sn, cs, K, fs, mov, false, 0.0, S, Q, P, mocap);
   }
   }
@@ -2215,7 +2208,7 @@ SAG_HD bool env_is_quiet(double clear, const RB& R) { return clear > R.travel_bo
 template <int Mode, class RB>
 SAG_HD int env_step(unsigned wmask, Scratch* S, const Dev& D, int e, float a0, float a1, float* obs_s, int ostride, double* reward2,
                      unsigned char* cost, unsigned char* done, bool pretest = true) {
-  constexpr bool QuietOnly = Mode == kStepQuiet || Mode == kStepNear, Coop = Mode == kStepCoop, Near = Mode == kStepNear;
+  constexpr bool Coop = Mode == kStepCoop, Near = Mode == kStepNear;
   SAG_CLK_DECL;
   Ctx C = {D, e, spec_for(D, D.task[e], RB::kGremlins), Slots(), D.task[e], global_objects(D, e)};
   C.L = make_slots(C.sp);
@@ -2288,7 +2281,7 @@ SAG_HD int env_step(unsigned wmask, Scratch* S, const Dev& D, int e, float a0, f
   // contact detection; the bound on the hinge point's travel is conservative (DESIGN.md 5).
   unsigned char fl = D.flags[e];
   int err = (fl & F_PHYS_ERROR) ? 1 : 0;  // a physics error is sticky until the env is reset
-  const bool quiet = QuietOnly ? true : env_is_quiet(D.clear[e], R);  // (gremlin environments keep clear = -1)
+  const bool quiet = Near ? true : env_is_quiet(D.clear[e], R);  // (gremlin environments keep clear = -1)
   (void)Coop;
   SAG_PROF(e, 7, quiet ? 0 : 1);
   double qacc_err[3] = {0.0, 0.0, 0.0};
@@ -2302,7 +2295,7 @@ SAG_HD int env_step(unsigned wmask, Scratch* S, const Dev& D, int e, float a0, f
 #pragma unroll 1
   for (int k = 0; k < kTrips; ++k) {
 #if defined(__CUDA_ARCH__)
-    if constexpr (Coop) { if (k % SAG_ALIGN_EVERY == 0) coop_align(); }
+    if constexpr (Coop) coop_align();
 #endif
     const bool fwd = Coop && k == RB::kNsub;
     if (fwd && err) { Pfwd.qacc[0] = qacc_err[0]; Pfwd.qacc[1] = qacc_err[1]; Pfwd.qacc[2] = qacc_err[2]; break; }  // :73-75, no forward()
@@ -2312,7 +2305,7 @@ SAG_HD int env_step(unsigned wmask, Scratch* S, const Dev& D, int e, float a0, f
     R.smooth(sn, cs, fs);
     bool need = false;
     bool taut = false;
-    if (tendon_task && (fwd || (Near ? pretest : (Mode != kStepQuiet && !quiet)))) {
+    if (tendon_task && (fwd || (Near ? pretest : !quiet))) {
       double tdx, tdy, tlen, tdist;
       taut = tendon_taut(C, R, tdx, tdy, tlen, tdist);
     }
@@ -2320,7 +2313,7 @@ SAG_HD int env_step(unsigned wmask, Scratch* S, const Dev& D, int e, float a0, f
 #if defined(__CUDA_ARCH__)
       need = (fwd || !quiet) && (gremlins || mov != 0 || taut || robot_overlaps_any_coop(C, R, sn, cs));
 #endif
-    } else if (!QuietOnly) {
+    } else if (!Near) {
       need = !quiet && (gremlins || mov != 0 || taut || robot_overlaps_any(C, R, sn, cs));
     }
     if constexpr (Near) {
@@ -2336,7 +2329,7 @@ SAG_HD int env_step(unsigned wmask, Scratch* S, const Dev& D, int e, float a0, f
         subq[0] = F.qacc[0]; subq[1] = F.qacc[1]; subq[2] = F.qacc[2];
       }
     }
-    if (!QuietOnly) {
+    if (!Near) {
       Phys P;
       P.fc[0] = fc[0]; P.fc[1] = fc[1]; P.fc[2] = fc[2]; P.wtau[0] = wtau[0]; P.wtau[1] = wtau[1];
       P.mov = mov; P.err = 0;
@@ -2480,6 +2473,45 @@ SAG_HD double slot_keepout(const Dev& D, const TaskSpec& sp, int kind) {
        : kind == K_PILLAR ? D.k_pillar : kind == K_GOAL ? kGoalKeepout : kind == K_BUTTON ? kButtonsKeepout : sp.box_keepout;
 }
 
+// The fresh episode after placement, shared by env_reset and env_reset_coop: the robot at rest at (x, y, yaw) and the
+// task state of environment C.e.  For a fresh Task instance (new_task) it makes the per-instance draws of World.__init__
+// (world.py:72-78): Task.ctrl_scale, standard Cauchy per actuator (task.py:85-89), and Task.constraint_bound
+// (task.py:91-94), on Philox stream 3, Cauchy by inversion; and it resets the task state (catch_goal.py:12-18,
+// press_buttons.py:20-24, collect.py:15-16).  Returns the Task instance's ctrl scales and bound: the fresh draws, which
+// the caller stores, when new_task, the stored ones otherwise.
+struct TaskDraws { double cscale[2], bound; };
+template <class RB>
+SAG_HD TaskDraws fresh_episode(const Dev& D, const Ctx& C, const Rng& rng, double x, double y, double yaw, bool new_task,
+                               RB& R, TaskState& T) {
+  const int e = C.e;
+  R.q[0] = x; R.q[1] = y; R.q[2] = yaw; R.v[0] = R.v[1] = R.v[2] = 0.0; R.ctrl[0] = R.ctrl[1] = 0.0;
+  if constexpr (RB::kKind == 1) { R.wheel[0] = R.wheel[1] = 0.0; R.cq[0] = 1.0; R.cq[1] = R.cq[2] = R.cq[3] = 0.0; }
+  R.damp_xy = C.sp.damp_xy; R.gear_x = C.sp.gear_x;
+  load_task_state(D, e, T);
+  TaskDraws d;
+  if (new_task) {
+    double u[2];
+    rng.pair(3u, 0u, u[0], u[1]);
+    for (int k = 0; k < 2; ++k) {
+      double tn, tc;
+      sag_sincos(kPi * (u[k] - 0.5), &tn, &tc);
+      d.cscale[k] = (tn / tc) * D.ctrl_range_scale + 1.0;
+    }
+    rng.pair(3u, 1u, u[0], u[1]);
+    d.bound = D.random_bound ? 0.0 + (D.max_bound - 0.0) * u[0] : D.max_bound;
+  } else {
+    d.cscale[0] = D.cscale0[e]; d.cscale[1] = D.cscale1[e]; d.bound = D.bound[e];
+  }
+  if (D.ctrl_range_scale != 0.0) {  // MuJoCo clamps the zero control of a fresh physics into an inverted range, too
+    R.ctrl[0] = clampd(0.0, -1.0 * d.cscale[0], 1.0 * d.cscale[0]); R.ctrl[1] = clampd(0.0, -1.0 * d.cscale[1], 1.0 * d.cscale[1]);
+  }
+  if (new_task) {
+    T.cgcur = 1.0; T.cgnext = 0.2; T.cgtimer = 0; T.bstate = 1; T.btimer = kButtonDelay; T.gbtn = 0;
+    T.amask = C.task == T_COLLECT ? (1 << C.L.nbtn) - 1 : 0; T.cgox = T.cgoy = 0.0; T.last0 = T.last1 = 0.0;
+  }
+  return d;
+}
+
 template <class RB>
 SAG_HD_NOINLINE void env_reset(const Dev& D, int e, uint32_t episode, bool new_task) {
   Ctx C = {D, e, spec_for(D, D.task[e], RB::kGremlins), Slots(), D.task[e], global_objects(D, e)};
@@ -2547,34 +2579,9 @@ SAG_HD_NOINLINE void env_reset(const Dev& D, int e, uint32_t episode, bool new_t
   if (C.sp.kind == 2 && C.sp.box_kind == K_BOX) { rng.pair(0u, ctr++, u1, u2); C.O.yaw[oix(C, C.L.box)] = kTwoPi * u1; }
   if (C.sp.kind == 1) for (int i = 0; i < C.L.nbtn; ++i) { rng.pair(0u, ctr++, u1, u2); C.O.yaw[oix(C, C.L.btn0 + i)] = kTwoPi * u1; }
   RB R;
-  R.q[0] = rxy[0]; R.q[1] = rxy[1]; R.q[2] = robot_rot; R.v[0] = R.v[1] = R.v[2] = 0.0; R.ctrl[0] = R.ctrl[1] = 0.0;
-  if constexpr (RB::kKind == 1) { R.wheel[0] = R.wheel[1] = 0.0; R.cq[0] = 1.0; R.cq[1] = R.cq[2] = R.cq[3] = 0.0; }
-  R.damp_xy = C.sp.damp_xy; R.gear_x = C.sp.gear_x;
   TaskState T;
-  load_task_state(D, e, T);
-  if (new_task) {
-    // World.__init__ (world.py:72-78): Task.ctrl_scale (standard Cauchy per actuator, task.py:85-89) and
-    // Task.constraint_bound (task.py:91-94) are drawn once per Task instance.  Philox stream 3, Cauchy by inversion.
-    double u[2];
-    rng.pair(3u, 0u, u[0], u[1]);
-    double sc[2];
-    for (int k = 0; k < 2; ++k) {
-      double tn, tc;
-      sag_sincos(kPi * (u[k] - 0.5), &tn, &tc);
-      sc[k] = (tn / tc) * D.ctrl_range_scale + 1.0;
-    }
-    D.cscale0[e] = sc[0]; D.cscale1[e] = sc[1];
-    rng.pair(3u, 1u, u[0], u[1]);
-    D.bound[e] = D.random_bound ? 0.0 + (D.max_bound - 0.0) * u[0] : D.max_bound;
-  }
-  if (D.ctrl_range_scale != 0.0) {  // MuJoCo clamps the zero control of a fresh physics into an inverted range, too
-    const double sc0 = D.cscale0[e], sc1 = D.cscale1[e];
-    R.ctrl[0] = clampd(0.0, -1.0 * sc0, 1.0 * sc0); R.ctrl[1] = clampd(0.0, -1.0 * sc1, 1.0 * sc1);
-  }
-  if (new_task) {  // fresh Task instance (catch_goal.py:12-18, press_buttons.py:20-24, collect.py:15-16)
-    T.cgcur = 1.0; T.cgnext = 0.2; T.cgtimer = 0; T.bstate = 1; T.btimer = kButtonDelay; T.gbtn = 0;
-    T.amask = C.task == T_COLLECT ? (1 << C.L.nbtn) - 1 : 0; T.cgox = T.cgoy = 0.0; T.last0 = T.last1 = 0.0;
-  }
+  const TaskDraws td = fresh_episode(D, C, rng, rxy[0], rxy[1], robot_rot, new_task, R, T);
+  if (new_task) { D.cscale0[e] = td.cscale[0]; D.cscale1[e] = td.cscale[1]; D.bound[e] = td.bound; }
   if (ok && task_reset(C, rng, 0u, ctr, R, T)) fl |= F_RESAMPLE_FAILED;
   T.ctr = 0;
   store_robot(D, e, R);
@@ -2797,30 +2804,9 @@ __device__ __noinline__ void env_reset_coop(const Dev& D, int e, uint32_t episod
   // from here on the object positions are read from the warp's shared memory (task_reset, clearance)
   C.O.x = px; C.O.y = py; C.O.stride = 1;
   RB R;
-  R.q[0] = rxy[0]; R.q[1] = rxy[1]; R.q[2] = robot_rot; R.v[0] = R.v[1] = R.v[2] = 0.0; R.ctrl[0] = R.ctrl[1] = 0.0;
-  if constexpr (RB::kKind == 1) { R.wheel[0] = R.wheel[1] = 0.0; R.cq[0] = 1.0; R.cq[1] = R.cq[2] = R.cq[3] = 0.0; }
-  R.damp_xy = C.sp.damp_xy; R.gear_x = C.sp.gear_x;
   TaskState T;
-  load_task_state(D, e, T);
-  double sc0 = D.cscale0[e], sc1 = D.cscale1[e];
-  if (new_task) {  // World.__init__ (world.py:72-78): per-Task-instance draws, Philox stream 3 (see env_reset)
-    double u[2];
-    rng.pair(3u, 0u, u[0], u[1]);
-    double sc[2];
-    for (int k = 0; k < 2; ++k) {
-      double tn, tc;
-      sag_sincos(kPi * (u[k] - 0.5), &tn, &tc);
-      sc[k] = (tn / tc) * D.ctrl_range_scale + 1.0;
-    }
-    sc0 = sc[0]; sc1 = sc[1];
-    rng.pair(3u, 1u, u[0], u[1]);
-    if (lane == 0) { D.cscale0[e] = sc0; D.cscale1[e] = sc1; D.bound[e] = D.random_bound ? 0.0 + (D.max_bound - 0.0) * u[0] : D.max_bound; }
-  }
-  if (D.ctrl_range_scale != 0.0) { R.ctrl[0] = clampd(0.0, -1.0 * sc0, 1.0 * sc0); R.ctrl[1] = clampd(0.0, -1.0 * sc1, 1.0 * sc1); }
-  if (new_task) {
-    T.cgcur = 1.0; T.cgnext = 0.2; T.cgtimer = 0; T.bstate = 1; T.btimer = kButtonDelay; T.gbtn = 0;
-    T.amask = C.task == T_COLLECT ? (1 << C.L.nbtn) - 1 : 0; T.cgox = T.cgoy = 0.0; T.last0 = T.last1 = 0.0;
-  }
+  const TaskDraws td = fresh_episode(D, C, rng, rxy[0], rxy[1], robot_rot, new_task, R, T);
+  if (new_task && lane == 0) { D.cscale0[e] = td.cscale[0]; D.cscale1[e] = td.cscale[1]; D.bound[e] = td.bound; }
   if (ok && task_reset_coop(C, rng, 0u, ctr, R, T)) fl |= F_RESAMPLE_FAILED;
   T.ctr = 0;
   __syncwarp();

@@ -79,8 +79,7 @@ struct Handle {
   uint8_t *cost_d, *done_d;
   cudaStream_t own_stream;
   cudaStream_t copy_stream;          // host-buffer API: bulk device-to-host copies that overlap the busy kernel
-  cudaEvent_t ev_quiet, ev_copied;
-  cudaEvent_t ev_chunk[8];
+  cudaEvent_t ev_free, ev_copied;   // host-buffer API: batch kernel done, bulk copy done
   unsigned long long launches;  // kernels launched on behalf of this handle (sag_launch_count)
   int busy_grid;  // CTAs of k_step_coop: resident CTAs per SM x SMs
 };
@@ -143,15 +142,13 @@ __device__ __forceinline__ void write_rows(const float* tile, int tstride, float
 template <class RB>
 __global__ void __launch_bounds__(kBS, RB::kKind == 1 ? 2 : 4) k_step_free(Dev D, const float* __restrict__ act, float* __restrict__ obs,
                                                     double* __restrict__ reward, double* __restrict__ reward2,
-                                                    uint8_t* __restrict__ cost, uint8_t* __restrict__ done, int e_first) {
-  // environments [e_first, e_first + gridDim.x * kBS) of the batch (the host-buffer step launches the batch in chunks
-  // so that the device-to-host copy of a chunk's observations runs under the next chunk's kernel); e_first % kBS == 0
+                                                    uint8_t* __restrict__ cost, uint8_t* __restrict__ done) {
   constexpr int kObs = RB::kObsDim;
   extern __shared__ __align__(16) unsigned char smem_raw[];
   float* tile = reinterpret_cast<float*>(smem_raw);  // [kObs][kTileStride]
-  const int e = e_first + blockIdx.x * kBS + threadIdx.x;
+  const int e = blockIdx.x * kBS + threadIdx.x;
   const int lane = threadIdx.x & 31;
-  if (e_first == 0 && blockIdx.x == 0 && threadIdx.x < 4) D.counts_next[threadIdx.x] = 0;
+  if (blockIdx.x == 0 && threadIdx.x < 4) D.counts_next[threadIdx.x] = 0;
   bool run = false, pretest = false;
   if (e < D.n) {
     RB R;
@@ -185,7 +182,7 @@ __global__ void __launch_bounds__(kBS, RB::kKind == 1 ? 2 : 4) k_step_free(Dev D
   // all kBS rows of the CTA in one coalesced sweep.  The columns of the work-list environments hold stale shared memory:
   // their rows are rewritten by the cooperative kernel, which always runs after this one on the same stream.
   __syncthreads();
-  write_tile4<kObs>(tile, obs, e_first + blockIdx.x * kBS, D.n);
+  write_tile4<kObs>(tile, obs, blockIdx.x * kBS, D.n);
 }
 
 // k_step_coop: the work list with ONE WARP per environment (sag_core.cuh "warp-cooperative variants"): the lanes run the
@@ -193,10 +190,7 @@ __global__ void __launch_bounds__(kBS, RB::kKind == 1 ? 2 : 4) k_step_free(Dev D
 // pre-test, the row set-up and the lidar pass between them.  A contact environment's step is a long dependent chain; what
 // bounds this kernel is that chain's latency, not throughput, so the lanes are spent on shortening it and the register
 // budget (<= 128) on keeping every work-list environment of the step resident at once (16 warps / SM).
-#ifndef SAG_COOP_WARPS
-#define SAG_COOP_WARPS 16
-#endif
-constexpr int kCoopWarps = SAG_COOP_WARPS;  // warps (= environments in flight) per CTA; 16 = one CTA per SM at 128 registers
+constexpr int kCoopWarps = 16;  // warps (= environments in flight) per CTA; 16 = one CTA per SM at 128 registers
 template <class RB>
 struct CoopCfg {
   static constexpr int kObs = RB::kObsDim;
@@ -205,11 +199,8 @@ struct CoopCfg {
   static constexpr size_t kSmemBytes = kPerWarp * kCoopWarps;
 };
 
-#ifndef SAG_COOP_MINBLOCKS
-#define SAG_COOP_MINBLOCKS (16 / SAG_COOP_WARPS)
-#endif
 template <class RB>
-__global__ void __launch_bounds__(32 * kCoopWarps, SAG_COOP_MINBLOCKS) k_step_coop(const __grid_constant__ Dev D, const float* __restrict__ act,
+__global__ void __launch_bounds__(32 * kCoopWarps, 1) k_step_coop(const __grid_constant__ Dev D, const float* __restrict__ act,
                                                               float* __restrict__ obs, double* __restrict__ reward,
                                                               double* __restrict__ reward2, uint8_t* __restrict__ cost,
                                                               uint8_t* __restrict__ done) {
@@ -218,7 +209,7 @@ __global__ void __launch_bounds__(32 * kCoopWarps, SAG_COOP_MINBLOCKS) k_step_co
   unsigned char* mine = smem_raw + (size_t)warp * CoopCfg<RB>::kPerWarp;
   float* tile = reinterpret_cast<float*>(mine);
   Scratch* big = reinterpret_cast<Scratch*>(mine + CoopCfg<RB>::kTileBytes);
-  // launched with programmatic stream serialization where possible (Ops::step_busy): the grid may be resident before the
+  // launched with programmatic stream serialization where possible (Ops::step_coop): the grid may be resident before the
   // preceding kernel has finished; everything that kernel wrote is visible after this call (no-op otherwise)
   cudaGridDependencySynchronize();
   const int count = D.counts[0];
@@ -272,33 +263,6 @@ __global__ void __launch_bounds__(kBS) k_observe(Dev D, float* __restrict__ obs)
   if (e < D.n) env_observe<RB>(wmask, &scratch[threadIdx.x >> 5], D, e, tile + threadIdx.x, kTileStride);
   __syncthreads();
   write_tile<RB::kObsDim>(tile, obs, e0, D.n);
-}
-
-template <class RB>
-__global__ void __launch_bounds__(kBS) k_rollout(Dev D, int k_steps, float* __restrict__ obs, double* __restrict__ reward,
-                                                  uint8_t* __restrict__ cost, uint8_t* __restrict__ done) {
-  extern __shared__ __align__(16) unsigned char smem_raw[];
-  float* tile = reinterpret_cast<float*>(smem_raw);
-  Scratch* scratch = reinterpret_cast<Scratch*>(smem_raw + TileCfg<RB>::kTileBytes);
-  const int e0 = blockIdx.x * kBS, e = e0 + threadIdx.x;
-  const unsigned wmask = __ballot_sync(0xffffffffu, e < D.n);
-  if (e < D.n) {
-    double rew[2] = {0.0, 0.0};
-    unsigned char c = 0, d = 0;
-    Rng rng = {D.seed, D.gid_base + (uint32_t)e, D.episode[e]};
-    uint32_t base = (uint32_t)D.nstep[e];
-    for (int k = 0; k < k_steps; ++k) {
-      double u1, u2;
-      rng.pair(2u, base + (uint32_t)k, u1, u2);
-      env_step<kStepFull, RB>(wmask, &scratch[threadIdx.x >> 5], D, e, (float)(2.0 * u1 - 1.0), (float)(2.0 * u2 - 1.0),
-                              tile + threadIdx.x, kTileStride, rew, &c, &d);
-    }
-    if (reward) reward[e] = rew[0];
-    if (cost) cost[e] = c;
-    if (done) done[e] = d;
-  }
-  __syncthreads();
-  if (obs) write_tile<RB::kObsDim>(tile, obs, e0, D.n);
 }
 
 // synthetic actions of sag_rollout: U(-1, 1) from Philox stream 2, counter = the environment's step count
@@ -541,10 +505,9 @@ struct Ops {
   static cudaError_t setup(Handle* H) {
     cudaError_t ce = cudaFuncSetAttribute(k_observe<RB>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TileCfg<RB>::kSmemBytes);
     if (ce == cudaSuccess) ce = cudaFuncSetAttribute(k_reset<RB, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ResetCfg<RB>::kSmemBytes);
-    if (ce == cudaSuccess) ce = cudaFuncSetAttribute(k_rollout<RB>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TileCfg<RB>::kSmemBytes);
     if (ce == cudaSuccess) ce = cudaFuncSetAttribute(k_step_coop<RB>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CoopCfg<RB>::kSmemBytes);
     if (ce != cudaSuccess) return ce;
-    // Local memory: the observation / auto-reset / rollout kernels carry the scalar contact path (stack frames of ~1.6 KB
+    // Local memory: the observation and auto-reset kernels carry the scalar contact path (stack frames of ~1.6 KB
     // per thread, above the default 1 KB limit), so the driver would re-size its local-memory pool whenever one of them
     // follows a run of step kernels -- a device-wide stall of tens to hundreds of milliseconds on the first env.reset()
     // after an episode (measured).  Raising the stack limit once to the largest frame keeps the pool at that size.
@@ -553,7 +516,6 @@ struct Ops {
       cudaFuncAttributes fa;
       if (cudaFuncGetAttributes(&fa, k_observe<RB>) == cudaSuccess && fa.localSizeBytes > need) need = fa.localSizeBytes;
       if (cudaFuncGetAttributes(&fa, k_reset<RB, true>) == cudaSuccess && fa.localSizeBytes > need) need = fa.localSizeBytes;
-      if (cudaFuncGetAttributes(&fa, k_rollout<RB>) == cudaSuccess && fa.localSizeBytes > need) need = fa.localSizeBytes;
       need = (need + 255) / 256 * 256;
       size_t cur = 0;
       if (cudaDeviceGetLimit(&cur, cudaLimitStackSize) == cudaSuccess && cur < need) cudaDeviceSetLimit(cudaLimitStackSize, need);
@@ -567,24 +529,16 @@ struct Ops {
   }
   static cudaError_t step(Handle* H, const float* act, float* obs, double* reward, double* reward2, uint8_t* cost, uint8_t* done,
                           cudaStream_t s) {
-    cudaError_t ce = step_quiet(H, act, obs, reward, reward2, cost, done, s);
+    cudaError_t ce = step_free(H, act, obs, reward, reward2, cost, done, s);
     if (ce != cudaSuccess) return ce;
-    return step_busy(H, act, obs, reward, reward2, cost, done, s);
+    return step_coop(H, act, obs, reward, reward2, cost, done, s);
   }
-  static cudaError_t step_quiet(Handle* H, const float* act, float* obs, double* reward, double* reward2, uint8_t* cost,
-                                uint8_t* done, cudaStream_t s) {
-    // two counter sets used alternately: this step's is zero already (cleared by the previous step's quiet kernel, which
+  static cudaError_t step_free(Handle* H, const float* act, float* obs, double* reward, double* reward2, uint8_t* cost,
+                               uint8_t* done, cudaStream_t s) {
+    // two counter sets used alternately: this step's is zero already (cleared by the previous step's batch kernel, which
     // saves a memset node per step); steps of one handle must be stream-ordered
     int* t = H->D.counts; H->D.counts = H->D.counts_next; H->D.counts_next = t;
-    k_step_free<RB><<<grid_for(H->D.n), kBS, TileCfg<RB>::kTileBytes, s>>>(H->D, act, obs, reward, reward2, cost, done, 0);
-    ++H->launches;
-    return cudaGetLastError();
-  }
-  // one chunk [e0, e1) of the batch kernel (e0 a multiple of kBS); the first chunk swaps the work-list counter sets
-  static cudaError_t step_free_range(Handle* H, int e0, int e1, const float* act, float* obs, double* reward, double* reward2,
-                                     uint8_t* cost, uint8_t* done, cudaStream_t s) {
-    if (e0 == 0) { int* t = H->D.counts; H->D.counts = H->D.counts_next; H->D.counts_next = t; }
-    k_step_free<RB><<<grid_for(e1 - e0), kBS, TileCfg<RB>::kTileBytes, s>>>(H->D, act, obs, reward, reward2, cost, done, e0);
+    k_step_free<RB><<<grid_for(H->D.n), kBS, TileCfg<RB>::kTileBytes, s>>>(H->D, act, obs, reward, reward2, cost, done);
     ++H->launches;
     return cudaGetLastError();
   }
@@ -595,7 +549,7 @@ struct Ops {
     ++H->launches;
     return cudaGetLastError();
   }
-  static cudaError_t step_busy(Handle* H, const float* act, float* obs, double* reward, double* reward2, uint8_t* cost, uint8_t* done,
+  static cudaError_t step_coop(Handle* H, const float* act, float* obs, double* reward, double* reward2, uint8_t* cost, uint8_t* done,
                                cudaStream_t s) {
     ++H->launches;
     const int need = (H->D.n + kCoopWarps - 1) / kCoopWarps;
@@ -617,15 +571,9 @@ struct Ops {
     return cudaGetLastError();
   }
   static cudaError_t rollout(Handle* H, int k_steps, float* obs, double* reward, uint8_t* cost, uint8_t* done, cudaStream_t s) {
-    // K x (action kernel + the two step kernels): the same path as sag_step, so a rollout runs at the step's speed (the
-    // single-launch scalar form k_rollout, one thread per environment with the contact solver inline, is 3x slower at
-    // BASELINE batch sizes; SAG_ROLLOUT_FUSED=1 selects it for comparison).  Outputs of the last step are returned.
-    static const bool fused = getenv("SAG_ROLLOUT_FUSED") != nullptr;
-    if (fused) {
-      k_rollout<RB><<<grid_for(H->D.n), kBS, TileCfg<RB>::kSmemBytes, s>>>(H->D, k_steps, obs, reward, cost, done);
-      ++H->launches;
-      return cudaGetLastError();
-    }
+    // K x (action kernel + the two step kernels): the same path as sag_step, so a rollout runs at the step's speed (a
+    // single-launch scalar form, one thread per environment with the contact solver inline, was 3x slower at BASELINE
+    // batch sizes).  Outputs of the last step are returned.
     float* o = obs ? obs : H->obs_d;
     double* r = reward ? reward : H->rew_d;
     uint8_t* c = cost ? cost : H->cost_d;
@@ -669,14 +617,7 @@ extern "C" {
 const char* sag_last_error(void) { return g_err; }
 int sag_abi_version(void) { return SAG_ABI_VERSION; }
 
-void sag_default_config(SagConfig* c) {
-  memset(c, 0, sizeof(*c));
-  c->n_envs = 1; c->robot = SAG_ROBOT_POINT; c->seed = 666;
-  c->placements_margin = 0.0; c->robot_keepout = 0.4;
-  c->hazards_size = 0.2; c->vases_size = 0.1; c->pillars_size = 0.2; c->gremlins_size = 0.1;
-  c->hazards_keepout = 0.18; c->gremlins_keepout = 0.4; c->vases_keepout = 0.15; c->pillars_keepout = 0.3;
-  c->gremlins_travel = 0.35; c->robot_ctrl_range_scale = 0.0; c->action_noise = 0.01; c->max_bound = 25.0;
-}
+void sag_default_config(SagConfig* c) { default_config(c); }
 
 int sag_create(const SagConfig* cfg, int device, void** handle) {
   if (!cfg || !handle) return fail("sag_create: null argument");
@@ -717,9 +658,8 @@ int sag_create(const SagConfig* cfg, int device, void** handle) {
   if (ce == cudaSuccess) { memset(H->err_h, 0, 4 * sizeof(int)); ce = cudaHostGetDevicePointer((void**)&D.errflags, H->err_h, 0); }
   if (ce == cudaSuccess) ce = cudaStreamCreateWithFlags(&H->own_stream, cudaStreamNonBlocking);
   if (ce == cudaSuccess) ce = cudaStreamCreateWithFlags(&H->copy_stream, cudaStreamNonBlocking);
-  if (ce == cudaSuccess) ce = cudaEventCreateWithFlags(&H->ev_quiet, cudaEventDisableTiming);
+  if (ce == cudaSuccess) ce = cudaEventCreateWithFlags(&H->ev_free, cudaEventDisableTiming);
   if (ce == cudaSuccess) ce = cudaEventCreateWithFlags(&H->ev_copied, cudaEventDisableTiming);
-  for (int k = 0; k < 8 && ce == cudaSuccess; ++k) ce = cudaEventCreateWithFlags(&H->ev_chunk[k], cudaEventDisableTiming);
   if (ce != cudaSuccess) { cudaFree(H->slab); delete H; return fail("sag_create: init", ce); }
   *handle = H;
   return 0;
@@ -733,9 +673,8 @@ int sag_destroy(void* handle) {
   if (H->err_h) cudaFreeHost(H->err_h);
   if (H->own_stream) cudaStreamDestroy(H->own_stream);
   if (H->copy_stream) cudaStreamDestroy(H->copy_stream);
-  if (H->ev_quiet) cudaEventDestroy(H->ev_quiet);
+  if (H->ev_free) cudaEventDestroy(H->ev_free);
   if (H->ev_copied) cudaEventDestroy(H->ev_copied);
-  for (int k = 0; k < 8; ++k) if (H->ev_chunk[k]) cudaEventDestroy(H->ev_chunk[k]);
   cudaFree(H->slab);
   delete H;
   return 0;
@@ -928,24 +867,17 @@ int sag_step_host(void* handle, const float* act_h, float* obs_h, double* reward
     // The copy of the observation rows (16 MB: the long pole of the step at PCIe speed) starts when the batch kernel is
     // done and runs under the contact kernel.  (Launching the batch kernel in chunks so that copies could start earlier
     // was measured and lost: the kernel's duration is the latency of one thread's step, not throughput, so every chunk
-    // costs as much as the whole batch -- e2e 1.51e8 -> 1.27e8.  SAG_HOST_CHUNKS re-enables it for experiments.)
+    // costs as much as the whole batch -- e2e 1.51e8 -> 1.27e8.)
     cudaStream_t c = H->copy_stream;
     // (Reading the actions straight from the pinned host buffer in the kernels instead of copying them first: no difference,
     // 1.556e8 either way.  A split copy -- head of the observation rows under the contact kernel, tail + reward / cost / done after it so that
     // the fix-up runs under the tail, split point adapted from the previous step's timings -- was measured and lost by 1-5 %:
     // the contact kernel's duration varies by +-20 us from step to step, and a copy engine that waits costs more than the
     // 27 us fix-up it hides.)
-    static const int env_chunks = getenv("SAG_HOST_CHUNKS") ? atoi(getenv("SAG_HOST_CHUNKS")) : 1;
-    const int nch = (env_chunks >= 1 && env_chunks <= 8 && n >= 8 * 4096) ? env_chunks : 1;
-    const int per = (((int)n + nch - 1) / nch + kBS - 1) / kBS * kBS;
-    for (int k = 0; k < nch; ++k) {
-      const int e0 = k * per, e1 = e0 + per < (int)n ? e0 + per : (int)n;
-      if (e0 >= e1) break;
-      CK(SAG_DISPATCH(H, step_free_range(H, e0, e1, H->act_d, H->obs_d, H->rew_d, nullptr, H->cost_d, H->done_d, s)));
-      CK(cudaEventRecord(H->ev_chunk[k], s));
-      CK(cudaStreamWaitEvent(c, H->ev_chunk[k], 0));
-      CK(cudaMemcpyAsync(obs_h + (size_t)e0 * od, H->obs_d + (size_t)e0 * od, (size_t)(e1 - e0) * od * sizeof(float), cudaMemcpyDeviceToHost, c));
-    }
+    CK(SAG_DISPATCH(H, step_free(H, H->act_d, H->obs_d, H->rew_d, nullptr, H->cost_d, H->done_d, s)));
+    CK(cudaEventRecord(H->ev_free, s));
+    CK(cudaStreamWaitEvent(c, H->ev_free, 0));
+    CK(cudaMemcpyAsync(obs_h, H->obs_d, n * od * sizeof(float), cudaMemcpyDeviceToHost, c));
     bool packed = is_packed_block(obs_h);  // a block from sag_host_alloc_outputs, used as handed out
     packed = packed && (char*)reward_h - (char*)obs_h == (char*)H->rew_d - (char*)H->obs_d &&
              (char*)cost_h - (char*)obs_h == (char*)H->cost_d - (char*)H->obs_d &&
@@ -962,7 +894,7 @@ int sag_step_host(void* handle, const float* act_h, float* obs_h, double* reward
     cudaEventRecord(te[3], c);   // bulk copy done
     cudaEventRecord(te[2], s);   // batch kernel done (the copy stream waited for the same point)
 #endif
-    CK(SAG_DISPATCH(H, step_busy(H, H->act_d, H->obs_d, H->rew_d, nullptr, H->cost_d, H->done_d, s)));
+    CK(SAG_DISPATCH(H, step_coop(H, H->act_d, H->obs_d, H->rew_d, nullptr, H->cost_d, H->done_d, s)));
 #if defined(SAG_E2E_TIMING)
     cudaEventRecord(te[4], s);   // contact kernel done
 #endif

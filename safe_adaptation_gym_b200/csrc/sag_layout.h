@@ -1,12 +1,23 @@
-// sag_layout.h -- host-side carving of the single state slab into the SoA arrays of sag::Dev.
+// sag_layout.h -- host-side carving of the single state slab into the SoA arrays of sag::Dev, and the configuration defaults.
 #pragma once
 #include <stddef.h>
 #include <stdint.h>
+#include <string.h>
 
 #include "../../include/sag_b200.h"
 #include "sag_core.cuh"
 
 namespace sag {
+
+// sag_default_config: World.DEFAULT (world.py:17-34), one environment, the point robot
+inline void default_config(SagConfig* c) {
+  memset(c, 0, sizeof(*c));
+  c->n_envs = 1; c->robot = SAG_ROBOT_POINT; c->seed = 666;
+  c->placements_margin = 0.0; c->robot_keepout = 0.4;
+  c->hazards_size = 0.2; c->vases_size = 0.1; c->pillars_size = 0.2; c->gremlins_size = 0.1;
+  c->hazards_keepout = 0.18; c->gremlins_keepout = 0.4; c->vases_keepout = 0.15; c->pillars_keepout = 0.3;
+  c->gremlins_travel = 0.35; c->robot_ctrl_range_scale = 0.0; c->action_noise = 0.01; c->max_bound = 25.0;
+}
 
 inline size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
 

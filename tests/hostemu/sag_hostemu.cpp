@@ -26,7 +26,6 @@ using namespace sag;
 namespace {
 constexpr int kBS = 128, kTileStride = kBS + 1, kObsMax = SAG_OBS_CAR;
 char g_err[512] = "";
-bool g_force_full = getenv("SAG_HOSTEMU_FULL") != nullptr;  // every environment through the full scalar path
 int fail(const char* w) { snprintf(g_err, sizeof(g_err), "%s", w); return 1; }
 struct Handle {
   Dev D;
@@ -81,7 +80,7 @@ void do_step(Handle* H, const float* act, float* obs, double* reward, double* re
         pretest = !env_is_quiet(D.clear[e], R);
       }
       bool bail = true;
-      if (run && !g_force_full) bail = env_step<kStepNear, RB>(1u, nullptr, D, e, act[2 * e], act[2 * e + 1], tile + t, kTileStride, rew, &c, &d, pretest) != 0;
+      if (run) bail = env_step<kStepNear, RB>(1u, nullptr, D, e, act[2 * e], act[2 * e + 1], tile + t, kTileStride, rew, &c, &d, pretest) != 0;
       if (bail) env_step<kStepFull, RB>(1u, &scratch, D, e, act[2 * e], act[2 * e + 1], tile + t, kTileStride, rew, &c, &d);
       reward[e] = rew[0];
       if (reward2) { reward2[2 * e] = rew[0]; reward2[2 * e + 1] = rew[1]; }
@@ -133,14 +132,7 @@ void do_rollout(Handle* H, int k_steps, float* obs, double* reward, uint8_t* cos
 extern "C" {
 const char* sag_last_error(void) { return g_err; }
 int sag_abi_version(void) { return SAG_ABI_VERSION; }
-void sag_default_config(SagConfig* c) {
-  memset(c, 0, sizeof(*c));
-  c->n_envs = 1; c->robot = SAG_ROBOT_POINT; c->seed = 666;
-  c->placements_margin = 0.0; c->robot_keepout = 0.4;
-  c->hazards_size = 0.2; c->vases_size = 0.1; c->pillars_size = 0.2; c->gremlins_size = 0.1;
-  c->hazards_keepout = 0.18; c->gremlins_keepout = 0.4; c->vases_keepout = 0.15; c->pillars_keepout = 0.3;
-  c->gremlins_travel = 0.35; c->robot_ctrl_range_scale = 0.0; c->action_noise = 0.01; c->max_bound = 25.0;
-}
+void sag_default_config(SagConfig* c) { default_config(c); }
 int sag_create(const SagConfig* cfg, int device, void** handle) {
   (void)device;
   if (!cfg || !handle || cfg->n_envs <= 0) return fail("sag_create: bad argument");
