@@ -15,6 +15,16 @@
  * several devices) may coexist in a process: every entry point switches to the handle's device and restores the
  * caller's.  The *_host entry points are synchronous and ordered after everything issued earlier on the device; the
  * stream entry points are ordered by the caller's stream.
+ *
+ * CUDA graphs.  These stream entry points may be recorded in a CUDA graph (stream capture) and the graph replayed any
+ * number of times: sag_step, sag_reset_obs / sag_reset with a mask or only_flagged != 0, sag_export_outputs,
+ * sag_observe, sag_rollout, sag_read_field / sag_write_field and sag_task_stats.  A replay behaves exactly like issuing
+ * the same calls again: everything the kernels read that can change after sag_create (the work-list counter sets and
+ * the step epoch that selects them, the Philox key, the task ids) lives in the handle's device memory, so sag_seed and
+ * sag_set_tasks issued between replays are seen by the graph.  The *_host entry points, sag_seed, sag_set_tasks_host,
+ * sag_bound_host, sag_create / sag_destroy and sag_probe_d2h synchronise and must not be called while a capture is
+ * open.  sag_launch_count counts host-side enqueues only: replays do not add to it.  Conditions recorded by replayed
+ * kernels are read with sag_error_flags as usual.
  */
 #ifndef SAG_B200_H
 #define SAG_B200_H
@@ -142,7 +152,8 @@ int sag_observe(void* handle, float* obs, void* stream);
 /* same as sag_step with HOST buffers: H2D, kernels, D2H, sync; returns when the outputs are in the host buffers.
  * Page-locked buffers (sag_host_alloc, cudaHostRegister, torch pin_memory) take the overlapped path: the bulk copy runs
  * under the contact kernel and that kernel's rows follow as writes into the mapped buffers.  Steps of one handle must be
- * issued in order (one stream, or externally ordered streams): consecutive steps alternate two work-list counter sets. */
+ * issued in order (one stream, or externally ordered streams): consecutive steps alternate two work-list counter sets,
+ * selected by a step epoch in device memory. */
 int sag_step_host(void* handle, const float* act_h, float* obs_h, double* reward_h, uint8_t* cost_h, uint8_t* done_h);
 int sag_observe_host(void* handle, float* obs_h);
 void* sag_host_alloc(size_t bytes);

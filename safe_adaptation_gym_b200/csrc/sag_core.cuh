@@ -176,7 +176,11 @@ struct Dev {
   double k_hazard, k_vase, k_gremlin, k_pillar;
   double max_bound, ctrl_range_scale;
   int random_bound;
+  // Philox key.  Kernels read it from the slab (*key): sag_seed may change it after kernels have been recorded in a CUDA
+  // graph, and a replayed kernel sees only device memory, not a new by-value argument.  `seed` is the by-value copy
+  // that a host build of this code reads (the host emulation of the tests, which has no slab on a device).
   unsigned long long seed;
+  unsigned long long* key;
   unsigned gid_base;
   int max_layout_draws, max_episode_steps;
   int num_gremlins;        // Task.obstacles[2] of a user-defined task (task.py:70); 0 in every shipped task
@@ -198,8 +202,10 @@ struct Dev {
   int* cgtimer;
   int* movmask;  // bit s: movable object s has a non-zero velocity (derived state, rebuilt by env_observe)
   // work list of the environments with a contact or a moving body in the current step (k_step_free -> k_step_coop)
-  int *worklist, *counts;  // work list segments and their lengths (sag_kernels.cu)
-  int* counts_next;        // the other counter set: zeroed by this step's quiet kernel for the next step
+  int* worklist;
+  int* counts;             // [2][8]: two counter sets used by alternate steps; counts[8 * (*epoch & 1)] is this step's
+  unsigned* epoch;         // [0] step epoch, advanced by the contact kernel's last CTA; [1] CTAs of that kernel that have
+                           // finished (sag_kernels.cu: k_step_free, k_step_coop)
   unsigned long long* dbg; // [16] section clocks of SAG_TIMING builds
   int* errflags;           // [4] sticky error words the host can read without a synchronisation (mapped pinned memory):
                            // [0] a layout / goal could not be sampled (ResamplingError), [1] task id out of range
@@ -237,12 +243,27 @@ SAG_HD void philox4x32_10(uint32_t c0, uint32_t c1, uint32_t c2, uint32_t c3, ui
   }
   out[0] = c0; out[1] = c1; out[2] = c2; out[3] = c3;
 }
+// The key an Rng draws with.  In kernels it is a pointer, loaded at every draw: holding the 64-bit key itself through a
+// step added spills to k_step_free, while the pointer (into the slab, or to a caller's local copy) is an argument the
+// compiler can reload.  A host build holds the key by value (Dev::seed).
+#if defined(__CUDA_ARCH__)
+typedef const unsigned long long* RngKey;
+SAG_HD RngKey rng_key(const Dev& D) { return D.key; }
+SAG_HD RngKey rng_key_of(const unsigned long long& k) { return &k; }
+SAG_HD uint64_t rng_key_value(RngKey k) { return *k; }
+#else
+typedef unsigned long long RngKey;
+SAG_HD RngKey rng_key(const Dev& D) { return D.seed; }
+SAG_HD RngKey rng_key_of(const unsigned long long& k) { return k; }
+SAG_HD uint64_t rng_key_value(RngKey k) { return k; }
+#endif
 struct Rng {
-  uint64_t seed;
+  RngKey seed;
   uint32_t gid, episode;
   SAG_HD void pair(uint32_t stream, uint32_t ctr, double& u1, double& u2) const {
     uint32_t r[4];
-    philox4x32_10(ctr, episode, gid, stream, (uint32_t)seed, (uint32_t)(seed >> 32), r);
+    const uint64_t key = rng_key_value(seed);
+    philox4x32_10(ctr, episode, gid, stream, (uint32_t)key, (uint32_t)(key >> 32), r);
     u1 = ((double)(r[0] >> 5) * 67108864.0 + (double)(r[1] >> 6)) * (1.0 / 9007199254740992.0);
     u2 = ((double)(r[2] >> 5) * 67108864.0 + (double)(r[3] >> 6)) * (1.0 / 9007199254740992.0);
   }
@@ -2230,7 +2251,7 @@ SAG_HD int env_step(unsigned wmask, Scratch* S, const Dev& D, int e, float a0, f
   load_robot(D, e, C.sp, R);
   TaskState T;
   load_task_state(D, e, T);
-  Rng rng = {D.seed, D.gid_base + (uint32_t)e, D.episode[e]};
+  Rng rng = {rng_key(D), D.gid_base + (uint32_t)e, D.episode[e]};
   double time = D.time[e];
   unsigned mov = (unsigned)D.movmask[e];
   const double h = RB::kH;
@@ -2446,7 +2467,7 @@ SAG_HD void env_observe(unsigned wmask, Scratch* S, const Dev& D, int e, float* 
   load_robot(D, e, C.sp, R);
   TaskState T;
   load_task_state(D, e, T);
-  Rng rng = {D.seed, D.gid_base + (uint32_t)e, D.episode[e]};
+  Rng rng = {rng_key(D), D.gid_base + (uint32_t)e, D.episode[e]};
   const PtConst K = R.consts(RB::kH);
   unsigned mov = 0;  // rebuilt from the velocities: state may have been injected
   for (int s = C.L.v0; s < C.L.n; ++s) {
@@ -2516,7 +2537,8 @@ template <class RB>
 SAG_HD_NOINLINE void env_reset(const Dev& D, int e, uint32_t episode, bool new_task) {
   Ctx C = {D, e, spec_for(D, D.task[e], RB::kGremlins), Slots(), D.task[e], global_objects(D, e)};
   C.L = make_slots(C.sp);
-  Rng rng = {D.seed, D.gid_base + (uint32_t)e, episode};
+  const unsigned long long key = rng_key_value(rng_key(D));  // once per layout: the rejection sampler draws in a loop
+  Rng rng = {rng_key_of(key), D.gid_base + (uint32_t)e, episode};
   uint32_t ctr = 0;
   long draws_left = D.max_layout_draws > 0 ? D.max_layout_draws : (1L << 22);
   unsigned char fl = 0;
@@ -2713,7 +2735,8 @@ __device__ __noinline__ void env_reset_coop(const Dev& D, int e, uint32_t episod
   Ctx C = {D, e, spec_for(D, D.task[e], RB::kGremlins), Slots(), D.task[e], global_objects(D, e)};
   C.L = make_slots(C.sp);
   const ObjView G = C.O;
-  Rng rng = {D.seed, D.gid_base + (uint32_t)e, episode};
+  const unsigned long long key = rng_key_value(rng_key(D));  // once per layout: the rejection sampler draws in a loop
+  Rng rng = {rng_key_of(key), D.gid_base + (uint32_t)e, episode};
   uint32_t ctr = 0;
   long draws_left = D.max_layout_draws > 0 ? D.max_layout_draws : (1L << 22);
   unsigned char fl = 0;

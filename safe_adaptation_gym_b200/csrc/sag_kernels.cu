@@ -133,8 +133,12 @@ __device__ __forceinline__ void write_rows(const float* tile, int tstride, float
 // k_step_coop: the work list, ONE WARP per environment (sag_core.cuh "warp-cooperative variants").  Keeping the contact
 //   code out of the batch kernel is what keeps that one at <= 128 registers and free of divergence.
 
-// The work list of a step: D.worklist[0 .. counts[0]); counts[1] = fetch counter of the cooperative kernel.  Two counter
-// sets are used alternately (the other one is cleared by this step's batch kernel for the next step).
+// The work list of a step: D.worklist[0 .. counts[0]).  Two counter sets are used alternately, selected on the device by
+// the step epoch (D.epoch[0], in the slab): a step's batch kernel appends to set epoch & 1 and clears the other set for
+// the next step, and the last CTA of its cooperative kernel to finish advances the epoch.  Once the batch kernel is
+// done the other set is zero, so the kernels after it read the length as the sum of both sets, without the epoch.
+// Nothing the host does between steps selects a set, so a step recorded in a CUDA graph behaves on every replay like a
+// step issued anew, with no memset node per step.
 
 // __launch_bounds__(kBS, 4): 4 CTAs / SM (<= 128 registers) so that the whole 65,536-env point batch is one wave.  The car's
 // contact-free step carries the two wheel-row pairs of its friction solve through ten substeps x ten sweeps: it needs
@@ -148,7 +152,7 @@ __global__ void __launch_bounds__(kBS, RB::kKind == 1 ? 2 : 4) k_step_free(Dev D
   float* tile = reinterpret_cast<float*>(smem_raw);  // [kObs][kTileStride]
   const int e = blockIdx.x * kBS + threadIdx.x;
   const int lane = threadIdx.x & 31;
-  if (blockIdx.x == 0 && threadIdx.x < 4) D.counts_next[threadIdx.x] = 0;
+  if (blockIdx.x == 0 && threadIdx.x < 4) D.counts[8 * ((*D.epoch & 1u) ^ 1u) + threadIdx.x] = 0;
   bool run = false, pretest = false;
   if (e < D.n) {
     RB R;
@@ -175,7 +179,7 @@ __global__ void __launch_bounds__(kBS, RB::kKind == 1 ? 2 : 4) k_step_free(Dev D
   const unsigned m = __ballot_sync(0xffffffffu, busy);
   if (m) {
     int base = 0;
-    if (lane == 0) base = atomicAdd(&D.counts[0], __popc(m));
+    if (lane == 0) base = atomicAdd(&D.counts[8 * (*D.epoch & 1u)], __popc(m));
     base = __shfl_sync(0xffffffffu, base, 0);
     if (busy) D.worklist[base + __popc(m & ((1u << lane) - 1u))] = e;
   }
@@ -212,7 +216,7 @@ __global__ void __launch_bounds__(32 * kCoopWarps, 1) k_step_coop(const __grid_c
   // launched with programmatic stream serialization where possible (Ops::step_coop): the grid may be resident before the
   // preceding kernel has finished; everything that kernel wrote is visible after this call (no-op otherwise)
   cudaGridDependencySynchronize();
-  const int count = D.counts[0];
+  const int count = D.counts[0] + D.counts[8];  // the other set was cleared by the batch kernel
   // Static assignment, entries strided over the CTAs so that a short list spreads over all SMs (one environment per SM
   // up to 148 entries: no two chains share a scheduler or an instruction cache before they have to); every warp of the
   // CTA runs the same number of rounds, which the phase alignment (sag_core.cuh: coop_align) relies on.
@@ -251,6 +255,12 @@ __global__ void __launch_bounds__(32 * kCoopWarps, 1) k_step_coop(const __grid_c
     for (int k = lane; k < CoopCfg<RB>::kObs; k += 32) dst[k] = tile[k];
     __syncwarp();
   }
+  // The last CTA to finish advances the step epoch for the next step's batch kernel (which runs after this kernel) and
+  // re-arms the counter: one atomic per CTA, no launch
+  if (threadIdx.x == 0 && atomicAdd(&D.epoch[1], 1u) == gridDim.x - 1) {
+    D.epoch[1] = 0u;
+    atomicAdd(&D.epoch[0], 1u);
+  }
 }
 
 template <class RB>
@@ -269,7 +279,7 @@ __global__ void __launch_bounds__(kBS) k_observe(Dev D, float* __restrict__ obs)
 __global__ void __launch_bounds__(256) k_rollout_actions(Dev D, float* __restrict__ act) {
   const int e = blockIdx.x * blockDim.x + threadIdx.x;
   if (e >= D.n) return;
-  Rng rng = {D.seed, D.gid_base + (uint32_t)e, D.episode[e]};
+  Rng rng = {rng_key(D), D.gid_base + (uint32_t)e, D.episode[e]};
   double u1, u2;
   rng.pair(2u, (uint32_t)D.nstep[e], u1, u2);
   reinterpret_cast<float2*>(act)[e] = make_float2((float)(2.0 * u1 - 1.0), (float)(2.0 * u2 - 1.0));
@@ -466,7 +476,7 @@ __global__ void __launch_bounds__(128) k_fixup_host(const __grid_constant__ Dev 
                                                     double* __restrict__ reward_h, uint8_t* __restrict__ cost_h,
                                                     uint8_t* __restrict__ done_h) {
   const int lane = threadIdx.x & 31, nw = gridDim.x * 4;
-  const int count = D.counts[0];
+  const int count = D.counts[0] + D.counts[8];  // the step that just ran (the other set is zero)
   for (int i = blockIdx.x * 4 + (threadIdx.x >> 5); i < count; i += nw) {
     const int e = D.worklist[i];
     const float* src = obs + (size_t)e * kObs;
@@ -535,9 +545,8 @@ struct Ops {
   }
   static cudaError_t step_free(Handle* H, const float* act, float* obs, double* reward, double* reward2, uint8_t* cost,
                                uint8_t* done, cudaStream_t s) {
-    // two counter sets used alternately: this step's is zero already (cleared by the previous step's batch kernel, which
-    // saves a memset node per step); steps of one handle must be stream-ordered
-    int* t = H->D.counts; H->D.counts = H->D.counts_next; H->D.counts_next = t;
+    // this step's counter set is zero already (cleared by the previous step's batch kernel, which saves a memset node per
+    // step) and the kernels find it from the step epoch on the device; steps of one handle must be stream-ordered
     k_step_free<RB><<<grid_for(H->D.n), kBS, TileCfg<RB>::kTileBytes, s>>>(H->D, act, obs, reward, reward2, cost, done);
     ++H->launches;
     return cudaGetLastError();
@@ -652,6 +661,7 @@ int sag_create(const SagConfig* cfg, int device, void** handle) {
   H->cost_d = (uint8_t*)(base + LY.cost_off); H->done_d = (uint8_t*)(base + LY.done_off);
   // episode counters start at 0xFFFFFFFF so that the first reset is episode 0
   ce = cudaMemset(D.episode, 0xFF, st * sizeof(unsigned));
+  if (ce == cudaSuccess) ce = cudaMemcpy(D.key, &cfg->seed, sizeof(*D.key), cudaMemcpyHostToDevice);
   H->stats_acc = (double*)(base + LY.acc_off);
   H->ids_d = (int32_t*)(base + LY.ids_off); H->mask_d = (uint8_t*)(base + LY.mask_off);
   if (ce == cudaSuccess) ce = cudaHostAlloc((void**)&H->err_h, 4 * sizeof(int), cudaHostAllocMapped);
@@ -746,8 +756,11 @@ int sag_seed(void* handle, uint64_t seed) {
   if (!H) return fail("sag_seed: null handle");
   DevGuard guard(H->device);
   CK(cudaDeviceSynchronize());
+  // the key lives in the slab, so that kernels recorded in a CUDA graph draw from the new key on their next replay
   H->D.seed = seed;
-  CK(cudaMemset(H->D.episode, 0xFF, (size_t)H->D.stride * sizeof(unsigned)));
+  CK(cudaMemcpyAsync(H->D.key, &seed, sizeof(seed), cudaMemcpyHostToDevice, H->own_stream));
+  CK(cudaMemsetAsync(H->D.episode, 0xFF, (size_t)H->D.stride * sizeof(unsigned), H->own_stream));
+  CK(cudaStreamSynchronize(H->own_stream));
   return 0;
 }
 

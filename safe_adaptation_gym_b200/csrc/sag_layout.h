@@ -70,8 +70,13 @@ inline void slab_bind(Dev& D, const SlabLayout& L, char* base) {
   D.rext = (double*)(base + L.off[SAG_F_ROBOT_EXT]);
   D.grem = (double*)(base + L.off[SAG_F_GREMLINS]);
   int32_t* sc = (int32_t*)(base + L.sched_off);
-  D.worklist = sc; D.counts = sc + 3 * st; D.counts_next = D.counts + 8;
-  D.dbg = (unsigned long long*)(sc + 3 * st + 16);  // 18 x u64 (36 ints) after the two counter sets (16 ints); the block is 96 ints
+  // the block after the work list is 96 ints: two counter sets (16), 18 x u64 (36), the step epoch and the contact
+  // kernel's finished-CTA counter (2), the Philox key (u64; 8-byte aligned: the block starts 256-aligned and 3 * st is a
+  // multiple of 96)
+  D.worklist = sc; D.counts = sc + 3 * st;
+  D.dbg = (unsigned long long*)(sc + 3 * st + 16);
+  D.epoch = (unsigned*)(sc + 3 * st + 52);
+  D.key = (unsigned long long*)(sc + 3 * st + 54);
 }
 
 inline void dev_from_config(Dev& D, const SagConfig& c) {
@@ -86,7 +91,7 @@ inline void dev_from_config(Dev& D, const SagConfig& c) {
   D.k_gremlin = c.gremlins_keepout < c.gremlins_size ? c.gremlins_size : c.gremlins_keepout;
   D.k_pillar = c.pillars_keepout < c.pillars_size ? c.pillars_size : c.pillars_keepout;
   D.max_bound = c.max_bound; D.ctrl_range_scale = c.robot_ctrl_range_scale; D.random_bound = c.random_bound;
-  D.seed = c.seed; D.gid_base = c.env_id_base;
+  D.seed = c.seed; D.gid_base = c.env_id_base;  // (the library also writes the key into the slab: sag_create)
   D.max_layout_draws = c.max_layout_draws; D.max_episode_steps = c.max_episode_steps;
   D.num_gremlins = c.num_gremlins; D.gremlins_travel = c.gremlins_travel;
 }

@@ -11,6 +11,13 @@ With ``max_episode_steps > 0`` the env auto-resets like a vectorised gym wrapper
 (time limit, or done after a physics error) is reset inside ``step``; its row of ``obs`` is the FIRST observation of the
 new episode, ``done`` is True for it and ``info['truncated']`` marks the time-limit endings.
 
+``step`` (both output modes, with or without auto-reset), ``rollout`` and ``observation`` may be recorded in a CUDA graph
+(``torch.cuda.graph``), together with the policy that computes the actions; every replay behaves like issuing the same
+calls again.  ``seed``, ``set_task`` and ``load_state_dict`` between replays are seen by the graph, except that a
+``set_task`` which changes whether any environment runs ``Unsupervised`` changes the reward buffer ``step`` records:
+capture again after it.  No Python runs during a replay, so errors recorded by replayed steps are raised by
+``check_errors()``.  The methods that synchronise raise ``RuntimeError`` while a capture is open.
+
 All per-step arithmetic (dynamics, reward / goal logic, cost, pseudo-lidar) runs in the CUDA library behind
 the C ABI of ``include/sag_b200.h``; this class only owns torch tensors and passes raw pointers.  There is
 no CPU fallback: without the built library and a CUDA device construction raises.
@@ -37,6 +44,14 @@ WORLD_DEFAULT = {
 # task of the reference's registry has 0 gremlins) -- gremlins per environment, world.py:157-165
 _EXTRA_KEYS = {'max_layout_draws', 'num_gremlins'}
 _ROBOT_TO_CONTROL_FREQUENCY = {'doggo': 12, 'point': 5, 'car': 10}  # safe_adaptation_gym.py:15-19
+
+
+def _capturing() -> bool:
+    """True while the current CUDA stream is recording a graph."""
+    try:
+        return torch.cuda.is_current_stream_capturing()
+    except RuntimeError:  # no usable CUDA driver: nothing can be recording
+        return False
 
 
 def _robot_name(path: str) -> str:
@@ -151,6 +166,12 @@ class BatchedSafeAdaptationGym:
     def _out(self, t):
         return t.clone() if self.copy_outputs else t
 
+    @staticmethod
+    def _forbid_capture(what: str):
+        if _capturing():
+            raise RuntimeError(f'{what} synchronises with the device and cannot be recorded in a CUDA graph; '
+                               'call it outside the capture (a graph replayed afterwards sees its effect)')
+
     def _raise_recorded_errors(self, where: str):
         """The reference raises out of the call in which the condition occurs; the kernels record it in mapped host
         memory instead, which is read here WITHOUT synchronising -- so an error of a step that is still in flight is
@@ -162,7 +183,14 @@ class BatchedSafeAdaptationGym:
             raise ValueError('task id out of range')
 
     def step(self, action):
-        """safe_adaptation_gym.py:56-83.  `action`: [N, 2] tensor / array in [-1, 1]."""
+        """safe_adaptation_gym.py:56-83.  `action`: [N, 2] tensor / array in [-1, 1].
+
+        May be recorded in a CUDA graph (``torch.cuda.graph``) with the action already a tensor on this env's device;
+        a host / numpy action raises ``RuntimeError`` under capture.  A replay runs no Python: conditions the replayed
+        steps record (a goal that could not be sampled) are raised by ``check_errors()``, which a graphed loop should
+        call at the points where it wants them surfaced.  The tensors returned during the capture are the ones every
+        replay rewrites.
+        """
         act = self._as_action(action)
         L = self._lib
         r2 = self._reward2 if self._any_unsupervised else None
@@ -198,6 +226,7 @@ class BatchedSafeAdaptationGym:
 
     def reset(self, *, seed: Optional[int] = None, return_info: bool = False, options: Optional[dict] = None):
         """safe_adaptation_gym.py:85-107"""
+        self._forbid_capture('reset')
         assert self._task_ids is not None or (options is not None and 'task' in options), (
             'A task should be first set before reset.')
         if seed is not None:
@@ -210,11 +239,16 @@ class BatchedSafeAdaptationGym:
 
     def seed(self, seed=None):
         """safe_adaptation_gym.py:113-118: new stream key; episode counters restart"""
+        self._forbid_capture('seed')
         self._seed = int(np.random.randint(2**32)) if seed is None else int(seed)
         self._lib.check(self._lib.L.sag_seed(self._h, C.c_uint64(self._seed)))
 
     def set_task(self, task):
-        """safe_adaptation_gym.py:165-168.  `task`: a Task, or a sequence of N Tasks (one per environment)."""
+        """safe_adaptation_gym.py:165-168.  `task`: a Task, or a sequence of N Tasks (one per environment).
+
+        A CUDA graph that records ``step`` must be captured again when this changes whether any environment runs
+        ``Unsupervised`` (its reward is a pair, written to another buffer)."""
+        self._forbid_capture('set_task')
         if isinstance(task, _tasks.Task):
             task_list = [task] * self.num_envs
         else:
@@ -264,6 +298,11 @@ class BatchedSafeAdaptationGym:
     # batched extras
     # ------------------------------------------------------------------------------------------
     def _as_action(self, action):
+        on_device = (torch.is_tensor(action) and action.device.type == self.device.type
+                     and (action.device.index or 0) == (self.device.index or 0))
+        if not on_device and _capturing():
+            raise RuntimeError('under CUDA graph capture the action must already be a tensor on the env\'s device '
+                               f'({self.device}); a host or numpy action would record a copy from pageable memory')
         if not torch.is_tensor(action):
             action = torch.as_tensor(np.asarray(action, dtype=np.float32))
         act = action.to(device=self.device, dtype=torch.float32).reshape(self.num_envs, 2).contiguous()
@@ -276,18 +315,21 @@ class BatchedSafeAdaptationGym:
             m = mask.to(device=self.device, dtype=torch.uint8).contiguous()
         L.check(L.L.sag_reset(self._h, self._p(m), 0, 1 if new_task else 0, self._stream()))
         if new_task and self.base_config['random_bound']:  # world.py:75-78: drawn once per Task instance
-            self._bound = self.get_field('task_f64')[14, :self.num_envs].clone()
+            self._bound.copy_(self.get_field('task_f64')[14, :self.num_envs])  # in place: a CUDA graph may export it
         if self.device.type == 'cuda':
             torch.cuda.current_stream(self.device).synchronize()  # reset raises like the reference does (world.py:189)
         self._raise_recorded_errors('reset')
 
     def reset_envs(self, mask):
         """Reset only the environments where `mask` is true (vectorised-wrapper helper)."""
+        self._forbid_capture('reset_envs')
         self._reset_all(new_task=False, mask=torch.as_tensor(mask))
         return self.observation
 
     def check_errors(self):
-        """Raise the reference's exceptions for conditions recorded on the device since the last check."""
+        """Raise the reference's exceptions for conditions recorded on the device since the last check.  This is how
+        conditions recorded by CUDA graph replays of `step` surface: no Python runs during a replay."""
+        self._forbid_capture('check_errors')
         if self.device.type == 'cuda':
             torch.cuda.current_stream(self.device).synchronize()
         self._raise_recorded_errors('step')
@@ -309,6 +351,7 @@ class BatchedSafeAdaptationGym:
         return t
 
     def set_field(self, name: str, value: torch.Tensor):
+        self._forbid_capture('set_field')
         fid, dt, lead = self._FIELDS[name]
         t = torch.as_tensor(value).to(device=self.device, dtype=dt).contiguous()
         assert tuple(t.shape) == tuple(lead) + (self.stride,), (t.shape, lead, self.stride)
@@ -321,11 +364,13 @@ class BatchedSafeAdaptationGym:
         """Everything a bit-exact continuation needs: the Philox key, every SoA state field (they carry the episode and
         in-step draw counters, the task ids and the cached clearance), and the host-side step budget.  The
         finished-episode statistics of `task_stats` are not part of it."""
+        self._forbid_capture('state_dict')
         return {'seed': self._seed, 'num_envs': self.num_envs, 'robot': self.robot_name,
                 'config': dict(self.base_config), 'env_id_base': self.env_id_base, 'max_episode_steps': self.max_episode_steps,
                 'fields': {name: self.get_field(name).cpu() for name in self._FIELDS}}
 
     def load_state_dict(self, sd: dict):
+        self._forbid_capture('load_state_dict')
         if sd['num_envs'] != self.num_envs or sd['robot'] != self.robot_name:
             raise ValueError('state_dict belongs to a different batch size / robot')
         for key, mine in (('config', dict(self.base_config)), ('env_id_base', self.env_id_base),
@@ -342,7 +387,7 @@ class BatchedSafeAdaptationGym:
         self._any_unsupervised = bool((ids == _tasks.Unsupervised.task_id).any())
         self._observation_space = None
         if self.base_config['random_bound']:
-            self._bound = self.get_field('task_f64')[14, :self.num_envs].clone()
+            self._bound.copy_(self.get_field('task_f64')[14, :self.num_envs])  # in place: a CUDA graph may export it
 
     def rollout(self, k_steps: int):
         """K steps per launch with on-device Philox U(-1,1) actions; returns the last step's outputs."""
