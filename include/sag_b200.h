@@ -18,12 +18,12 @@
  *
  * CUDA graphs.  These stream entry points may be recorded in a CUDA graph (stream capture) and the graph replayed any
  * number of times: sag_step, sag_reset_obs / sag_reset with a mask or only_flagged != 0, sag_export_outputs,
- * sag_observe, sag_rollout, sag_read_field / sag_write_field and sag_task_stats.  A replay behaves exactly like issuing
- * the same calls again: everything the kernels read that can change after sag_create (the work-list counter sets and
- * the step epoch that selects them, the Philox key, the task ids) lives in the handle's device memory, so sag_seed and
- * sag_set_tasks issued between replays are seen by the graph.  The *_host entry points, sag_seed, sag_set_tasks_host,
- * sag_bound_host, sag_create / sag_destroy and sag_probe_d2h synchronise and must not be called while a capture is
- * open.  sag_launch_count counts host-side enqueues only: replays do not add to it.  Conditions recorded by replayed
+ * sag_observe, sag_rollout, sag_read_field / sag_write_field, sag_task_stats, sag_set_next_tasks and sag_bound.  A replay
+ * behaves exactly like issuing the same calls again: everything the kernels read that can change after sag_create (the
+ * work-list counter sets and the step epoch that selects them, the Philox key, the task ids, the queued next tasks)
+ * lives in the handle's device memory, so sag_seed and sag_set_tasks issued between replays are seen by the graph.  The
+ * *_host entry points, sag_seed, sag_set_tasks_host, sag_set_next_tasks_host, sag_bound_host, sag_create / sag_destroy
+ * and sag_probe_d2h synchronise and must not be called while a capture is open.  sag_launch_count counts host-side enqueues only: replays do not add to it.  Conditions recorded by replayed
  * kernels are read with sag_error_flags as usual.
  */
 #ifndef SAG_B200_H
@@ -86,6 +86,7 @@ enum {
   SAG_F_ROBOT_EXT = 5,/* double [6][stride]: car only -- wheel rates (2), castor ball-joint quaternion w,x,y,z (4) */
   SAG_F_GREMLINS = 6, /* double [2 + 3 * SAG_MAX_GREMLINS][stride]: mocap position of the last kinematics pass (x, y), then the weld
                          anchor (spawn x, y, yaw) of each gremlin */
+  SAG_F_NEXT_TASK = 7,/* int32 [stride]: task queued for the environment's next reset, -1 = none (sag_set_next_tasks) */
   SAG_NUM_FIELDS
 };
 
@@ -112,10 +113,27 @@ int sag_debug_read(void* handle, unsigned long long* out18_host);
  * the previous task are folded into the per-task totals first.  An id outside [0, SAG_NUM_TASKS) is replaced by
  * SAG_T_GO_TO_GOAL and reported through sag_error_flags (SAG_ERR_BAD_TASK_ID). */
 int sag_set_tasks(void* handle, const int32_t* task_ids_dev, void* stream);
-/* same with a HOST int32[n_envs] array (validated: out-of-range ids fail the call); synchronous */
+/* same with a HOST int32[n_envs] array (validated: out-of-range ids fail the call); synchronous.  sag_set_tasks and
+ * sag_set_tasks_host also clear every environment's queued next task. */
 int sag_set_tasks_host(void* handle, const int32_t* task_ids_host);
-/* info['bound'] (safe_adaptation_gym.py:79, world.py:75-78): HOST double[n_envs] constraint bound of every environment's
- * current Task instance; synchronous */
+/* Task switches at episode boundaries, per environment.  Every environment has a "next task" slot (SAG_F_NEXT_TASK,
+ * -1 = none) that its next reset consumes, whichever path resets it: the auto-reset of sag_reset_obs(only_flagged = 1),
+ * sag_reset / sag_reset_obs with or without a mask, sag_reset_host.  At that reset the environment (1) credits a
+ * finished episode to the task it ran under, as every reset does, (2) folds its statistics into the per-task totals
+ * under that old task, as sag_set_tasks does, (3) takes the queued id and clears the slot to -1, and (4) is reset as a
+ * fresh Task instance of the new task (as with new_task != 0, for this environment only, even if the id is unchanged):
+ * new ctrl-range scale and bound draws, new task state.  Environments with no task queued reset as the call asks.  A
+ * queued id outside [0, SAG_NUM_TASKS) is not applied: the slot is cleared and SAG_ERR_BAD_TASK_ID is reported through
+ * sag_error_flags.
+ * sag_set_next_tasks replaces every environment's slot from a DEVICE int32[n_envs] array (-1 = none); stream-ordered. */
+int sag_set_next_tasks(void* handle, const int32_t* task_ids_dev, void* stream);
+/* same with a HOST int32[n_envs] array (validated: an id outside [-1, SAG_NUM_TASKS) fails the call); synchronous */
+int sag_set_next_tasks_host(void* handle, const int32_t* task_ids_host);
+/* info['bound'] (safe_adaptation_gym.py:79, world.py:75-78): DEVICE double[n_envs] constraint bound of every
+ * environment's current Task instance; stream-ordered.  After task switches with SagConfig.random_bound this is how a
+ * caller's bound buffer follows the new draws. */
+int sag_bound(void* handle, double* bound_dev, void* stream);
+/* same into a HOST double[n_envs] buffer; synchronous */
 int sag_bound_host(void* handle, double* bound_host);
 /* Sticky error conditions recorded by the kernels since the last call with clear != 0, readable WITHOUT synchronising
  * (the kernels write them into mapped host memory): SAG_FLAG_RESAMPLE_FAILED -- a layout (world.py:189) or a goal

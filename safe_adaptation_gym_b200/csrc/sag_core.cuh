@@ -2494,6 +2494,31 @@ SAG_HD double slot_keepout(const Dev& D, const TaskSpec& sp, int kind) {
        : kind == K_PILLAR ? D.k_pillar : kind == K_GOAL ? kGoalKeepout : kind == K_BUTTON ? kButtonsKeepout : sp.box_keepout;
 }
 
+// The per-environment "next task" slot (SAG_F_NEXT_TASK, -1 = none), consumed by the next reset of environment e, whatever
+// the reset path.  Called by k_reset (lane 0 of the warp that resets e) and by the host emulation's reset, after the
+// finished episode has been credited to the per-environment statistics.  A queued task: the statistics gathered under
+// the old task are folded into the per-task accumulator `acc` (as k_set_tasks does), e takes the new task id and is
+// reset as a fresh Task instance even if the id is unchanged.  An id outside [0, T_COUNT) is not applied: the slot is
+// cleared and SAG_ERR_BAD_TASK_ID recorded.  Returns whether e is reset as a fresh Task instance.
+SAG_HD bool take_next_task(const Dev& D, int e, int* next_task, double* sret, double* scost, double* sn, double* acc,
+                           bool new_task) {
+  const int id = next_task[e];
+  if (id == -1) return new_task;
+  next_task[e] = -1;
+  if (id < 0 || id >= T_COUNT) { D.errflags[1] = 1; return new_task; }
+  const int old = D.task[e];
+  if (sn[e] != 0.0 && old >= 0 && old < T_COUNT) {
+#if defined(__CUDA_ARCH__)
+    atomicAdd(acc + 3 * old, sret[e]); atomicAdd(acc + 3 * old + 1, scost[e]); atomicAdd(acc + 3 * old + 2, sn[e]);
+#else
+    acc[3 * old] += sret[e]; acc[3 * old + 1] += scost[e]; acc[3 * old + 2] += sn[e];
+#endif
+  }
+  sret[e] = 0.0; scost[e] = 0.0; sn[e] = 0.0;
+  D.task[e] = id;
+  return true;
+}
+
 // The fresh episode after placement, shared by env_reset and env_reset_coop: the robot at rest at (x, y, yaw) and the
 // task state of environment C.e.  For a fresh Task instance (new_task) it makes the per-instance draws of World.__init__
 // (world.py:72-78): Task.ctrl_scale, standard Cauchy per actuator (task.py:85-89), and Task.constraint_bound

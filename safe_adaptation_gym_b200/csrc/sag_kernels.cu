@@ -69,6 +69,7 @@ struct Handle {
   size_t field_bytes[SAG_NUM_FIELDS];
   double *sret, *scost, *sn;  // per-env finished-episode statistics (under the env's current task)
   double* stats_acc;          // [SAG_NUM_TASKS][3]: statistics folded away when environments changed task
+  int32_t* next_task;         // [stride] SAG_F_NEXT_TASK: task queued for the next reset (-1 = none); k_reset consumes it
   int* err_h;                 // mapped pinned int[4]: sticky error words written by the kernels (sag_error_flags)
   int32_t* ids_d;             // staging for sag_set_tasks_host
   uint8_t* mask_d;            // staging for sag_reset_host
@@ -293,6 +294,9 @@ __global__ void __launch_bounds__(256) k_rollout_actions(Dev D, float* __restric
 // keeps every SM full of warps.
 // Statistics: an episode counts when it FINISHED (time limit or done: the NEEDS_RESET flag), under the task it ran with;
 // a manual reset of an unfinished episode is not an episode.
+// Next task: an environment with a task queued in next_task[e] takes it at this reset, whatever the reset path, and
+// starts a fresh Task instance of it (sag_core.cuh: take_next_task; its statistics are folded into `acc` under the old
+// task first).  The others reset as the call asks.
 // obs != nullptr: the environments that were reset get the first observation of their new episode written into their
 // row (the others' rows are left alone) and was_reset[e] = 1 / 0 tells the caller which (auto-reset, env.py).
 constexpr int kResetWarps = 4;
@@ -305,7 +309,8 @@ struct ResetCfg {
 };
 template <class RB, bool WithObs>
 __global__ void __launch_bounds__(32 * kResetWarps) k_reset(Dev D, const uint8_t* __restrict__ mask, int only_flagged, int new_task,
-                                                            double* sret, double* scost, double* sn, float* __restrict__ obs,
+                                                            double* sret, double* scost, double* sn, double* acc,
+                                                            int* next_task, float* __restrict__ obs,
                                                             uint8_t* __restrict__ was_reset, int gpc) {
   // gpc: environments per CTA (4 .. 32): small batches get one warp per environment, large ones eight per warp
   extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -330,10 +335,15 @@ __global__ void __launch_bounds__(32 * kResetWarps) k_reset(Dev D, const uint8_t
     const int e = blockIdx.x * gpc + (__ffs((int)todo) - 1);
     const unsigned char fl = D.flags[e];
     const unsigned episode = D.episode[e] + 1u;
-    if (lane == 0 && (fl & F_NEEDS_RESET) && D.nstep[e] > 0) { sret[e] += D.epret[e]; scost[e] += D.epcost[e]; sn[e] += 1.0; }
-    __syncwarp();
+    int fresh = new_task != 0;
+    if (lane == 0) {
+      if ((fl & F_NEEDS_RESET) && D.nstep[e] > 0) { sret[e] += D.epret[e]; scost[e] += D.epcost[e]; sn[e] += 1.0; }
+      fresh = take_next_task(D, e, next_task, sret, scost, sn, acc, fresh != 0);
+    }
+    fresh = __shfl_sync(0xffffffffu, fresh, 0);
+    __syncwarp();  // lane 0's writes (a new D.task[e]) are seen by the whole warp
 #if defined(__CUDA_ARCH__)
-    env_reset_coop<RB>(D, e, episode, new_task != 0, px, py, pk);
+    env_reset_coop<RB>(D, e, episode, fresh != 0, px, py, pk);
 #endif
     if (lane == 0 && (D.flags[e] & F_RESAMPLE_FAILED)) D.errflags[0] = 1;
     if constexpr (WithObs) {
@@ -347,8 +357,10 @@ __global__ void __launch_bounds__(32 * kResetWarps) k_reset(Dev D, const uint8_t
 }
 
 // env.set_task: statistics gathered under the old task are folded into the per-task accumulator first (so that they
-// are not re-labelled), including an episode that has finished but has not been reset yet; ids are validated.
-__global__ void k_set_tasks(Dev D, const int32_t* __restrict__ ids, double* sret, double* scost, double* sn, double* acc) {
+// are not re-labelled), including an episode that has finished but has not been reset yet; ids are validated; queued
+// next tasks are dropped.
+__global__ void k_set_tasks(Dev D, const int32_t* __restrict__ ids, double* sret, double* scost, double* sn, double* acc,
+                            int* next_task) {
   const int e = blockIdx.x * blockDim.x + threadIdx.x;
   if (e >= D.n) return;
   const int old = D.task[e];
@@ -359,6 +371,7 @@ __global__ void k_set_tasks(Dev D, const int32_t* __restrict__ ids, double* sret
   int id = ids[e];
   if (id < 0 || id >= SAG_NUM_TASKS) { id = SAG_T_GO_TO_GOAL; D.errflags[1] = 1; }
   D.task[e] = id;
+  next_task[e] = -1;
 }
 
 // per-task statistic reduction: out[task][3] += (sum return, sum cost, episodes) of finished episodes
@@ -601,10 +614,10 @@ struct Ops {
     const int grid = (H->D.n + gpc - 1) / gpc;
     ++H->launches;
     if (obs && (mask || only_flagged)) {  // selective reset: the first observation of the new episodes is written by the same kernel
-      k_reset<RB, true><<<grid, 32 * kResetWarps, ResetCfg<RB>::kSmemBytes, s>>>(H->D, mask, only_flagged, new_task, H->sret, H->scost, H->sn, obs, was_reset, gpc);
+      k_reset<RB, true><<<grid, 32 * kResetWarps, ResetCfg<RB>::kSmemBytes, s>>>(H->D, mask, only_flagged, new_task, H->sret, H->scost, H->sn, H->stats_acc, H->next_task, obs, was_reset, gpc);
       return cudaGetLastError();
     }
-    k_reset<RB, false><<<grid, 32 * kResetWarps, ResetCfg<RB>::kPlaceBytes * kResetWarps, s>>>(H->D, mask, only_flagged, new_task, H->sret, H->scost, H->sn, nullptr, was_reset, gpc);
+    k_reset<RB, false><<<grid, 32 * kResetWarps, ResetCfg<RB>::kPlaceBytes * kResetWarps, s>>>(H->D, mask, only_flagged, new_task, H->sret, H->scost, H->sn, H->stats_acc, H->next_task, nullptr, was_reset, gpc);
     cudaError_t ce = cudaGetLastError();
     if (ce == cudaSuccess && obs) ce = observe(H, obs, s);  // whole-batch reset: one thread per environment is the faster observation pass
     return ce;
@@ -664,6 +677,8 @@ int sag_create(const SagConfig* cfg, int device, void** handle) {
   if (ce == cudaSuccess) ce = cudaMemcpy(D.key, &cfg->seed, sizeof(*D.key), cudaMemcpyHostToDevice);
   H->stats_acc = (double*)(base + LY.acc_off);
   H->ids_d = (int32_t*)(base + LY.ids_off); H->mask_d = (uint8_t*)(base + LY.mask_off);
+  H->next_task = (int32_t*)H->field_ptr[SAG_F_NEXT_TASK];
+  if (ce == cudaSuccess) ce = cudaMemset(H->next_task, 0xFF, st * sizeof(int32_t));  // -1: no task queued
   if (ce == cudaSuccess) ce = cudaHostAlloc((void**)&H->err_h, 4 * sizeof(int), cudaHostAllocMapped);
   if (ce == cudaSuccess) { memset(H->err_h, 0, 4 * sizeof(int)); ce = cudaHostGetDevicePointer((void**)&D.errflags, H->err_h, 0); }
   if (ce == cudaSuccess) ce = cudaStreamCreateWithFlags(&H->own_stream, cudaStreamNonBlocking);
@@ -711,7 +726,7 @@ int sag_set_tasks(void* handle, const int32_t* ids, void* stream) {
   Handle* H = (Handle*)handle;
   if (!H || !ids) return fail("sag_set_tasks: null argument");
   DevGuard guard(H->device);
-  k_set_tasks<<<(H->D.n + 255) / 256, 256, 0, (cudaStream_t)stream>>>(H->D, ids, H->sret, H->scost, H->sn, H->stats_acc);
+  k_set_tasks<<<(H->D.n + 255) / 256, 256, 0, (cudaStream_t)stream>>>(H->D, ids, H->sret, H->scost, H->sn, H->stats_acc, H->next_task);
   ++H->launches;
   CK(cudaGetLastError());
   return 0;
@@ -725,10 +740,40 @@ int sag_set_tasks_host(void* handle, const int32_t* ids_host) {
   DevGuard guard(H->device);
   CK(cudaDeviceSynchronize());  // the host API is ordered after everything issued through the stream API
   CK(cudaMemcpyAsync(H->ids_d, ids_host, (size_t)H->D.n * sizeof(int32_t), cudaMemcpyHostToDevice, H->own_stream));
-  k_set_tasks<<<(H->D.n + 255) / 256, 256, 0, H->own_stream>>>(H->D, H->ids_d, H->sret, H->scost, H->sn, H->stats_acc);
+  k_set_tasks<<<(H->D.n + 255) / 256, 256, 0, H->own_stream>>>(H->D, H->ids_d, H->sret, H->scost, H->sn, H->stats_acc, H->next_task);
   ++H->launches;
   CK(cudaGetLastError());
   CK(cudaStreamSynchronize(H->own_stream));
+  return 0;
+}
+
+int sag_set_next_tasks(void* handle, const int32_t* ids, void* stream) {
+  Handle* H = (Handle*)handle;
+  if (!H || !ids) return fail("sag_set_next_tasks: null argument");
+  DevGuard guard(H->device);
+  // the ids are checked where they are consumed (k_reset), like ids written with sag_write_field
+  CK(cudaMemcpyAsync(H->next_task, ids, (size_t)H->D.n * sizeof(int32_t), cudaMemcpyDeviceToDevice, (cudaStream_t)stream));
+  return 0;
+}
+
+int sag_set_next_tasks_host(void* handle, const int32_t* ids_host) {
+  Handle* H = (Handle*)handle;
+  if (!H || !ids_host) return fail("sag_set_next_tasks_host: null argument");
+  for (int e = 0; e < H->D.n; ++e)
+    if (ids_host[e] < -1 || ids_host[e] >= SAG_NUM_TASKS)
+      return fail("sag_set_next_tasks_host: task id out of range [-1, SAG_NUM_TASKS)");
+  DevGuard guard(H->device);
+  CK(cudaDeviceSynchronize());  // the host API is ordered after everything issued through the stream API
+  CK(cudaMemcpyAsync(H->next_task, ids_host, (size_t)H->D.n * sizeof(int32_t), cudaMemcpyHostToDevice, H->own_stream));
+  CK(cudaStreamSynchronize(H->own_stream));
+  return 0;
+}
+
+int sag_bound(void* handle, double* bound, void* stream) {
+  Handle* H = (Handle*)handle;
+  if (!H || !bound) return fail("sag_bound: null argument");
+  DevGuard guard(H->device);
+  CK(cudaMemcpyAsync(bound, H->D.bound, (size_t)H->D.n * sizeof(double), cudaMemcpyDeviceToDevice, (cudaStream_t)stream));
   return 0;
 }
 

@@ -36,6 +36,7 @@ inline SlabLayout slab_layout(int n, int stride, int obs_dim) {
   L.bytes[SAG_F_FLAGS] = st;
   L.bytes[SAG_F_ROBOT_EXT] = 6 * st * sizeof(double);
   L.bytes[SAG_F_GREMLINS] = (2 + 3 * (size_t)SAG_MAX_GREMLINS) * st * sizeof(double);
+  L.bytes[SAG_F_NEXT_TASK] = st * sizeof(int32_t);  // not bound into Dev: the reset kernels take it as an argument
   size_t total = 0;
   for (int f = 0; f < SAG_NUM_FIELDS; ++f) { L.off[f] = total; total += align_up(L.bytes[f], 256); }
   L.stats_off = total; total += align_up(3 * st * sizeof(double), 256);

@@ -18,6 +18,14 @@ calls again.  ``seed``, ``set_task`` and ``load_state_dict`` between replays are
 capture again after it.  No Python runs during a replay, so errors recorded by replayed steps are raised by
 ``check_errors()``.  The methods that synchronise raise ``RuntimeError`` while a capture is open.
 
+Task switches per environment: ``set_next_task`` queues a task for each environment's NEXT reset (the auto-reset inside
+``step``, ``reset``, ``reset_envs``), so that every environment of a staggered batch moves on to its next task when its
+own episode ends, without cutting any running episode short.  At that reset the environment's finished episode and
+statistics stay with the old task (``task_stats``), and it starts a fresh Task instance of the queued task (new
+ctrl-range scale and bound draws).  With a device tensor of ids it may be recorded in a CUDA graph with the policy and
+``step``, so a graphed adaptation loop can walk through tasks; ``task_ids`` tells which task each environment runs now.
+``set_task(task, mask)`` switches the masked environments at once (their running episodes are cut short and not counted).
+
 All per-step arithmetic (dynamics, reward / goal logic, cost, pseudo-lidar) runs in the CUDA library behind
 the C ABI of ``include/sag_b200.h``; this class only owns torch tensors and passes raw pointers.  There is
 no CPU fallback: without the built library and a CUDA device construction raises.
@@ -136,6 +144,7 @@ class BatchedSafeAdaptationGym:
         self._task_ids = None
         self._tasks = None
         self._any_unsupervised = False
+        self._next_armed = False   # set_next_task has been called: step refreshes a random bound after the auto-reset
         self._action_space = Box(-1, 1, (2,), dtype=np.float32)  # safe_adaptation_gym.py:49-50 (nu = 2)
         self._observation_space = None
 
@@ -203,6 +212,9 @@ class BatchedSafeAdaptationGym:
             # into their rows and reports which ones it reset
             L.check(L.L.sag_reset_obs(self._h, None, 1, 0, self._p(self._obs), self._p(self._was_reset), self._stream()))
             was_reset = self._was_reset.to(torch.bool)
+            if self._next_armed and self.base_config['random_bound']:
+                # an environment that switched task drew a new bound (world.py:75-78); in place: a graph may export it
+                L.check(L.L.sag_bound(self._h, self._p(self._bound), self._stream()))
         if self.copy_outputs:
             # fresh arrays, as the reference returns them (safe_adaptation_gym.py:80-83) -- one launch for all of them
             n, dev = self.num_envs, self.device
@@ -243,12 +255,8 @@ class BatchedSafeAdaptationGym:
         self._seed = int(np.random.randint(2**32)) if seed is None else int(seed)
         self._lib.check(self._lib.L.sag_seed(self._h, C.c_uint64(self._seed)))
 
-    def set_task(self, task):
-        """safe_adaptation_gym.py:165-168.  `task`: a Task, or a sequence of N Tasks (one per environment).
-
-        A CUDA graph that records ``step`` must be captured again when this changes whether any environment runs
-        ``Unsupervised`` (its reward is a pair, written to another buffer)."""
-        self._forbid_capture('set_task')
+    def _task_list(self, task, allow_none: bool):
+        """A Task, or a sequence of N Tasks (or None where `allow_none`), validated -> list of N."""
         if isinstance(task, _tasks.Task):
             task_list = [task] * self.num_envs
         else:
@@ -256,15 +264,95 @@ class BatchedSafeAdaptationGym:
             if len(task_list) != self.num_envs:
                 raise ValueError(f'need {self.num_envs} tasks, got {len(task_list)}')
         for t in task_list:
+            if t is None and allow_none:
+                continue
             if t.name in _tasks.DEVICE_UNSUPPORTED:
                 raise NotImplementedError(f"task '{t.name}' is not implemented on the device path yet")
+        return task_list
+
+    def set_task(self, task, mask=None):
+        """safe_adaptation_gym.py:165-168.  `task`: a Task, or a sequence of N Tasks (one per environment).
+
+        Without `mask` every environment starts a fresh Task instance now, and tasks queued with ``set_next_task`` are
+        dropped.  With `mask` (N booleans) only the masked environments switch now, to fresh Task instances of their
+        entries of `task`; their running episodes are cut short and not counted in ``task_stats``.  The others keep
+        running and keep their queued tasks.
+
+        A CUDA graph that records ``step`` must be captured again when this changes whether any environment runs
+        ``Unsupervised`` (its reward is a pair, written to another buffer)."""
+        self._forbid_capture('set_task')
+        task_list = self._task_list(task, allow_none=False)
         ids = torch.tensor([t.task_id for t in task_list], dtype=torch.int32)
+        if mask is not None:
+            m = torch.as_tensor(mask).to(device=self.device, dtype=torch.bool).reshape(self.num_envs)
+            unsup = ids == _tasks.Unsupervised.task_id
+            self._any_unsupervised = self._any_unsupervised or bool(unsup[m.cpu()].any())
+            # the masked environments get the task queued and are reset: the reset consumes the slot
+            queued = torch.where(m, ids.to(self.device), self.get_field('next_task')[:self.num_envs]).contiguous()
+            self._lib.check(self._lib.L.sag_set_next_tasks(self._h, self._p(queued), self._stream()))
+            self._reset_all(new_task=False, mask=m, switch=True)
+            self._tasks_from_ids(self.task_ids.cpu())
+            return
         self._tasks = task_list
         self._task_ids = ids.to(self.device)
         self._any_unsupervised = bool((ids == _tasks.Unsupervised.task_id).any())
         self._lib.check(self._lib.L.sag_set_tasks(self._h, self._p(self._task_ids), self._stream()))
         self._observation_space = None
         self._reset_all(new_task=True)
+
+    def set_next_task(self, task):
+        """Queue the task each environment takes at its NEXT reset (-1 / None = none); replaces every environment's
+        queue slot.  `task`: a Task (all environments), a sequence of N Tasks or None, or an int32 tensor [N] of task
+        ids on this env's device.
+
+        The next reset of an environment with a queued task -- the auto-reset inside ``step``, ``reset``,
+        ``reset_envs`` -- credits its finished episode and its statistics to the task it ran under, then starts a fresh
+        Task instance of the queued task (new ctrl-range scale and bound draws, even if the id is unchanged) and clears
+        the slot.  The other environments reset as before.  ``set_task`` without a mask clears every slot.
+
+        May be recorded in a CUDA graph with a device tensor (a host sequence raises ``RuntimeError`` under capture).
+        Host input is validated; a device tensor is checked where it is consumed: an id outside [-1, 14) is not applied
+        and raises ``ValueError`` at the next call that checks errors (``step``, ``check_errors``).  Queuing
+        ``Unsupervised`` into a batch whose reward is not the pair raises ``ValueError``: ``step`` would have to record
+        another reward buffer, so use ``set_task`` for that.  With a device tensor this is the caller's rule.  With
+        ``random_bound``, ``step`` refreshes ``info['bound']`` after the auto-reset once this has been called: capture
+        a graph of ``step`` after the first call."""
+        on_device = (torch.is_tensor(task) and task.device.type == self.device.type
+                     and (task.device.index or 0) == (self.device.index or 0))
+        if on_device:
+            if task.dtype != torch.int32 or tuple(task.shape) != (self.num_envs,):
+                raise ValueError(f'need an int32 tensor of shape ({self.num_envs},), got {task.dtype} {tuple(task.shape)}')
+            ids = task.contiguous()
+        else:
+            if _capturing():
+                raise RuntimeError('under CUDA graph capture set_next_task needs an int32 tensor of task ids on the env\'s '
+                                   f'device ({self.device}); a host sequence would record a copy from pageable memory')
+            if torch.is_tensor(task) or isinstance(task, np.ndarray):
+                by_id = {cls.task_id: cls for cls in _tasks.TASK_CLASSES}
+                raw = [int(i) for i in np.asarray(task.cpu() if torch.is_tensor(task) else task).reshape(-1)]
+                bad = [i for i in raw if i != -1 and i not in by_id]
+                if bad:
+                    raise ValueError(f'task id {bad[0]} out of range [-1, {_abi.NUM_TASKS})')
+                task = [None if i == -1 else by_id[i]() for i in raw]
+            task_list = self._task_list(task, allow_none=True)
+            if not self._any_unsupervised and any(isinstance(t, _tasks.Unsupervised) for t in task_list):
+                raise ValueError("Unsupervised's reward is a pair, which this batch's step does not record: "
+                                 'switch to it with set_task')
+            ids = torch.tensor([-1 if t is None else t.task_id for t in task_list], dtype=torch.int32).to(self.device)
+        self._lib.check(self._lib.L.sag_set_next_tasks(self._h, self._p(ids), self._stream()))
+        self._next_armed = True
+
+    @property
+    def task_ids(self) -> torch.Tensor:
+        """int32 [N] on the env's device: the task each environment runs now (it changes at the resets that consume
+        queued tasks).  May be read inside a CUDA graph."""
+        return self.get_field('task_i32')[0, :self.num_envs]
+
+    def _tasks_from_ids(self, ids: torch.Tensor):
+        """The host-side task list from the ids the device holds (int32 [N] on the host)."""
+        by_id = {cls.task_id: cls for cls in _tasks.TASK_CLASSES}
+        self._tasks = [by_id[int(i)]() for i in ids.tolist()]
+        self._task_ids = ids.to(self.device)
 
     def render(self, mode='human'):
         raise NotImplementedError('rendering is outside the B200 hot path (reference: safe_adaptation_gym.py:109-111)')
@@ -308,13 +396,14 @@ class BatchedSafeAdaptationGym:
         act = action.to(device=self.device, dtype=torch.float32).reshape(self.num_envs, 2).contiguous()
         return act
 
-    def _reset_all(self, new_task: bool, mask: Optional[torch.Tensor] = None):
+    def _reset_all(self, new_task: bool, mask: Optional[torch.Tensor] = None, switch: bool = False):
         L = self._lib
         m = None
         if mask is not None:
             m = mask.to(device=self.device, dtype=torch.uint8).contiguous()
         L.check(L.L.sag_reset(self._h, self._p(m), 0, 1 if new_task else 0, self._stream()))
-        if new_task and self.base_config['random_bound']:  # world.py:75-78: drawn once per Task instance
+        # world.py:75-78: drawn once per Task instance (also by the environments that took a queued task)
+        if (new_task or switch or self._next_armed) and self.base_config['random_bound']:
             self._bound.copy_(self.get_field('task_f64')[14, :self.num_envs])  # in place: a CUDA graph may export it
         if self.device.type == 'cuda':
             torch.cuda.current_stream(self.device).synchronize()  # reset raises like the reference does (world.py:189)
@@ -340,7 +429,8 @@ class BatchedSafeAdaptationGym:
     _FIELDS = {'robot': (_abi.F_ROBOT, torch.float64, (6,)), 'objects': (_abi.F_OBJECTS, torch.float64, (6, _abi.MAX_SLOTS)),
                'task_f64': (_abi.F_TASK_F64, torch.float64, (15,)), 'task_i32': (_abi.F_TASK_I32, torch.int32, (10,)),
                'flags': (_abi.F_FLAGS, torch.uint8, ()), 'robot_ext': (_abi.F_ROBOT_EXT, torch.float64, (6,)),
-               'gremlins': (_abi.F_GREMLINS, torch.float64, (2 + 3 * _abi.MAX_GREMLINS,))}
+               'gremlins': (_abi.F_GREMLINS, torch.float64, (2 + 3 * _abi.MAX_GREMLINS,)),
+               'next_task': (_abi.F_NEXT_TASK, torch.int32, ())}
 
     def get_field(self, name: str) -> torch.Tensor:
         """Copy of an internal SoA state field, shape (*lead, stride) (see include/sag_b200.h SAG_F_*)."""
@@ -362,8 +452,8 @@ class BatchedSafeAdaptationGym:
     # ---- checkpoint / resume ------------------------------------------------------------------
     def state_dict(self) -> dict:
         """Everything a bit-exact continuation needs: the Philox key, every SoA state field (they carry the episode and
-        in-step draw counters, the task ids and the cached clearance), and the host-side step budget.  The
-        finished-episode statistics of `task_stats` are not part of it."""
+        in-step draw counters, the task ids, the queued next tasks and the cached clearance), and the host-side step
+        budget.  The finished-episode statistics of `task_stats` are not part of it."""
         self._forbid_capture('state_dict')
         return {'seed': self._seed, 'num_envs': self.num_envs, 'robot': self.robot_name,
                 'config': dict(self.base_config), 'env_id_base': self.env_id_base, 'max_episode_steps': self.max_episode_steps,
@@ -380,10 +470,12 @@ class BatchedSafeAdaptationGym:
         self.seed(sd['seed'])
         for name, value in sd['fields'].items():
             self.set_field(name, value)
+        if 'next_task' not in sd['fields']:   # saved before tasks could be queued: nothing queued
+            self.set_field('next_task', torch.full((self.stride,), -1, dtype=torch.int32))
+        if bool((sd['fields'].get('next_task', torch.full((1,), -1)) != -1).any()):
+            self._next_armed = True
         ids = sd['fields']['task_i32'][0, :self.num_envs].to(torch.int32)
-        by_id = {cls.task_id: cls for cls in _tasks.TASK_CLASSES}
-        self._tasks = [by_id[int(i)]() for i in ids.tolist()]
-        self._task_ids = ids.to(self.device)
+        self._tasks_from_ids(ids)
         self._any_unsupervised = bool((ids == _tasks.Unsupervised.task_id).any())
         self._observation_space = None
         if self.base_config['random_bound']:
