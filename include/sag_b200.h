@@ -18,11 +18,13 @@
  *
  * CUDA graphs.  These stream entry points may be recorded in a CUDA graph (stream capture) and the graph replayed any
  * number of times: sag_step, sag_reset_obs / sag_reset with a mask or only_flagged != 0, sag_export_outputs,
- * sag_observe, sag_rollout, sag_read_field / sag_write_field, sag_task_stats, sag_set_next_tasks and sag_bound.  A replay
+ * sag_observe, sag_rollout, sag_read_field / sag_write_field, sag_task_stats, sag_set_next_tasks, sag_bound and
+ * sag_copy_envs.  A replay
  * behaves exactly like issuing the same calls again: everything the kernels read that can change after sag_create (the
  * work-list counter sets and the step epoch that selects them, the Philox key, the task ids, the queued next tasks)
  * lives in the handle's device memory, so sag_seed and sag_set_tasks issued between replays are seen by the graph.  The
- * *_host entry points, sag_seed, sag_set_tasks_host, sag_set_next_tasks_host, sag_bound_host, sag_create / sag_destroy
+ * *_host entry points, sag_seed, sag_set_tasks_host, sag_set_next_tasks_host, sag_bound_host, sag_copy_envs_host,
+ * sag_create / sag_destroy
  * and sag_probe_d2h synchronise and must not be called while a capture is open.  sag_launch_count counts host-side enqueues only: replays do not add to it.  Conditions recorded by replayed
  * kernels are read with sag_error_flags as usual.
  */
@@ -52,8 +54,8 @@ enum {
 };
 /* per-env flag bits (sag_read_field(SAG_F_FLAGS)) */
 enum { SAG_FLAG_PHYSICS_ERROR = 1, SAG_FLAG_RESAMPLE_FAILED = 2, SAG_FLAG_NEEDS_RESET = 4 };
-/* additional bit of sag_error_flags() */
-enum { SAG_ERR_BAD_TASK_ID = 8 };
+/* additional bits of sag_error_flags() */
+enum { SAG_ERR_BAD_TASK_ID = 8, SAG_ERR_BAD_ENV_INDEX = 16 };
 
 /* World.DEFAULT (world.py:17-34) + batching parameters.  POD, copied at sag_create. */
 typedef struct SagConfig {
@@ -74,7 +76,8 @@ typedef struct SagConfig {
 } SagConfig;
 
 /* state fields for injection / extraction (parity tests, checkpointing).  All arrays are SoA,
- * environment-minor with element stride sag_stride(h):  field[k][env]. */
+ * environment-minor with element stride sag_stride(h):  field[k][env].  Together with the Philox key and the global
+ * environment id they are the complete state of an environment: sag_copy_envs copies every row of every field. */
 enum {
   SAG_F_ROBOT = 0,    /* double [6][stride]: x, y, yaw, vx, vy, w */
   SAG_F_OBJECTS = 1,  /* double [6][SAG_MAX_SLOTS][stride]: x, y, yaw, vx, vy, w per object slot */
@@ -138,8 +141,40 @@ int sag_bound_host(void* handle, double* bound_host);
 /* Sticky error conditions recorded by the kernels since the last call with clear != 0, readable WITHOUT synchronising
  * (the kernels write them into mapped host memory): SAG_FLAG_RESAMPLE_FAILED -- a layout (world.py:189) or a goal
  * (go_to_goal.py:80) could not be sampled, i.e. the reference would have raised ResamplingError out of reset / step;
- * SAG_ERR_BAD_TASK_ID.  A condition raised by a kernel that is still running shows up in a later call. */
+ * SAG_ERR_BAD_TASK_ID; SAG_ERR_BAD_ENV_INDEX (sag_copy_envs).  A condition raised by a kernel that is still running
+ * shows up in a later call. */
 int sag_error_flags(void* handle, int clear);
+
+/* Copy environment states, within one handle or from another handle of the same device (lookahead from the live
+ * state, resets to chosen states).  src_of_dst holds one int32 per destination environment: every environment j of
+ * `dst` with src_of_dst[j] = s >= 0 takes the complete state of environment s of `src` (src may be dst); -1 leaves j
+ * untouched.  A gather: a destination never receives two sources, and one source may go to many destinations.
+ *  - Copied: every row of every SAG_F_* field (robot, objects, task_f64, task_i32, flags, robot_ext, gremlins,
+ *    next_task), bit for bit, also rows the robot model does not use.  The derived values (moving mask, clearance) come
+ *    with them, so no sag_observe is needed.  So do the episode number and the in-step draw counter: with the same seed
+ *    and an env_id_base that gives the copy the source's global id, the copy replays the source exactly (goal and
+ *    button resamples, auto-resets, queued task switches); with another global id it follows the source until its
+ *    first in-step draw.  The running return and cost (task_f64 rows 8-9) come too: the copy's episode is credited in
+ *    full to dst when it finishes.
+ *  - Not copied (they belong to the handle or the slot): the Philox key and the global id, so the copy draws from dst's
+ *    streams; the finished-episode statistics; the work list, counter sets and step epoch; the error words.
+ *  - Statistics: before its state is replaced, the destination is settled as a reset settles it: an episode that has
+ *    finished (time limit or done) but has not been reset yet is credited to its OLD task, an unfinished one is dropped
+ *    and not counted.  Its finished-episode statistics are then folded into dst's per-task totals under its OLD task
+ *    and cleared (the rule of sag_set_tasks), so that sag_task_stats does not credit them to the copied task.
+ *  - Aliasing: a pair j <- s with s != j is applied only if s is not itself overwritten by the call, i.e. src_of_dst[s]
+ *    is -1 or s (dst == src only); j <- j does nothing.  Decided from the read-only index array: race-free, deterministic.
+ *  - Compatibility: the call fails (nothing enqueued) unless both handles are on the same device and agree in robot,
+ *    num_gremlins, every object size and (effective) keepout, placements_margin, robot_keepout, gremlins_travel,
+ *    robot_ctrl_range_scale, random_bound and max_bound.  They may differ in n_envs, seed, env_id_base,
+ *    max_episode_steps, max_layout_draws and action_noise.
+ * sag_copy_envs: src_of_dst_dev is a DEVICE int32[dst n_envs] array; stream-ordered.  A pair whose index is outside
+ * [-1, src n_envs) or that breaks the aliasing rule is not applied and SAG_ERR_BAD_ENV_INDEX is reported through
+ * dst's sag_error_flags. */
+int sag_copy_envs(void* dst, void* src, const int32_t* src_of_dst_dev, void* stream);
+/* same with a HOST int32[dst n_envs] array (validated: an index out of range or a pair that breaks the aliasing rule
+ * fails the call); synchronous */
+int sag_copy_envs_host(void* dst, void* src, const int32_t* src_of_dst_host);
 
 /* env.seed (safe_adaptation_gym.py:113-118): new Philox key; per-env episode counters restart */
 int sag_seed(void* handle, uint64_t seed);

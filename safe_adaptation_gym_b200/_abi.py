@@ -15,7 +15,7 @@ NUM_TASKS = 14
 MAX_SLOTS = 32
 MAX_GREMLINS = 4
 F_ROBOT, F_OBJECTS, F_TASK_F64, F_TASK_I32, F_FLAGS, F_ROBOT_EXT, F_GREMLINS, F_NEXT_TASK = range(8)
-FLAG_PHYSICS_ERROR, FLAG_RESAMPLE_FAILED, FLAG_NEEDS_RESET, ERR_BAD_TASK_ID = 1, 2, 4, 8
+FLAG_PHYSICS_ERROR, FLAG_RESAMPLE_FAILED, FLAG_NEEDS_RESET, ERR_BAD_TASK_ID, ERR_BAD_ENV_INDEX = 1, 2, 4, 8, 16
 
 
 class SagConfig(C.Structure):
@@ -42,7 +42,7 @@ class SagLib:
     SYMBOLS = [
         "sag_last_error", "sag_abi_version", "sag_default_config", "sag_create", "sag_destroy", "sag_stride",
         "sag_obs_dim", "sag_field_bytes", "sag_launch_count", "sag_debug_read", "sag_set_tasks", "sag_set_tasks_host", "sag_bound_host",
-        "sag_set_next_tasks", "sag_set_next_tasks_host", "sag_bound",
+        "sag_set_next_tasks", "sag_set_next_tasks_host", "sag_bound", "sag_copy_envs", "sag_copy_envs_host",
         "sag_error_flags", "sag_reset_obs", "sag_reset_host", "sag_seed", "sag_reset", "sag_step", "sag_observe",
         "sag_step_host", "sag_observe_host", "sag_host_alloc", "sag_host_alloc_outputs", "sag_probe_d2h", "sag_host_free", "sag_rollout", "sag_read_field",
         "sag_write_field", "sag_task_stats", "sag_lidar", "sag_cost", "sag_export_outputs",
@@ -74,6 +74,9 @@ class SagLib:
         if hasattr(L, "sag_set_next_tasks"):
             L.sag_set_next_tasks.argtypes = [vp, vp, vp]
             L.sag_bound.argtypes = [vp, dp, vp]
+        if hasattr(L, "sag_copy_envs"):
+            L.sag_copy_envs.argtypes = [vp, vp, vp, vp]
+            L.sag_copy_envs_host.argtypes = [vp, vp, vp]
         L.sag_seed.argtypes = [vp, C.c_uint64]
         L.sag_error_flags.argtypes = [vp, i32]
         L.sag_reset_obs.argtypes = [vp, u8p, i32, i32, fp, u8p, vp]

@@ -208,7 +208,8 @@ struct Dev {
                            // finished (sag_kernels.cu: k_step_free, k_step_coop)
   unsigned long long* dbg; // [16] section clocks of SAG_TIMING builds
   int* errflags;           // [4] sticky error words the host can read without a synchronisation (mapped pinned memory):
-                           // [0] a layout / goal could not be sampled (ResamplingError), [1] task id out of range
+                           // [0] a layout / goal could not be sampled (ResamplingError), [1] task id out of range,
+                           // [2] a bad sag_copy_envs pair
   double *time, *clear;
   unsigned *ctr, *episode;
   int* nstep;
@@ -2517,6 +2518,44 @@ SAG_HD bool take_next_task(const Dev& D, int e, int* next_task, double* sret, do
   sret[e] = 0.0; scost[e] = 0.0; sn[e] = 0.0;
   D.task[e] = id;
   return true;
+}
+
+// sag_copy_envs, the rule for destination j of the destination handle D: returns the source environment whose state j
+// takes, or -1 when j is left untouched.  -1 in src_of_dst[j] and the no-op j <- j leave j alone.  A pair is bad, and
+// not applied, when its index is outside [-1, n_src) or, within one handle, when its source is itself overwritten by the
+// call (src_of_dst[s] not in {-1, s}): read from the index array alone, so every thread decides alike.  With `fold`
+// (k_copy_envs_fold, one thread per destination, before any field is overwritten; the host emulation's loop), a bad
+// pair records SAG_ERR_BAD_ENV_INDEX, and for an applied one j's statistics are settled as a reset or k_set_tasks
+// settles them before j's state is replaced: an episode that has finished (NEEDS_RESET, nstep > 0) but has not been
+// reset yet is credited, then j's finished-episode statistics are folded into the per-task accumulator `acc` under j's
+// OLD task and cleared, so that they are not credited to the copied task.  An unfinished episode of j is dropped.
+SAG_HD int copy_env_source(const Dev& D, const int32_t* src_of_dst, int j, int n_src, bool same_handle, bool fold,
+                           double* sret, double* scost, double* sn, double* acc) {
+  const int s = src_of_dst[j];
+  if (s == -1 || (same_handle && s == j)) return -1;
+  bool bad = s < -1 || s >= n_src;
+  if (!bad && same_handle) {
+    const int t = src_of_dst[s];
+    bad = t != -1 && t != s;
+  }
+  if (bad) {
+    if (fold) D.errflags[2] = 1;
+    return -1;
+  }
+  if (fold) {
+    const int old = D.task[j];
+    double r = sret[j], c = scost[j], k = sn[j];
+    if ((D.flags[j] & F_NEEDS_RESET) && D.nstep[j] > 0) { r += D.epret[j]; c += D.epcost[j]; k += 1.0; }
+    if (k != 0.0 && old >= 0 && old < T_COUNT) {
+#if defined(__CUDA_ARCH__)
+      atomicAdd(acc + 3 * old, r); atomicAdd(acc + 3 * old + 1, c); atomicAdd(acc + 3 * old + 2, k);
+#else
+      acc[3 * old] += r; acc[3 * old + 1] += c; acc[3 * old + 2] += k;
+#endif
+    }
+    sret[j] = 0.0; scost[j] = 0.0; sn[j] = 0.0;
+  }
+  return s;
 }
 
 // The fresh episode after placement, shared by env_reset and env_reset_coop: the robot at rest at (x, y, yaw) and the

@@ -374,6 +374,62 @@ __global__ void k_set_tasks(Dev D, const int32_t* __restrict__ ids, double* sret
   next_task[e] = -1;
 }
 
+// sag_copy_envs: environment states gathered column by column.  The fields are SoA and environment-minor, so the
+// threads run over (chunk of field rows, destination) with the destination fastest: the stores of a warp are one
+// contiguous segment per row, and the loads are too for contiguous sources, or a broadcast for K copies of one source.
+// A chunk is up to kCopyRows rows of one field; each thread issues all its loads before its stores.  Memory-bound: no
+// arithmetic besides the pair rule (sag_core.cuh: copy_env_source).  The destination's statistics are settled by
+// k_copy_envs_fold, launched before it on the same stream: it reads the destination's flags, step count, episode return
+// and cost and task id, which k_copy_envs overwrites from other chunks.
+constexpr int kCopyRows = 8, kCopyThreads = 256;
+struct CopyFields {
+  char* dst[SAG_NUM_FIELDS];
+  const char* src[SAG_NUM_FIELDS];
+  int rows[SAG_NUM_FIELDS], elem[SAG_NUM_FIELDS];
+};
+constexpr int copy_chunks() {
+  int c = 0;
+  for (int f = 0; f < SAG_NUM_FIELDS; ++f) c += (kFieldShape[f].rows + kCopyRows - 1) / kCopyRows;
+  return c;
+}
+
+template <class T>
+__device__ __forceinline__ void copy_rows(char* dst, const char* src, int r0, int nr, int dst_stride, int src_stride,
+                                          int j, int s) {
+  const T* sp = reinterpret_cast<const T*>(src) + (size_t)r0 * src_stride + s;
+  T* dp = reinterpret_cast<T*>(dst) + (size_t)r0 * dst_stride + j;
+  T v[kCopyRows];
+#pragma unroll
+  for (int k = 0; k < kCopyRows; ++k) if (k < nr) v[k] = sp[(size_t)k * src_stride];
+#pragma unroll
+  for (int k = 0; k < kCopyRows; ++k) if (k < nr) dp[(size_t)k * dst_stride] = v[k];
+}
+
+// one thread per destination: records bad pairs and settles the statistics of the destinations that will be replaced
+__global__ void k_copy_envs_fold(Dev D, const int32_t* __restrict__ src_of_dst, int n_src, int same_handle, double* sret,
+                                 double* scost, double* sn, double* acc) {
+  const int j = blockIdx.x * blockDim.x + threadIdx.x;
+  if (j < D.n) copy_env_source(D, src_of_dst, j, n_src, same_handle != 0, true, sret, scost, sn, acc);
+}
+
+__global__ void __launch_bounds__(kCopyThreads) k_copy_envs(Dev D, CopyFields F, const int32_t* __restrict__ src_of_dst,
+                                                            int n_src, int src_stride, int same_handle) {
+  const int j = blockIdx.x * kCopyThreads + threadIdx.x;
+  if (j >= D.n) return;
+  int f = 0, c = blockIdx.y;
+  for (; f < SAG_NUM_FIELDS - 1; ++f) {
+    const int nc = (F.rows[f] + kCopyRows - 1) / kCopyRows;
+    if (c < nc) break;
+    c -= nc;
+  }
+  const int r0 = c * kCopyRows, nr = min(kCopyRows, F.rows[f] - r0);
+  const int s = copy_env_source(D, src_of_dst, j, n_src, same_handle != 0, false, nullptr, nullptr, nullptr, nullptr);
+  if (s < 0) return;
+  if (F.elem[f] == 8) copy_rows<unsigned long long>(F.dst[f], F.src[f], r0, nr, D.stride, src_stride, j, s);
+  else if (F.elem[f] == 4) copy_rows<unsigned>(F.dst[f], F.src[f], r0, nr, D.stride, src_stride, j, s);
+  else copy_rows<unsigned char>(F.dst[f], F.src[f], r0, nr, D.stride, src_stride, j, s);
+}
+
 // per-task statistic reduction: out[task][3] += (sum return, sum cost, episodes) of finished episodes
 __global__ void k_task_stats(Dev D, const double* sret, const double* scost, const double* sn, double* out) {
   __shared__ double acc[SAG_NUM_TASKS][3];
@@ -777,6 +833,57 @@ int sag_bound(void* handle, double* bound, void* stream) {
   return 0;
 }
 
+static int copy_envs_check(const Handle* D, const Handle* S, const char* who) {
+  if (!D || !S) { snprintf(g_err, sizeof(g_err), "%s: null handle", who); return 1; }
+  if (D->device != S->device) { snprintf(g_err, sizeof(g_err), "%s: the handles are on different devices", who); return 1; }
+  if (const char* what = copy_incompatibility(D->D, S->D)) {
+    snprintf(g_err, sizeof(g_err), "%s: the handles differ in %s", who, what);
+    return 1;
+  }
+  return 0;
+}
+
+static int launch_copy_envs(Handle* H, const Handle* S, const int32_t* src_of_dst, cudaStream_t s) {
+  CopyFields F;
+  for (int f = 0; f < SAG_NUM_FIELDS; ++f) {
+    F.dst[f] = (char*)H->field_ptr[f]; F.src[f] = (const char*)S->field_ptr[f];
+    F.rows[f] = kFieldShape[f].rows; F.elem[f] = kFieldShape[f].elem;
+  }
+  const int blocks = (H->D.n + kCopyThreads - 1) / kCopyThreads;
+  k_copy_envs_fold<<<blocks, kCopyThreads, 0, s>>>(H->D, src_of_dst, S->D.n, H == S, H->sret, H->scost, H->sn, H->stats_acc);
+  ++H->launches;
+  CK(cudaGetLastError());
+  k_copy_envs<<<dim3(blocks, copy_chunks()), kCopyThreads, 0, s>>>(H->D, F, src_of_dst, S->D.n, S->D.stride, H == S);
+  ++H->launches;
+  CK(cudaGetLastError());
+  return 0;
+}
+
+int sag_copy_envs(void* dst, void* src, const int32_t* src_of_dst, void* stream) {
+  Handle *H = (Handle*)dst, *S = (Handle*)src;
+  if (!src_of_dst) return fail("sag_copy_envs: null argument");
+  if (copy_envs_check(H, S, "sag_copy_envs")) return 1;
+  DevGuard guard(H->device);
+  // the pairs are checked in the kernel (copy_env_source): bad ones are not applied and set SAG_ERR_BAD_ENV_INDEX
+  return launch_copy_envs(H, S, src_of_dst, (cudaStream_t)stream);
+}
+
+int sag_copy_envs_host(void* dst, void* src, const int32_t* src_of_dst_host) {
+  Handle *H = (Handle*)dst, *S = (Handle*)src;
+  if (!src_of_dst_host) return fail("sag_copy_envs_host: null argument");
+  if (copy_envs_check(H, S, "sag_copy_envs_host")) return 1;
+  if (const char* what = copy_index_error(src_of_dst_host, H->D.n, S->D.n, H == S)) {
+    snprintf(g_err, sizeof(g_err), "sag_copy_envs_host: %s", what);
+    return 1;
+  }
+  DevGuard guard(H->device);
+  CK(cudaDeviceSynchronize());  // the host API is ordered after everything issued through the stream API
+  CK(cudaMemcpyAsync(H->ids_d, src_of_dst_host, (size_t)H->D.n * sizeof(int32_t), cudaMemcpyHostToDevice, H->own_stream));
+  if (launch_copy_envs(H, S, H->ids_d, H->own_stream)) return 1;
+  CK(cudaStreamSynchronize(H->own_stream));
+  return 0;
+}
+
 int sag_bound_host(void* handle, double* bound_host) {
   Handle* H = (Handle*)handle;
   if (!H || !bound_host) return fail("sag_bound_host: null argument");
@@ -792,7 +899,8 @@ int sag_error_flags(void* handle, int clear) {
   int w = 0;
   if (H->err_h[0]) w |= SAG_FLAG_RESAMPLE_FAILED;
   if (H->err_h[1]) w |= SAG_ERR_BAD_TASK_ID;
-  if (clear) { H->err_h[0] = 0; H->err_h[1] = 0; }
+  if (H->err_h[2]) w |= SAG_ERR_BAD_ENV_INDEX;
+  if (clear) { H->err_h[0] = 0; H->err_h[1] = 0; H->err_h[2] = 0; }
   return w;
 }
 

@@ -26,17 +26,25 @@ struct SlabLayout {
   size_t stats_off, sched_off, act_off, obs_off, rew_off, cost_off, done_off, acc_off, ids_off, mask_off, total;
 };
 
+// The per-environment shape of every state field: rows of `elem`-byte elements, each row `stride` elements long
+// (field[row][env]).  The one list of the fields: the slab is carved from it, and sag_copy_envs copies every row it
+// names, so a field added here is carried by a copy without touching the kernel.
+struct FieldShape { int rows, elem; };
+constexpr FieldShape kFieldShape[SAG_NUM_FIELDS] = {
+    {6, 8},                          // SAG_F_ROBOT
+    {6 * SAG_MAX_SLOTS, 8},          // SAG_F_OBJECTS
+    {15, 8},                         // SAG_F_TASK_F64
+    {10, 4},                         // SAG_F_TASK_I32
+    {1, 1},                          // SAG_F_FLAGS
+    {6, 8},                          // SAG_F_ROBOT_EXT
+    {2 + 3 * SAG_MAX_GREMLINS, 8},   // SAG_F_GREMLINS
+    {1, 4},                          // SAG_F_NEXT_TASK: not bound into Dev, the reset kernels take it as an argument
+};
+
 inline SlabLayout slab_layout(int n, int stride, int obs_dim) {
   SlabLayout L;
   const size_t st = (size_t)stride;
-  L.bytes[SAG_F_ROBOT] = 6 * st * sizeof(double);
-  L.bytes[SAG_F_OBJECTS] = 6 * (size_t)SAG_MAX_SLOTS * st * sizeof(double);
-  L.bytes[SAG_F_TASK_F64] = 15 * st * sizeof(double);
-  L.bytes[SAG_F_TASK_I32] = 10 * st * sizeof(int32_t);
-  L.bytes[SAG_F_FLAGS] = st;
-  L.bytes[SAG_F_ROBOT_EXT] = 6 * st * sizeof(double);
-  L.bytes[SAG_F_GREMLINS] = (2 + 3 * (size_t)SAG_MAX_GREMLINS) * st * sizeof(double);
-  L.bytes[SAG_F_NEXT_TASK] = st * sizeof(int32_t);  // not bound into Dev: the reset kernels take it as an argument
+  for (int f = 0; f < SAG_NUM_FIELDS; ++f) L.bytes[f] = (size_t)kFieldShape[f].rows * kFieldShape[f].elem * st;
   size_t total = 0;
   for (int f = 0; f < SAG_NUM_FIELDS; ++f) { L.off[f] = total; total += align_up(L.bytes[f], 256); }
   L.stats_off = total; total += align_up(3 * st * sizeof(double), 256);
@@ -95,6 +103,38 @@ inline void dev_from_config(Dev& D, const SagConfig& c) {
   D.seed = c.seed; D.gid_base = c.env_id_base;  // (the library also writes the key into the slab: sag_create)
   D.max_layout_draws = c.max_layout_draws; D.max_episode_steps = c.max_episode_steps;
   D.num_gremlins = c.num_gremlins; D.gremlins_travel = c.gremlins_travel;
+}
+
+// sag_copy_envs: two handles whose environments can exchange states -- every configuration value that the layout
+// samplers or the step read from Dev, except the Philox key, the global ids and the per-handle budgets (n_envs,
+// max_episode_steps, max_layout_draws, action_noise).  Returns the first difference, or nullptr.
+inline const char* copy_incompatibility(const Dev& a, const Dev& b) {
+  if (a.robot != b.robot) return "robot";
+  if (a.num_gremlins != b.num_gremlins) return "num_gremlins";
+  if (a.hazards_size != b.hazards_size || a.vases_size != b.vases_size || a.pillars_size != b.pillars_size ||
+      a.gremlins_size != b.gremlins_size)
+    return "object size";
+  if (a.k_hazard != b.k_hazard || a.k_vase != b.k_vase || a.k_gremlin != b.k_gremlin || a.k_pillar != b.k_pillar)
+    return "keepout";
+  if (a.placements_margin != b.placements_margin) return "placements_margin";
+  if (a.robot_keepout != b.robot_keepout) return "robot_keepout";
+  if (a.gremlins_travel != b.gremlins_travel) return "gremlins_travel";
+  if (a.ctrl_range_scale != b.ctrl_range_scale) return "robot_ctrl_range_scale";
+  if (a.random_bound != b.random_bound) return "random_bound";
+  if (a.max_bound != b.max_bound) return "max_bound";
+  return nullptr;
+}
+
+// sag_copy_envs_host: the checks the device path makes per pair (copy_env_source), for a whole host index array, so
+// that a bad array fails the call instead of being reported afterwards.  Returns nullptr or the message.
+inline const char* copy_index_error(const int32_t* src_of_dst, int n_dst, int n_src, bool same_handle) {
+  for (int j = 0; j < n_dst; ++j) {
+    const int s = src_of_dst[j];
+    if (s < -1 || s >= n_src) return "source index out of range [-1, source n_envs)";
+    if (same_handle && s >= 0 && s != j && src_of_dst[s] != -1 && src_of_dst[s] != s)
+      return "a source environment is itself overwritten by the same call";
+  }
+  return nullptr;
 }
 
 }  // namespace sag

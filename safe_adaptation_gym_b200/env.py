@@ -190,6 +190,9 @@ class BatchedSafeAdaptationGym:
             raise ResamplingError('Failed to generate goal' if where == 'step' else 'Failed to generate layout')  # go_to_goal.py:80 / world.py:189
         if w & _abi.ERR_BAD_TASK_ID:
             raise ValueError('task id out of range')
+        if w & _abi.ERR_BAD_ENV_INDEX:
+            raise IndexError('copy_envs: a source index was out of range or named an environment the same call '
+                             'overwrites; those pairs were not applied')
 
     def step(self, action):
         """safe_adaptation_gym.py:56-83.  `action`: [N, 2] tensor / array in [-1, 1].
@@ -341,6 +344,108 @@ class BatchedSafeAdaptationGym:
             ids = torch.tensor([-1 if t is None else t.task_id for t in task_list], dtype=torch.int32).to(self.device)
         self._lib.check(self._lib.L.sag_set_next_tasks(self._h, self._p(ids), self._stream()))
         self._next_armed = True
+
+    def _copy_world(self) -> dict:
+        """The configuration two batches must share for their environments to exchange states, as the library compares
+        it (sag_layout.h: copy_incompatibility): a keepout counts as the larger of it and its object's size
+        (world.py:60-66)."""
+        c = self.base_config
+        w = {'robot': self.robot_name, 'num_gremlins': int(c.get('num_gremlins', 0)), 'random_bound': bool(c['random_bound'])}
+        for k in ('placements_margin', 'robot_keepout', 'gremlins_travel', 'robot_ctrl_range_scale', 'max_bound'):
+            w[k] = float(c[k])
+        for kind in ('hazards', 'vases', 'pillars', 'gremlins'):
+            w[kind + '_size'] = float(c[kind + '_size'])
+            w[kind + '_keepout (effective)'] = max(float(c[kind + '_keepout']), float(c[kind + '_size']))
+        return w
+
+    def copy_envs(self, index, source=None):
+        """Give environments of this batch the complete state of environments of `source` (default: this batch).
+
+        `index` has one entry per environment j of this batch: j takes the state of environment index[j] of `source`,
+        -1 leaves j untouched.  So K copies of each of N environments of `env` into a planning batch of N*K is
+        ``plan.copy_envs(torch.arange(N * K, device=dev, dtype=torch.int32) // K, source=env)``.  `index` is an int32
+        tensor [num_envs] on this env's device (stream-ordered, may be recorded in a CUDA graph) or a host sequence /
+        ndarray / tensor (validated here; raises ``RuntimeError`` under capture).
+
+        What a copy carries: every state field (robot, objects, task state and id, flags, car extras, gremlins, the
+        queued next task), bit for bit, with the episode number and the in-step draw counter.  What it does not: the
+        Philox key and the global environment id -- the copy draws its action noise and its goal, button and radius
+        resamples from THIS batch's streams.  So with the same seed and an ``env_id_base`` that gives a copy its
+        source's global id, the copy replays the source exactly (through goal resamples, auto-resets and queued task
+        switches); with another global id it follows the source until its first in-step draw.
+
+        Statistics (``task_stats``): the destination's own episode is settled as a reset settles it -- one that has
+        finished (time limit or done) but has not been reset yet counts under its old task, an unfinished one is dropped;
+        its earlier finished episodes stay with its old task; the copied episode, with the return and cost it has gathered so far, is
+        credited to this batch in full when it finishes.
+
+        Within one batch a pair j <- s (s != j) is applied only if s is not itself overwritten by the same call
+        (index[s] is -1 or s); j <- j does nothing.  Host input breaking that rule, of the wrong length or dtype raises
+        ``ValueError``, an index outside [-1, source.num_envs) ``IndexError``.  On a device tensor such pairs are not
+        applied and raise ``IndexError`` at the next call that checks errors (``step``, ``check_errors``).
+
+        The two batches must be on the same device and share robot, gremlins, object sizes, keepouts, placement margins,
+        gremlin travel, ctrl-range scale and the bound settings (``ValueError`` otherwise); they may differ in
+        num_envs, seed, env_id_base, max_episode_steps, max_layout_draws and action_noise -- a noise-free planning
+        batch without a time limit is the intended use.  A copy may bring ``Unsupervised`` (whose reward is a pair)
+        into this batch only if its ``step`` already records the pair: host input checks the copied environments, a
+        device tensor is refused whenever `source` records the pair and this batch does not."""
+        src = self if source is None else source
+        self._check_copy_source(src)
+        on_device = (torch.is_tensor(index) and index.device.type == self.device.type
+                     and (index.device.index or 0) == (self.device.index or 0))
+        if on_device:
+            if index.dtype != torch.int32 or tuple(index.shape) != (self.num_envs,):
+                raise ValueError(f'need an int32 tensor of shape ({self.num_envs},), got {index.dtype} {tuple(index.shape)}')
+            if src._any_unsupervised and not self._any_unsupervised:
+                raise ValueError("the source batch records Unsupervised's reward pair and this batch does not: a copy "
+                                 'could bring Unsupervised in (set_task it here first)')
+            idx = index.contiguous()
+        else:
+            if _capturing():
+                raise RuntimeError('under CUDA graph capture copy_envs needs an int32 tensor of indices on the env\'s '
+                                   f'device ({self.device}); a host sequence would record a copy from pageable memory')
+            raw = np.asarray(index.cpu() if torch.is_tensor(index) else index)
+            if raw.shape != (self.num_envs,):
+                raise ValueError(f'need {self.num_envs} source indices, got shape {raw.shape}')
+            if raw.dtype.kind not in 'iu':
+                raise ValueError(f'source indices must be integers, got {raw.dtype}')
+            raw = raw.astype(np.int64)
+            bad = raw[(raw < -1) | (raw >= src.num_envs)]
+            if bad.size:
+                raise IndexError(f'source index {int(bad[0])} out of range [-1, {src.num_envs})')
+            if src is self:
+                j = np.nonzero((raw >= 0) & (raw != np.arange(self.num_envs)))[0]
+                t = raw[raw[j]]
+                clash = (t != -1) & (t != raw[j])
+                if clash.any():
+                    k = int(j[clash][0])
+                    raise ValueError(f'environment {k} copies environment {int(raw[k])}, which the same call overwrites')
+            if not self._any_unsupervised:
+                used = torch.as_tensor(raw[raw >= 0], device=src.device)
+                unsup = _tasks.Unsupervised.task_id
+                if bool((src.task_ids[used] == unsup).any() | (src.get_field('next_task')[used] == unsup).any()):
+                    raise ValueError("a copied environment runs or has queued Unsupervised, whose reward is a pair that "
+                                     'this batch\'s step does not record: set_task it here first')
+            idx = torch.as_tensor(raw, dtype=torch.int32).to(self.device)
+        self._lib.check(self._lib.L.sag_copy_envs(self._h, src._h, self._p(idx), self._stream()))
+        self._next_armed = self._next_armed or src._next_armed   # copies carry queued next tasks
+        if self.base_config['random_bound']:
+            # the copies carry their source's bound draw; in place: a CUDA graph may export it
+            self._lib.check(self._lib.L.sag_bound(self._h, self._p(self._bound), self._stream()))
+        if not on_device:
+            self._tasks_from_ids(self.task_ids.cpu())
+
+    def _check_copy_source(self, src):
+        if not isinstance(src, BatchedSafeAdaptationGym):
+            raise TypeError(f'source must be a BatchedSafeAdaptationGym, got {type(src).__name__}')
+        same_device = (src.device.type, src.device.index or 0) == (self.device.type, self.device.index or 0)
+        if src._lib is not self._lib or not same_device:
+            raise ValueError(f'the source batch runs on another device or library ({src.device} != {self.device})')
+        mine, theirs = self._copy_world(), src._copy_world()
+        for k, v in mine.items():
+            if theirs[k] != v:
+                raise ValueError(f'the batches differ in {k}: {theirs[k]!r} != {v!r}')
 
     @property
     def task_ids(self) -> torch.Tensor:
