@@ -18,8 +18,8 @@
  *
  * CUDA graphs.  These stream entry points may be recorded in a CUDA graph (stream capture) and the graph replayed any
  * number of times: sag_step, sag_reset_obs / sag_reset with a mask or only_flagged != 0, sag_export_outputs,
- * sag_observe, sag_rollout, sag_read_field / sag_write_field, sag_task_stats, sag_set_next_tasks, sag_bound and
- * sag_copy_envs.  A replay
+ * sag_observe, sag_rollout, sag_read_field / sag_write_field, sag_task_stats, sag_set_next_tasks, sag_bound,
+ * sag_copy_envs and sag_evaluate_actions.  A replay
  * behaves exactly like issuing the same calls again: everything the kernels read that can change after sag_create (the
  * work-list counter sets and the step epoch that selects them, the Philox key, the task ids, the queued next tasks)
  * lives in the handle's device memory, so sag_seed and sag_set_tasks issued between replays are seen by the graph.  The
@@ -217,6 +217,23 @@ int sag_probe_d2h(void* handle, size_t bytes, int reps, double* seconds);
  * a step needs a single device-to-host copy; free with sag_host_free(*obs_h) */
 int sag_host_alloc_outputs(void* handle, float** obs_h, double** reward_h, uint8_t** cost_h, uint8_t** done_h);
 void sag_host_free(void* p);
+
+/* Score a horizon of actions: h_steps >= 1 steps with act[h] (DEVICE float[h_steps][n][2]), enqueued in one call:
+ * h_steps x (the two step kernels).  Every environment takes all h_steps steps, exactly as h_steps sag_step calls with
+ * act[0], act[1], ... would take them: afterwards every SAG_F_* field, the statistics and the Philox draw counters are
+ * bit-identical to theirs (sag_step does not reset; neither does this call, also with a time limit).  Outputs, DEVICE:
+ *   obs     float[n][obs_dim]: the observation of the last step (bit-identical to the last sag_step's);
+ *   ret     double[n] (ret_cols = 1) or double[n][2] (ret_cols = 2, Unsupervised's pair, as sag_step's reward2);
+ *   cost    double[n];  length  int32[n].
+ * With w_0 = 1, w_{h+1} = w_h * discount (float64, formed on the host left to right) and L_e = min(h_steps, 1 + the
+ * first step at which environment e reported done -- a physics error):
+ *   ret[e] = sum over h < L_e of w_h * reward_h[e], cost[e] = the same with the binary step cost, length[e] = L_e,
+ * each product rounded before it is added, summed in step order from zero.  With discount = 1 that is the sum a loop
+ * `ret += reward` over sag_step calls forms, stopped at the first done.  Steps after L_e still run but do not count.
+ * Only the last step builds the observation: the steps before it skip the lidar, the sensors and the observation
+ * write-out.  Stream-ordered; may be recorded in a CUDA graph (h_steps and discount are fixed by the capture). */
+int sag_evaluate_actions(void* handle, int h_steps, const float* act, double discount, float* obs, double* ret, int ret_cols,
+                         double* cost, int32_t* length, void* stream);
 
 /* The outputs of a step as fresh arrays in one launch (device pointers): obs rows, reward (reward_cols = 1, or 2 for the
  * Unsupervised task's pair), cost as float32 -- the reference returns float(cost > 0.), world.py:155 --, done as bool bytes,

@@ -45,7 +45,7 @@ class SagLib:
         "sag_set_next_tasks", "sag_set_next_tasks_host", "sag_bound", "sag_copy_envs", "sag_copy_envs_host",
         "sag_error_flags", "sag_reset_obs", "sag_reset_host", "sag_seed", "sag_reset", "sag_step", "sag_observe",
         "sag_step_host", "sag_observe_host", "sag_host_alloc", "sag_host_alloc_outputs", "sag_probe_d2h", "sag_host_free", "sag_rollout", "sag_read_field",
-        "sag_write_field", "sag_task_stats", "sag_lidar", "sag_cost", "sag_export_outputs",
+        "sag_write_field", "sag_task_stats", "sag_lidar", "sag_cost", "sag_export_outputs", "sag_evaluate_actions",
     ]
 
     def __init__(self, path, host_api=True):
@@ -77,6 +77,8 @@ class SagLib:
         if hasattr(L, "sag_copy_envs"):
             L.sag_copy_envs.argtypes = [vp, vp, vp, vp]
             L.sag_copy_envs_host.argtypes = [vp, vp, vp]
+        if hasattr(L, "sag_evaluate_actions"):
+            L.sag_evaluate_actions.argtypes = [vp, i32, fp, C.c_double, fp, dp, i32, dp, vp, vp]
         L.sag_seed.argtypes = [vp, C.c_uint64]
         L.sag_error_flags.argtypes = [vp, i32]
         L.sag_reset_obs.argtypes = [vp, u8p, i32, i32, fp, u8p, vp]

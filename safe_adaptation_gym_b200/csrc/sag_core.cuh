@@ -1993,8 +1993,8 @@ __device__ __forceinline__ void coop_lidar_apply(const LidarHit& H, float* bins,
   atomicMax(reinterpret_cast<int*>(bins + bp * bstride), __float_as_int(H.sp));
   atomicMax(reinterpret_cast<int*>(bins + bm * bstride), __float_as_int(H.sm));
 }
-// pass A of end_of_step with one object per lane: obstacle lidar, hazard flag, min squared distances per kind
-template <class RB>
+// pass A of end_of_step with one object per lane: obstacle lidar (Obs), hazard flag, min squared distances per kind
+template <class RB, bool Obs = true>
 __device__ __forceinline__ void pass_a_coop(const Ctx& C, const RB& R, double cs, double sn, float* obs_s, int ostride, bool& hz,
                                             double& d2v, double& d2p, double& d2b, double& d2x) {
   const Dev& D = C.D;
@@ -2010,7 +2010,7 @@ __device__ __forceinline__ void pass_a_coop(const Ctx& C, const RB& R, double cs
       if (s < C.L.v0) hzl = hazard_hit(d2, D.hazards_size);
       else if (s < C.L.p0) lv = d2;
       else lp = d2;
-      coop_lidar_apply(lidar_eval(wx, wy, cs, sn), obs_s, ostride);
+      if constexpr (Obs) coop_lidar_apply(lidar_eval(wx, wy, cs, sn), obs_s, ostride);
     } else {
       int kind = slot_kind(C.sp, C.L, s);
       if (kind_collidable(kind)) { if (kind == K_BUTTON) lb = d2; else lx = d2; }
@@ -2022,7 +2022,10 @@ __device__ __forceinline__ void pass_a_coop(const Ctx& C, const RB& R, double cs
 }
 #endif
 
-template <int Mode, class RB>
+// Obs = false (sag_evaluate_actions' steps before the last): no observation.  obs_s is not touched -- no zeroing, no
+// lidar, no pass B, no sensors -- and everything that feeds the state, the reward, the cost or the clearance is computed
+// as with Obs = true, in the same order.
+template <int Mode, class RB, bool Obs = true>
 SAG_HD void end_of_step(unsigned wmask, Scratch* S, const SolveConsts& Q, const Ctx& C, const RB& R, TaskState& T, const Rng& rng, const PtConst& K,
                         unsigned mov, bool phys_err, const double* qacc_err, bool with_reward, float* obs_s, int ostride, EndOut& O,
                         const Phys* Pfwd = nullptr, unsigned cand = 0xffffffffu, const double* mocap = nullptr) {
@@ -2033,15 +2036,25 @@ SAG_HD void end_of_step(unsigned wmask, Scratch* S, const SolveConsts& Q, const 
   SAG_CLK_DECL;
   double sn, cs;
   sag_sincos(R.q[2], &sn, &cs);
-  for (int k = 0; k < 48; ++k) obs_s[k * ostride] = 0.0f;
+  if constexpr (Obs) for (int k = 0; k < 48; ++k) obs_s[k * ostride] = 0.0f;
   // ---- pass A: hazards / vases / gremlins / pillars -> obstacle lidar, hazard cost, clearance
   bool hz = false;
   double d2v = 1e300, d2p = 1e300, d2b = 1e300, d2x = 1e300;  // min squared centre distance per collidable kind
   if constexpr (Coop) {
 #if defined(__CUDA_ARCH__)
-    pass_a_coop(C, R, cs, sn, obs_s, ostride, hz, d2v, d2p, d2b, d2x);
+    pass_a_coop<RB, Obs>(C, R, cs, sn, obs_s, ostride, hz, d2v, d2p, d2b, d2x);
 #endif
   } else {
+  if constexpr (!Obs) {  // the distances and the hazard flag alone
+    for (int s = 0; s < C.L.t0; ++s) {
+      size_t i = oix(C, s);
+      double wx = C.O.x[i] - R.q[0], wy = C.O.y[i] - R.q[1];
+      double d2 = wx * wx + wy * wy;
+      if (s < C.L.v0) hz = hz || hazard_hit(d2, D.hazards_size);
+      else if (s < C.L.p0) { if (d2 < d2v) d2v = d2; }
+      else { if (d2 < d2p) d2p = d2; }
+    }
+  } else
   // obstacle slots [0, t0) in trips of three: loads and the sqrt / atan2 chains of a trip are independent, the
   // shared-memory bin updates come last (the compiler has to keep those in order)
   for (int s0 = 0; s0 < C.L.t0; s0 += 3) {
@@ -2149,6 +2162,10 @@ SAG_HD void end_of_step(unsigned wmask, Scratch* S, const SolveConsts& Q, const 
       O.cost = (hz || (touch & obstacle_mask)) ? 1.0 : 0.0;                  // :78, world.py:144-155
     }
   }
+  if constexpr (!Obs) {
+    if constexpr (Coop) SAG_CLK(9);
+    return;
+  }
   // ---- pass B: task objects -> objects / goal lidar (safe_adaptation_gym.py:133-139, world.py:219-231)
   if constexpr (Coop) {
 #if defined(__CUDA_ARCH__)
@@ -2227,7 +2244,8 @@ SAG_HD bool env_is_quiet(double clear, const RB& R) { return clear > R.travel_bo
 // ------------------------------------------------------------------------------------------------
 // SafeAdaptationGym.step for one environment (safe_adaptation_gym.py:56-83)
 // ------------------------------------------------------------------------------------------------
-template <int Mode, class RB>
+// Obs = false: the step without its observation (end_of_step); obs_s is not touched
+template <int Mode, class RB, bool Obs = true>
 SAG_HD int env_step(unsigned wmask, Scratch* S, const Dev& D, int e, float a0, float a1, float* obs_s, int ostride, double* reward2,
                      unsigned char* cost, unsigned char* done, bool pretest = true) {
   constexpr bool Coop = Mode == kStepCoop, Near = Mode == kStepNear;
@@ -2415,7 +2433,7 @@ SAG_HD int env_step(unsigned wmask, Scratch* S, const Dev& D, int e, float a0, f
     if constexpr (Coop) SAG_CLK(6);
   }
   EndOut O;
-  end_of_step<Mode, RB>(wmask, S, Q, C, R, T, rng, K, mov, err != 0, qacc_err, true, obs_s, ostride, O, Coop ? &Pfwd : nullptr, cand, moc_new);
+  end_of_step<Mode, RB, Obs>(wmask, S, Q, C, R, T, rng, K, mov, err != 0, qacc_err, true, obs_s, ostride, O, Coop ? &Pfwd : nullptr, cand, moc_new);
   if constexpr (Coop) SAG_CLK_RESET;
   if constexpr (Near) { if (O.bail) return 1; }
   unsigned char dn = 0;
@@ -2457,6 +2475,51 @@ SAG_HD int env_step(unsigned wmask, Scratch* S, const Dev& D, int e, float a0, f
   *done = dn;
   if constexpr (Coop) SAG_CLK(10);
   return 0;
+}
+
+// ------------------------------------------------------------------------------------------------
+// sag_evaluate_actions: return, cost and length over a horizon of H steps, accumulated by the step kernels where a step
+// stores reward / cost / done.  Every environment is finished by exactly one kernel per step, so nothing races.
+//   L_e = min(H, 1 + first step that reported done); ret += w_h r_h and cost += w_h c_h for h < L_e, each product
+//   rounded before the sum (no FMA), in step order.
+// Step 0 writes the accumulators (0 + w_0 r_0: a sum that starts at zero) instead of reading them, so no memset is
+// needed.  While an environment still counts, its length holds minus the steps counted so far; a done, or the last
+// step, stores the final (positive) length.
+// ------------------------------------------------------------------------------------------------
+struct EvalAcc {
+  double* ret;      // [n] or [n][2] (Unsupervised's pair)
+  double* cost;     // [n]
+  int32_t* length;  // [n]
+  double w;         // this step's weight
+  int cols, first, last;
+};
+
+SAG_HD double mul_rn(double a, double b) {
+#if defined(__CUDA_ARCH__)
+  return __dmul_rn(a, b);
+#else
+  return a * b;  // (the host build has -ffp-contract=off)
+#endif
+}
+SAG_HD double add_rn(double a, double b) {
+#if defined(__CUDA_ARCH__)
+  return __dadd_rn(a, b);
+#else
+  return a + b;
+#endif
+}
+
+SAG_HD void eval_accumulate(const EvalAcc& A, int e, const double* rew, unsigned char c, unsigned char d) {
+  if (!A.first && A.length[e] >= 0) return;  // ended by a done at an earlier step
+  const int k = A.first ? 1 : 1 - A.length[e];
+  if (A.cols == 2) {
+    A.ret[2 * e] = add_rn(A.first ? 0.0 : A.ret[2 * e], mul_rn(A.w, rew[0]));
+    A.ret[2 * e + 1] = add_rn(A.first ? 0.0 : A.ret[2 * e + 1], mul_rn(A.w, rew[1]));
+  } else {
+    A.ret[e] = add_rn(A.first ? 0.0 : A.ret[e], mul_rn(A.w, rew[0]));
+  }
+  A.cost[e] = add_rn(A.first ? 0.0 : A.cost[e], mul_rn(A.w, c ? 1.0 : 0.0));
+  A.length[e] = (d || A.last) ? k : -k;
 }
 
 // observation at the current state (reset return value / refresh after state injection)

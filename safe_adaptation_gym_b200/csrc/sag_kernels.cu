@@ -141,14 +141,21 @@ __device__ __forceinline__ void write_rows(const float* tile, int tstride, float
 // Nothing the host does between steps selects a set, so a step recorded in a CUDA graph behaves on every replay like a
 // step issued anew, with no memset node per step.
 
+// What a step kernel does with a step's outputs.  kOutStep: sag_step -- the observation, reward, cost and done.  The
+// other two are the steps of sag_evaluate_actions: the epilogue adds the weighted reward and cost into the horizon's
+// sums (sag_core.cuh: eval_accumulate) instead of storing them, and only the last step of the horizon (kOutAccumObs)
+// builds and writes the observation; the ones before it (kOutAccum) skip the lidar, the sensors and the tile write-out.
+constexpr int kOutStep = 0, kOutAccum = 1, kOutAccumObs = 2;
+
 // __launch_bounds__(kBS, 4): 4 CTAs / SM (<= 128 registers) so that the whole 65,536-env point batch is one wave.  The car's
 // contact-free step carries the two wheel-row pairs of its friction solve through ten substeps x ten sweeps: it needs
 // the registers more than the occupancy (32,768 envs are 7 warps / SM), so it gets 2 CTAs / SM and no spills.
-template <class RB>
+template <class RB, int Out = kOutStep>
 __global__ void __launch_bounds__(kBS, RB::kKind == 1 ? 2 : 4) k_step_free(Dev D, const float* __restrict__ act, float* __restrict__ obs,
                                                     double* __restrict__ reward, double* __restrict__ reward2,
-                                                    uint8_t* __restrict__ cost, uint8_t* __restrict__ done) {
+                                                    uint8_t* __restrict__ cost, uint8_t* __restrict__ done, EvalAcc A) {
   constexpr int kObs = RB::kObsDim;
+  constexpr bool Obs = Out != kOutAccum;  // kOutAccum: no tile in shared memory
   extern __shared__ __align__(16) unsigned char smem_raw[];
   float* tile = reinterpret_cast<float*>(smem_raw);  // [kObs][kTileStride]
   const int e = blockIdx.x * kBS + threadIdx.x;
@@ -167,12 +174,16 @@ __global__ void __launch_bounds__(kBS, RB::kKind == 1 ? 2 : 4) k_step_free(Dev D
     float2 a = reinterpret_cast<const float2*>(act)[e];
     double rew[2];
     unsigned char c, d;
-    bail = env_step<kStepNear, RB>(0u, nullptr, D, e, a.x, a.y, tile + threadIdx.x, kTileStride, rew, &c, &d, pretest) != 0;
+    bail = env_step<kStepNear, RB, Obs>(0u, nullptr, D, e, a.x, a.y, tile + threadIdx.x, kTileStride, rew, &c, &d, pretest) != 0;
     if (!bail) {
-      reward[e] = rew[0];
-      if (reward2) { reward2[2 * e] = rew[0]; reward2[2 * e + 1] = rew[1]; }
-      cost[e] = c;
-      done[e] = d;
+      if constexpr (Out == kOutStep) {
+        reward[e] = rew[0];
+        if (reward2) { reward2[2 * e] = rew[0]; reward2[2 * e + 1] = rew[1]; }
+        cost[e] = c;
+        done[e] = d;
+      } else {
+        eval_accumulate(A, e, rew, c, d);
+      }
     }
   }
   // work list append, one atomic per warp
@@ -186,8 +197,10 @@ __global__ void __launch_bounds__(kBS, RB::kKind == 1 ? 2 : 4) k_step_free(Dev D
   }
   // all kBS rows of the CTA in one coalesced sweep.  The columns of the work-list environments hold stale shared memory:
   // their rows are rewritten by the cooperative kernel, which always runs after this one on the same stream.
-  __syncthreads();
-  write_tile4<kObs>(tile, obs, blockIdx.x * kBS, D.n);
+  if constexpr (Obs) {
+    __syncthreads();
+    write_tile4<kObs>(tile, obs, blockIdx.x * kBS, D.n);
+  }
 }
 
 // k_step_coop: the work list with ONE WARP per environment (sag_core.cuh "warp-cooperative variants"): the lanes run the
@@ -204,11 +217,12 @@ struct CoopCfg {
   static constexpr size_t kSmemBytes = kPerWarp * kCoopWarps;
 };
 
-template <class RB>
+template <class RB, int Out = kOutStep>
 __global__ void __launch_bounds__(32 * kCoopWarps, 1) k_step_coop(const __grid_constant__ Dev D, const float* __restrict__ act,
                                                               float* __restrict__ obs, double* __restrict__ reward,
                                                               double* __restrict__ reward2, uint8_t* __restrict__ cost,
-                                                              uint8_t* __restrict__ done) {
+                                                              uint8_t* __restrict__ done, EvalAcc A) {
+  constexpr bool Obs = Out != kOutAccum;
   extern __shared__ __align__(16) unsigned char smem_raw[];
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   unsigned char* mine = smem_raw + (size_t)warp * CoopCfg<RB>::kPerWarp;
@@ -234,7 +248,7 @@ __global__ void __launch_bounds__(32 * kCoopWarps, 1) k_step_coop(const __grid_c
     float2 a = reinterpret_cast<const float2*>(act)[e];
     double rew[2];
     unsigned char c, d;
-    env_step<kStepCoop, RB>(0xffffffffu, big, D, e, a.x, a.y, tile, 1, rew, &c, &d);
+    env_step<kStepCoop, RB, Obs>(0xffffffffu, big, D, e, a.x, a.y, tile, 1, rew, &c, &d);
 #if defined(SAG_TIMING)
     if (lane == 0) {
       const unsigned long long tot = (unsigned long long)(clock64() - clk_);
@@ -247,13 +261,19 @@ __global__ void __launch_bounds__(32 * kCoopWarps, 1) k_step_coop(const __grid_c
 #endif
     __syncwarp();
     if (lane == 0) {
-      reward[e] = rew[0];
-      if (reward2) { reward2[2 * e] = rew[0]; reward2[2 * e + 1] = rew[1]; }
-      cost[e] = c;
-      done[e] = d;
+      if constexpr (Out == kOutStep) {
+        reward[e] = rew[0];
+        if (reward2) { reward2[2 * e] = rew[0]; reward2[2 * e + 1] = rew[1]; }
+        cost[e] = c;
+        done[e] = d;
+      } else {
+        eval_accumulate(A, e, rew, c, d);
+      }
     }
-    float* dst = obs + (size_t)e * CoopCfg<RB>::kObs;
-    for (int k = lane; k < CoopCfg<RB>::kObs; k += 32) dst[k] = tile[k];
+    if constexpr (Obs) {
+      float* dst = obs + (size_t)e * CoopCfg<RB>::kObs;
+      for (int k = lane; k < CoopCfg<RB>::kObs; k += 32) dst[k] = tile[k];
+    }
     __syncwarp();
   }
   // The last CTA to finish advances the step epoch for the next step's batch kernel (which runs after this kernel) and
@@ -585,6 +605,8 @@ struct Ops {
     cudaError_t ce = cudaFuncSetAttribute(k_observe<RB>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TileCfg<RB>::kSmemBytes);
     if (ce == cudaSuccess) ce = cudaFuncSetAttribute(k_reset<RB, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ResetCfg<RB>::kSmemBytes);
     if (ce == cudaSuccess) ce = cudaFuncSetAttribute(k_step_coop<RB>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CoopCfg<RB>::kSmemBytes);
+    if (ce == cudaSuccess) ce = cudaFuncSetAttribute(k_step_coop<RB, kOutAccum>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CoopCfg<RB>::kSmemBytes);
+    if (ce == cudaSuccess) ce = cudaFuncSetAttribute(k_step_coop<RB, kOutAccumObs>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CoopCfg<RB>::kSmemBytes);
     if (ce != cudaSuccess) return ce;
     // Local memory: the observation and auto-reset kernels carry the scalar contact path (stack frames of ~1.6 KB
     // per thread, above the default 1 KB limit), so the driver would re-size its local-memory pool whenever one of them
@@ -612,11 +634,13 @@ struct Ops {
     if (ce != cudaSuccess) return ce;
     return step_coop(H, act, obs, reward, reward2, cost, done, s);
   }
+  template <int Out = kOutStep>
   static cudaError_t step_free(Handle* H, const float* act, float* obs, double* reward, double* reward2, uint8_t* cost,
-                               uint8_t* done, cudaStream_t s) {
+                               uint8_t* done, cudaStream_t s, const EvalAcc& A = EvalAcc{}) {
     // this step's counter set is zero already (cleared by the previous step's batch kernel, which saves a memset node per
     // step) and the kernels find it from the step epoch on the device; steps of one handle must be stream-ordered
-    k_step_free<RB><<<grid_for(H->D.n), kBS, TileCfg<RB>::kTileBytes, s>>>(H->D, act, obs, reward, reward2, cost, done);
+    const size_t smem = Out == kOutAccum ? 0 : TileCfg<RB>::kTileBytes;
+    k_step_free<RB, Out><<<grid_for(H->D.n), kBS, smem, s>>>(H->D, act, obs, reward, reward2, cost, done, A);
     ++H->launches;
     return cudaGetLastError();
   }
@@ -627,8 +651,9 @@ struct Ops {
     ++H->launches;
     return cudaGetLastError();
   }
+  template <int Out = kOutStep>
   static cudaError_t step_coop(Handle* H, const float* act, float* obs, double* reward, double* reward2, uint8_t* cost, uint8_t* done,
-                               cudaStream_t s) {
+                               cudaStream_t s, const EvalAcc& A = EvalAcc{}) {
     ++H->launches;
     const int need = (H->D.n + kCoopWarps - 1) / kCoopWarps;
     cudaLaunchConfig_t cfg = {};
@@ -641,7 +666,28 @@ struct Ops {
     attr[0].val.programmaticStreamSerializationAllowed = 1;  // hides this launch's latency behind the previous kernel's tail
     cfg.attrs = attr;
     cfg.numAttrs = 1;
-    return cudaLaunchKernelEx(&cfg, k_step_coop<RB>, H->D, act, obs, reward, reward2, cost, done);
+    return cudaLaunchKernelEx(&cfg, k_step_coop<RB, Out>, H->D, act, obs, reward, reward2, cost, done, A);
+  }
+  // sag_evaluate_actions: H x (k_step_free + k_step_coop) with the accumulating epilogue, the observation on the last
+  // step only.  The weights are formed here, left to right in float64, and passed by value.
+  static cudaError_t evaluate(Handle* H, int h_steps, const float* act, double discount, float* obs, double* ret, int ret_cols,
+                              double* cost, int32_t* length, cudaStream_t s) {
+    double w = 1.0;
+    for (int h = 0; h < h_steps; ++h) {
+      const EvalAcc A = {ret, cost, length, w, ret_cols, h == 0, h == h_steps - 1};
+      const float* a = act + (size_t)h * H->D.n * 2;
+      cudaError_t ce;
+      if (h < h_steps - 1) {
+        ce = step_free<kOutAccum>(H, a, nullptr, nullptr, nullptr, nullptr, nullptr, s, A);
+        if (ce == cudaSuccess) ce = step_coop<kOutAccum>(H, a, nullptr, nullptr, nullptr, nullptr, nullptr, s, A);
+      } else {
+        ce = step_free<kOutAccumObs>(H, a, obs, nullptr, nullptr, nullptr, nullptr, s, A);
+        if (ce == cudaSuccess) ce = step_coop<kOutAccumObs>(H, a, obs, nullptr, nullptr, nullptr, nullptr, s, A);
+      }
+      if (ce != cudaSuccess) return ce;
+      w *= discount;
+    }
+    return cudaSuccess;
   }
   static cudaError_t observe(Handle* H, float* obs, cudaStream_t s) {
     k_observe<RB><<<grid_for(H->D.n), kBS, TileCfg<RB>::kSmemBytes, s>>>(H->D, obs);
@@ -957,6 +1003,16 @@ int sag_step(void* handle, const float* act, float* obs, double* reward, double*
   if (!H || !act || !obs || !reward || !cost || !done) return fail("sag_step: null argument");
   DevGuard guard(H->device);
   CK(SAG_DISPATCH(H, step(H, act, obs, reward, reward2, cost, done, (cudaStream_t)stream)));
+  return 0;
+}
+
+int sag_evaluate_actions(void* handle, int h_steps, const float* act, double discount, float* obs, double* ret, int ret_cols,
+                         double* cost, int32_t* length, void* stream) {
+  Handle* H = (Handle*)handle;
+  if (!H || !act || !obs || !ret || !cost || !length || h_steps <= 0 || (ret_cols != 1 && ret_cols != 2))
+    return fail("sag_evaluate_actions: bad argument");
+  DevGuard guard(H->device);
+  CK(SAG_DISPATCH(H, evaluate(H, h_steps, act, discount, obs, ret, ret_cols, cost, length, (cudaStream_t)stream)));
   return 0;
 }
 

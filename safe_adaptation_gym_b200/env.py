@@ -11,7 +11,8 @@ With ``max_episode_steps > 0`` the env auto-resets like a vectorised gym wrapper
 (time limit, or done after a physics error) is reset inside ``step``; its row of ``obs`` is the FIRST observation of the
 new episode, ``done`` is True for it and ``info['truncated']`` marks the time-limit endings.
 
-``step`` (both output modes, with or without auto-reset), ``rollout`` and ``observation`` may be recorded in a CUDA graph
+``step`` (both output modes, with or without auto-reset), ``rollout``, ``observation``, ``copy_envs`` and
+``evaluate_actions`` (with device tensors) may be recorded in a CUDA graph
 (``torch.cuda.graph``), together with the policy that computes the actions; every replay behaves like issuing the same
 calls again.  ``seed``, ``set_task`` and ``load_state_dict`` between replays are seen by the graph, except that a
 ``set_task`` which changes whether any environment runs ``Unsupervised`` changes the reward buffer ``step`` records:
@@ -140,6 +141,8 @@ class BatchedSafeAdaptationGym:
         self._cost = torch.empty((n,), dtype=torch.uint8, device=dev)
         self._done = torch.empty((n,), dtype=torch.uint8, device=dev)
         self._was_reset = torch.zeros((n,), dtype=torch.uint8, device=dev)
+        self._eval_cost = torch.empty((n,), dtype=torch.float64, device=dev)     # evaluate_actions (copy_outputs=False)
+        self._eval_length = torch.empty((n,), dtype=torch.int32, device=dev)
         self._bound = torch.full((n,), float(cfg['max_bound']), dtype=torch.float64, device=dev)
         self._task_ids = None
         self._tasks = None
@@ -238,6 +241,61 @@ class BatchedSafeAdaptationGym:
             done = done | was_reset
         self._raise_recorded_errors('step')
         return obs, rew, done, info
+
+    def evaluate_actions(self, actions, discount: float = 1.0):
+        """Run a horizon of actions and return what a planner scores a candidate by: ``obs, ret, cost, length``.
+
+        `actions`: float32 tensor [H, N, 2] on this env's device, H >= 1.  Every environment takes exactly H steps with
+        ``actions[h]``; afterwards its state (every ``_FIELDS`` field, ``task_stats``, the Philox draw counters) is
+        bit-identical to what H calls of ``step(actions[h])`` leave.  With weights ``w_0 = 1``, ``w_{h+1} = w_h *
+        discount`` (float64, formed left to right) and ``L_e = min(H, 1 + the first h at which step h reported
+        done[e])`` (a physics error):
+
+        - ``obs``: float32 [N, obs_dim], the observation of the last step, bit-identical to the H-th ``step``'s;
+        - ``ret``: float64 [N] (or [N, 2] when this batch records Unsupervised's reward pair, as ``step``),
+          ``sum_{h < L_e} w_h * r_h[e]``, each product rounded and then added, in step order from zero;
+        - ``cost``: float64 [N], the same sum over the binary step cost;
+        - ``length``: int32 [N], ``L_e``.
+
+        With ``discount=1.0`` the sums equal those of a loop ``ret += r; cost += info['cost']`` over H ``step`` calls,
+        stopped at each environment's first done.  Steps after ``L_e`` still run but do not count.  Only the last step
+        builds an observation, so a horizon costs less than H steps.  Outputs follow ``copy_outputs`` like ``step``.
+
+        A batch with ``max_episode_steps > 0`` is refused (``ValueError``): ``step`` would auto-reset in the middle of
+        the horizon.  May be recorded in a CUDA graph (with ``copy_envs`` and the policy or sampler that fills
+        `actions`); H and `discount` are fixed by the capture.  Errors recorded during the call (a goal that could not
+        be resampled) raise as they do for ``step``, and through ``check_errors()`` after replays."""
+        if self.max_episode_steps > 0:
+            raise ValueError('evaluate_actions needs a batch without a time limit (max_episode_steps = 0): step would '
+                             'auto-reset environments in the middle of the horizon')
+        on_device = (torch.is_tensor(actions) and actions.device.type == self.device.type
+                     and (actions.device.index or 0) == (self.device.index or 0))
+        if not on_device:
+            if _capturing():
+                raise RuntimeError('under CUDA graph capture evaluate_actions needs the actions already on the env\'s '
+                                   f'device ({self.device}); a host array would record a copy from pageable memory')
+            raise ValueError(f'actions must be a float32 tensor on {self.device}')
+        if actions.dtype != torch.float32 or actions.dim() != 3 or tuple(actions.shape[1:]) != (self.num_envs, 2) \
+                or actions.shape[0] < 1:
+            raise ValueError(f'need a float32 tensor of shape (H >= 1, {self.num_envs}, 2), got {actions.dtype} '
+                             f'{tuple(actions.shape)}')
+        act = actions.contiguous()
+        n, dev = self.num_envs, self.device
+        cols = 2 if self._any_unsupervised else 1
+        if self.copy_outputs:
+            obs = torch.empty((n, self.obs_dim), dtype=torch.float32, device=dev)
+            ret = torch.empty((n, 2) if cols == 2 else (n,), dtype=torch.float64, device=dev)
+            cost = torch.empty((n,), dtype=torch.float64, device=dev)
+            length = torch.empty((n,), dtype=torch.int32, device=dev)
+        else:  # the internal buffers, valid until the next call
+            obs, cost, length = self._obs, self._eval_cost, self._eval_length
+            ret = self._reward2 if cols == 2 else self._reward
+        L = self._lib
+        L.check(L.L.sag_evaluate_actions(self._h, int(act.shape[0]), self._p(act), C.c_double(float(discount)),
+                                         self._p(obs), self._p(ret), cols, self._p(cost), self._p(length),
+                                         self._stream()))
+        self._raise_recorded_errors('step')
+        return obs, ret, cost, length
 
     def reset(self, *, seed: Optional[int] = None, return_info: bool = False, options: Optional[dict] = None):
         """safe_adaptation_gym.py:85-107"""
