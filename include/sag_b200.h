@@ -24,8 +24,10 @@
  * work-list counter sets and the step epoch that selects them, the Philox key, the task ids, the queued next tasks)
  * lives in the handle's device memory, so sag_seed and sag_set_tasks issued between replays are seen by the graph.  The
  * *_host entry points, sag_seed, sag_set_tasks_host, sag_set_next_tasks_host, sag_bound_host, sag_copy_envs_host,
- * sag_create / sag_destroy
- * and sag_probe_d2h synchronise and must not be called while a capture is open.  sag_launch_count counts host-side enqueues only: replays do not add to it.  Conditions recorded by replayed
+ * sag_create / sag_destroy, sag_define_task
+ * and sag_probe_d2h synchronise and must not be called while a capture is open.  The first sag_define_task of a handle
+ * switches it to the kernel set that reads the user-defined task table, so a graph captured before it must be captured
+ * again.  sag_launch_count counts host-side enqueues only: replays do not add to it.  Conditions recorded by replayed
  * kernels are read with sag_error_flags as usual.
  */
 #ifndef SAG_B200_H
@@ -43,6 +45,7 @@ extern "C" {
 #define SAG_OBS_CAR 72      /* + ballangvel_rear (3) + quat2mat(ballquat_rear) (9), car.xml:37-38 */
 #define SAG_MAX_SLOTS 32
 #define SAG_MAX_GREMLINS 4
+#define SAG_MAX_CUSTOM_TASKS 16  /* user-defined tasks per handle (sag_define_task) */
 
 enum { SAG_ROBOT_POINT = 0, SAG_ROBOT_CAR = 1 };
 /* task ids: alphabetical registry order of the reference, benchmark/__init__.py:16-20 */
@@ -113,7 +116,7 @@ unsigned long long sag_launch_count(void* handle);
 int sag_debug_read(void* handle, unsigned long long* out18_host);
 
 /* env.set_task (safe_adaptation_gym.py:165-168): task_ids is a DEVICE int32[n_envs] array.  Statistics gathered under
- * the previous task are folded into the per-task totals first.  An id outside [0, SAG_NUM_TASKS) is replaced by
+ * the previous task are folded into the per-task totals first.  An id outside [0, sag_num_task_ids) is replaced by
  * SAG_T_GO_TO_GOAL and reported through sag_error_flags (SAG_ERR_BAD_TASK_ID). */
 int sag_set_tasks(void* handle, const int32_t* task_ids_dev, void* stream);
 /* same with a HOST int32[n_envs] array (validated: out-of-range ids fail the call); synchronous.  sag_set_tasks and
@@ -126,11 +129,11 @@ int sag_set_tasks_host(void* handle, const int32_t* task_ids_host);
  * under that old task, as sag_set_tasks does, (3) takes the queued id and clears the slot to -1, and (4) is reset as a
  * fresh Task instance of the new task (as with new_task != 0, for this environment only, even if the id is unchanged):
  * new ctrl-range scale and bound draws, new task state.  Environments with no task queued reset as the call asks.  A
- * queued id outside [0, SAG_NUM_TASKS) is not applied: the slot is cleared and SAG_ERR_BAD_TASK_ID is reported through
+ * queued id outside [0, sag_num_task_ids) is not applied: the slot is cleared and SAG_ERR_BAD_TASK_ID is reported through
  * sag_error_flags.
  * sag_set_next_tasks replaces every environment's slot from a DEVICE int32[n_envs] array (-1 = none); stream-ordered. */
 int sag_set_next_tasks(void* handle, const int32_t* task_ids_dev, void* stream);
-/* same with a HOST int32[n_envs] array (validated: an id outside [-1, SAG_NUM_TASKS) fails the call); synchronous */
+/* same with a HOST int32[n_envs] array (validated: an id outside [-1, sag_num_task_ids) fails the call); synchronous */
 int sag_set_next_tasks_host(void* handle, const int32_t* task_ids_host);
 /* info['bound'] (safe_adaptation_gym.py:79, world.py:75-78): DEVICE double[n_envs] constraint bound of every
  * environment's current Task instance; stream-ordered.  After task switches with SagConfig.random_bound this is how a
@@ -251,8 +254,29 @@ int sag_rollout(void* handle, int k_steps, float* obs, double* reward, uint8_t* 
 /* state injection / extraction; buffers are DEVICE pointers of sag_field_bytes(field) bytes */
 int sag_read_field(void* handle, int field, void* dst_dev, void* stream);
 int sag_write_field(void* handle, int field, const void* src_dev, void* stream);
+/* User-defined tasks (a subclass of a registry task that overrides Task.obstacles and Task.placement_extents,
+ * task.py:14-98).  base_task is the registry id whose reward, goal / button / box logic, dynamics variant and
+ * goal / button / box rectangles the task keeps; obstacles = {hazards, vases, gremlins, pillars}; placement_extents =
+ * {x_min, y_min, x_max, y_max}: free placements draw x in [x_min + k, x_max - k] and y in [y_min + k, y_max - k] for an
+ * object of keepout k. */
+typedef struct SagTaskDef {
+  int32_t base_task;
+  int32_t obstacles[4];
+  double placement_extents[4];
+} SagTaskDef;
+/* Define a task on this handle; synchronous.  *task_id receives SAG_NUM_TASKS, SAG_NUM_TASKS + 1, ... in order of
+ * definition.  Fails (nothing defined) unless base_task is a registry id, every count is >= 0, obstacles[2] equals
+ * SagConfig.num_gremlins, hazards + vases + gremlins + pillars + the base's task objects <= SAG_MAX_SLOTS,
+ * x_min < x_max, y_min < y_max, and fewer than SAG_MAX_CUSTOM_TASKS tasks are defined.  Once a handle has a definition,
+ * sag_task_stats writes sag_num_task_ids rows, and sag_set_tasks*, sag_set_next_tasks* and the queued-task rule accept
+ * ids below sag_num_task_ids (SAG_ERR_BAD_TASK_ID covers the ids outside it).  A layout that cannot be sampled is
+ * reported at reset as for registry tasks (SAG_FLAG_RESAMPLE_FAILED). */
+int sag_define_task(void* handle, const SagTaskDef* def, int32_t* task_id);
+/* SAG_NUM_TASKS + the number of tasks defined on this handle */
+int sag_num_task_ids(void* handle);
+
 /* per-task statistics of the episodes that FINISHED (time limit or done) since the last call with reset != 0, under the
- * task they ran with: DEVICE double out[SAG_NUM_TASKS][3] = {sum of episode returns, sum of episode costs, number of
+ * task they ran with: DEVICE double out[sag_num_task_ids(handle)][3] = {sum of episode returns, sum of episode costs, number of
  * episodes} (the buffer NCCL all-reduces).  Episodes cut short by a manual reset / set_task are not counted. */
 int sag_task_stats(void* handle, double* out_dev, int reset, void* stream);
 

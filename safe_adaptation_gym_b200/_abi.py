@@ -14,6 +14,7 @@ LIB_PATH = os.environ.get("SAG_B200_LIB") or os.path.join(_HERE, "csrc", "libsag
 NUM_TASKS = 14
 MAX_SLOTS = 32
 MAX_GREMLINS = 4
+MAX_CUSTOM_TASKS = 16
 F_ROBOT, F_OBJECTS, F_TASK_F64, F_TASK_I32, F_FLAGS, F_ROBOT_EXT, F_GREMLINS, F_NEXT_TASK = range(8)
 FLAG_PHYSICS_ERROR, FLAG_RESAMPLE_FAILED, FLAG_NEEDS_RESET, ERR_BAD_TASK_ID, ERR_BAD_ENV_INDEX = 1, 2, 4, 8, 16
 
@@ -32,6 +33,10 @@ class SagConfig(C.Structure):
     ]
 
 
+class SagTaskDef(C.Structure):
+    _fields_ = [("base_task", C.c_int32), ("obstacles", C.c_int32 * 4), ("placement_extents", C.c_double * 4)]
+
+
 class SagError(RuntimeError):
     pass
 
@@ -46,6 +51,7 @@ class SagLib:
         "sag_error_flags", "sag_reset_obs", "sag_reset_host", "sag_seed", "sag_reset", "sag_step", "sag_observe",
         "sag_step_host", "sag_observe_host", "sag_host_alloc", "sag_host_alloc_outputs", "sag_probe_d2h", "sag_host_free", "sag_rollout", "sag_read_field",
         "sag_write_field", "sag_task_stats", "sag_lidar", "sag_cost", "sag_export_outputs", "sag_evaluate_actions",
+        "sag_define_task", "sag_num_task_ids",
     ]
 
     def __init__(self, path, host_api=True):
@@ -79,6 +85,9 @@ class SagLib:
             L.sag_copy_envs_host.argtypes = [vp, vp, vp]
         if hasattr(L, "sag_evaluate_actions"):
             L.sag_evaluate_actions.argtypes = [vp, i32, fp, C.c_double, fp, dp, i32, dp, vp, vp]
+        if hasattr(L, "sag_define_task"):
+            L.sag_define_task.argtypes = [vp, C.POINTER(SagTaskDef), C.POINTER(C.c_int32)]
+            L.sag_num_task_ids.argtypes = [vp]
         L.sag_seed.argtypes = [vp, C.c_uint64]
         L.sag_error_flags.argtypes = [vp, i32]
         L.sag_reset_obs.argtypes = [vp, u8p, i32, i32, fp, u8p, vp]

@@ -137,6 +137,21 @@ SAG_HD TaskSpec task_spec(int t) {
   return s;
 }
 
+// User-defined tasks (sag_define_task): ids T_COUNT, T_COUNT + 1, ... of a handle.  An entry is the base task's
+// descriptor with the user's obstacle counts (nh, nv, ng, np) and placement extents (x_min, y_min, x_max, y_max); `base`
+// is the registry id whose reward, goal / button / box logic and dynamics variant the task keeps.  The table lives in
+// the handle's slab (custom_table); only the *C instantiations read it.
+constexpr int kMaxCustomTasks = 16;
+struct CustomTask {
+  TaskSpec sp;
+  int base;
+  double ext[4];
+};
+struct CustomTable {
+  int count;
+  CustomTask t[kMaxCustomTasks];
+};
+
 // task descriptor of an environment of this handle: the task's table entry + the handle's gremlin count
 struct Dev;
 SAG_HD TaskSpec spec_for(const Dev& D, int t, bool gremlins);
@@ -217,8 +232,25 @@ struct Dev {
   unsigned char* flags;
 };
 
+// the user-defined task table of a handle: at the end of the slab, its address in the scheduling block at
+// D.counts + kCustomTablePtr (sag_layout.h: slab_bind); read by the *C instantiations only
+constexpr int kCustomTablePtr = 56;
+SAG_HD const CustomTable& custom_table(const Dev& D) {
+  return **reinterpret_cast<const CustomTable* const*>(D.counts + kCustomTablePtr);
+}
+
 // gremlins = RB::kGremlins: in the default instantiations the count is the compile-time constant 0 of the task table
 SAG_HD TaskSpec spec_for(const Dev& D, int t, bool gremlins) { TaskSpec s = task_spec(t); if (gremlins) s.ng = D.num_gremlins; return s; }
+// custom = RB::kCustom: the *C instantiations look ids >= T_COUNT up in the handle's table (whose gremlin count is the
+// handle's); the others never see such an id and compile to the registry lookup alone
+SAG_HD TaskSpec spec_for(const Dev& D, int t, bool gremlins, bool custom) {
+  if (custom && t >= T_COUNT) return custom_table(D).t[t - T_COUNT].sp;
+  return spec_for(D, t, gremlins);
+}
+// the registry id whose logic an environment with task id t runs (Ctx::task)
+SAG_HD int logic_task(const Dev& D, int t, bool custom) { return custom && t >= T_COUNT ? custom_table(D).t[t - T_COUNT].base : t; }
+// the ids a handle accepts: the registry's, and with custom (RB::kCustom) the defined ones
+SAG_HD int num_task_ids(const Dev& D, bool custom) { return custom ? T_COUNT + custom_table(D).count : T_COUNT; }
 SAG_HD size_t oidx(const Dev& D, int slot, int e) { return (size_t)slot * D.stride + e; }
 
 // View of ONE environment's object arrays: field[slot * stride].  Global memory: pointers offset by the environment
@@ -577,6 +609,7 @@ constexpr CarModel kCar = car_model();
 struct PointRobot {
   static constexpr int kKind = 0, kNGeom = 2, kNsub = kPtNsub, kObsDim = 60;
   static constexpr bool kGremlins = false;  // the gremlin code paths exist only in the *G instantiations (below)
+  static constexpr bool kCustom = false;    // the user-defined task table is read only by the *C instantiations (below)
   static constexpr double kH = kPtH, kReach = kRobotReach;
   double q[3], v[3];
   double ctrl[2];
@@ -611,6 +644,7 @@ struct PointRobot {
 struct CarRobot {
   static constexpr int kKind = 1, kNGeom = kCarNGeom, kNsub = kCarNsub, kObsDim = 72;
   static constexpr bool kGremlins = false;
+  static constexpr bool kCustom = false;
   static constexpr double kH = kCarH, kReach = 0.22;  // >= farthest footprint corner (wheel: hypot(0.155, 0.15))
   double q[3], v[3];
   double ctrl[2];
@@ -665,6 +699,13 @@ struct CarRobot {
 // with kGremlins = true; the default instantiations carry none of the weld / mocap code.
 struct PointRobotG : PointRobot { static constexpr bool kGremlins = true; };
 struct CarRobotG : CarRobot { static constexpr bool kGremlins = true; };
+// Handles with user-defined tasks (sag_define_task) run the same code instantiated with kCustom = true: the task
+// descriptor of an id >= T_COUNT comes from the handle's table (spec_for), and free placements take the task's
+// rectangle.  The default instantiations carry none of it.
+struct PointRobotC : PointRobot { static constexpr bool kCustom = true; };
+struct CarRobotC : CarRobot { static constexpr bool kCustom = true; };
+struct PointRobotGC : PointRobotG { static constexpr bool kCustom = true; };
+struct CarRobotGC : CarRobotG { static constexpr bool kCustom = true; };
 
 SAG_HD bool bad_val(double x) { return !(fabs(x) <= 1e10); }
 
@@ -1245,15 +1286,21 @@ SAG_HD void contact_pass_body(const Ctx& C, const RB& R, double sn, double cs, c
   P.wtau[0] = P.wtau[1] = 0.0;
   // ---- which constraint rows exist?
   unsigned touched = 0;
+  bool any_row = false;
   for (int i = 0; i < ncon; ++i) {
     const Con& c = con[i];
     if (!(c.dist < 0.0) || (c.ba < 0 && c.bb < 0)) continue;
-    touched |= 0x80000000u;  // marker: at least one active row (slot 31 is never a movable body)
+    // bit 31 marks an active row where no registry task has a movable body in slot 31; a user-defined task can have
+    // its box there (*C instantiations: a flag of its own)
+    if constexpr (RB::kCustom) any_row = true;
+    else touched |= 0x80000000u;
     if (c.ba > 0) touched |= 1u << (c.ba - 1);
     if (c.bb > 0) touched |= 1u << (c.bb - 1);
   }
-  const bool any_row = (touched & 0x80000000u) != 0;
-  touched &= 0x7fffffffu;
+  if constexpr (!RB::kCustom) {
+    any_row = (touched & 0x80000000u) != 0;
+    touched &= 0x7fffffffu;
+  }
   int nactive = 0;  // contact rows (counted only where weld rows share the row table)
   if constexpr (RB::kGremlins) for (int i = 0; i < ncon; ++i) { const Con& c = con[i]; if (c.dist < 0.0 && !(c.ba < 0 && c.bb < 0)) ++nactive; }
   double tdx = 0.0, tdy = 0.0, tlen = 0.0, tdist = 0.0;
@@ -2250,7 +2297,8 @@ SAG_HD int env_step(unsigned wmask, Scratch* S, const Dev& D, int e, float a0, f
                      unsigned char* cost, unsigned char* done, bool pretest = true) {
   constexpr bool Coop = Mode == kStepCoop, Near = Mode == kStepNear;
   SAG_CLK_DECL;
-  Ctx C = {D, e, spec_for(D, D.task[e], RB::kGremlins), Slots(), D.task[e], global_objects(D, e)};
+  Ctx C = {D, e, spec_for(D, D.task[e], RB::kGremlins, RB::kCustom), Slots(), logic_task(D, D.task[e], RB::kCustom),
+           global_objects(D, e)};
   C.L = make_slots(C.sp);
 #if defined(__CUDA_ARCH__)
   if constexpr (Coop) {  // stage the object arrays in the warp's working set, one slot per lane; written back at the end
@@ -2525,7 +2573,8 @@ SAG_HD void eval_accumulate(const EvalAcc& A, int e, const double* rew, unsigned
 // observation at the current state (reset return value / refresh after state injection)
 template <class RB>
 SAG_HD void env_observe(unsigned wmask, Scratch* S, const Dev& D, int e, float* obs_s, int ostride) {
-  Ctx C = {D, e, spec_for(D, D.task[e], RB::kGremlins), Slots(), D.task[e], global_objects(D, e)};
+  Ctx C = {D, e, spec_for(D, D.task[e], RB::kGremlins, RB::kCustom), Slots(), logic_task(D, D.task[e], RB::kCustom),
+           global_objects(D, e)};
   C.L = make_slots(C.sp);
   RB R;
   load_robot(D, e, C.sp, R);
@@ -2553,6 +2602,13 @@ SAG_HD void env_observe(unsigned wmask, Scratch* S, const Dev& D, int e, float* 
 // reset: layout rejection sampling (world.py:172-217, utils.py:22-70), yaw draws (world.py:108-137),
 // fresh physics (mujoco_bridge.py:170-175), task.reset (world.py:167-170)
 // ------------------------------------------------------------------------------------------------
+// the placement extents (x_min, y_min, x_max, y_max) of a user-defined task; a registry id keeps (-e, -e, e, e)
+SAG_HD void custom_extents(const Dev& D, int t, double* rect) {
+  if (t < T_COUNT) return;
+  const double* x = custom_table(D).t[t - T_COUNT].ext;
+  rect[0] = x[0]; rect[1] = x[1]; rect[2] = x[2]; rect[3] = x[3];
+}
+
 SAG_HD double slot_keepout(const Dev& D, const TaskSpec& sp, int kind) {
   return kind == K_HAZARD ? D.k_hazard : kind == K_VASE ? D.k_vase : kind == K_GREMLIN ? D.k_gremlin
        : kind == K_PILLAR ? D.k_pillar : kind == K_GOAL ? kGoalKeepout : kind == K_BUTTON ? kButtonsKeepout : sp.box_keepout;
@@ -2562,16 +2618,17 @@ SAG_HD double slot_keepout(const Dev& D, const TaskSpec& sp, int kind) {
 // the reset path.  Called by k_reset (lane 0 of the warp that resets e) and by the host emulation's reset, after the
 // finished episode has been credited to the per-environment statistics.  A queued task: the statistics gathered under
 // the old task are folded into the per-task accumulator `acc` (as k_set_tasks does), e takes the new task id and is
-// reset as a fresh Task instance even if the id is unchanged.  An id outside [0, T_COUNT) is not applied: the slot is
-// cleared and SAG_ERR_BAD_TASK_ID recorded.  Returns whether e is reset as a fresh Task instance.
+// reset as a fresh Task instance even if the id is unchanged.  An id outside [0, nids) is not applied: the slot is
+// cleared and SAG_ERR_BAD_TASK_ID recorded.  nids: the handle's ids (num_task_ids).  Returns whether e is reset as a
+// fresh Task instance.
 SAG_HD bool take_next_task(const Dev& D, int e, int* next_task, double* sret, double* scost, double* sn, double* acc,
-                           bool new_task) {
+                           bool new_task, int nids = T_COUNT) {
   const int id = next_task[e];
   if (id == -1) return new_task;
   next_task[e] = -1;
-  if (id < 0 || id >= T_COUNT) { D.errflags[1] = 1; return new_task; }
+  if (id < 0 || id >= nids) { D.errflags[1] = 1; return new_task; }
   const int old = D.task[e];
-  if (sn[e] != 0.0 && old >= 0 && old < T_COUNT) {
+  if (sn[e] != 0.0 && old >= 0 && old < nids) {
 #if defined(__CUDA_ARCH__)
     atomicAdd(acc + 3 * old, sret[e]); atomicAdd(acc + 3 * old + 1, scost[e]); atomicAdd(acc + 3 * old + 2, sn[e]);
 #else
@@ -2593,7 +2650,7 @@ SAG_HD bool take_next_task(const Dev& D, int e, int* next_task, double* sret, do
 // reset yet is credited, then j's finished-episode statistics are folded into the per-task accumulator `acc` under j's
 // OLD task and cleared, so that they are not credited to the copied task.  An unfinished episode of j is dropped.
 SAG_HD int copy_env_source(const Dev& D, const int32_t* src_of_dst, int j, int n_src, bool same_handle, bool fold,
-                           double* sret, double* scost, double* sn, double* acc) {
+                           double* sret, double* scost, double* sn, double* acc, int nids = T_COUNT) {
   const int s = src_of_dst[j];
   if (s == -1 || (same_handle && s == j)) return -1;
   bool bad = s < -1 || s >= n_src;
@@ -2609,7 +2666,7 @@ SAG_HD int copy_env_source(const Dev& D, const int32_t* src_of_dst, int j, int n
     const int old = D.task[j];
     double r = sret[j], c = scost[j], k = sn[j];
     if ((D.flags[j] & F_NEEDS_RESET) && D.nstep[j] > 0) { r += D.epret[j]; c += D.epcost[j]; k += 1.0; }
-    if (k != 0.0 && old >= 0 && old < T_COUNT) {
+    if (k != 0.0 && old >= 0 && old < nids) {
 #if defined(__CUDA_ARCH__)
       atomicAdd(acc + 3 * old, r); atomicAdd(acc + 3 * old + 1, c); atomicAdd(acc + 3 * old + 2, k);
 #else
@@ -2662,7 +2719,8 @@ SAG_HD TaskDraws fresh_episode(const Dev& D, const Ctx& C, const Rng& rng, doubl
 
 template <class RB>
 SAG_HD_NOINLINE void env_reset(const Dev& D, int e, uint32_t episode, bool new_task) {
-  Ctx C = {D, e, spec_for(D, D.task[e], RB::kGremlins), Slots(), D.task[e], global_objects(D, e)};
+  Ctx C = {D, e, spec_for(D, D.task[e], RB::kGremlins, RB::kCustom), Slots(), logic_task(D, D.task[e], RB::kCustom),
+           global_objects(D, e)};
   C.L = make_slots(C.sp);
   const unsigned long long key = rng_key_value(rng_key(D));  // once per layout: the rejection sampler draws in a loop
   Rng rng = {rng_key_of(key), D.gid_base + (uint32_t)e, episode};
@@ -2672,6 +2730,8 @@ SAG_HD_NOINLINE void env_reset(const Dev& D, int e, uint32_t episode, bool new_t
   double rxy[2] = {0.0, 0.0};
   bool ok = false;
   const double ext = C.sp.extent;
+  double rect[4] = {-ext, -ext, ext, ext};  // free placements (*C instantiations: a user-defined task's own extents)
+  if constexpr (RB::kCustom) custom_extents(D, D.task[e], rect);
   // the placed bodies' positions and keepout + margin, thread-private (the rejection loop below reads them ~10^3 times)
   double px[kMaxObj], py[kMaxObj], pk[kMaxObj];
   for (int j = 0; j < kMaxObj; ++j) { px[j] = 0.0; py[j] = 0.0; pk[j] = 0.0; }
@@ -2683,17 +2743,21 @@ SAG_HD_NOINLINE void env_reset(const Dev& D, int e, uint32_t episode, bool new_t
       int kind = idx < 0 ? K_NONE : slot_kind(C.sp, C.L, idx);
       double keepout = idx < 0 ? D.robot_keepout : slot_keepout(D, C.sp, kind);
       double half = ext;  // free placement in the task extents
-      if (kind == K_GOAL) half = 1.5;
-      else if (kind == K_BUTTON) half = C.sp.button_rect;
-      else if ((kind == K_BOX || kind == K_ROD || kind == K_BALL) && C.sp.box_rect > 0.0) half = C.sp.box_rect;
-      double xmin = -half + keepout, xmax = half - keepout;
+      bool free_xy = true;
+      if (kind == K_GOAL) { half = 1.5; free_xy = false; }
+      else if (kind == K_BUTTON) { half = C.sp.button_rect; free_xy = false; }
+      else if ((kind == K_BOX || kind == K_ROD || kind == K_BALL) && C.sp.box_rect > 0.0) { half = C.sp.box_rect; free_xy = false; }
+      double xmin = -half + keepout, xmax = half - keepout, ymin = xmin, ymax = xmax;
+      if constexpr (RB::kCustom) {
+        if (free_xy) { xmin = rect[0] + keepout; ymin = rect[1] + keepout; xmax = rect[2] - keepout; ymax = rect[3] - keepout; }
+      }
       bool placed = false;
       double x = 0.0, y = 0.0;
       for (int k = 0; k < 1000; ++k) {
         if (--draws_left < 0) { failed = true; break; }
         double u1, u2;
         rng.pair(0u, ctr++, u1, u2);
-        x = xmin + (xmax - xmin) * u1; y = xmin + (xmax - xmin) * u2;
+        x = xmin + (xmax - xmin) * u1; y = ymin + (ymax - ymin) * u2;
         bool valid = true;
         if (idx >= 0) {
           double dx = x - rxy[0], dy = y - rxy[1];
@@ -2859,7 +2923,8 @@ template <class RB>
 __device__ __noinline__ void env_reset_coop(const Dev& D, int e, uint32_t episode, bool new_task, double* px, double* py, double* pk) {
   const int lane = coop_lane();
   const int cand = lane >> 2, grp = lane & 3;  // 8 placement candidates per round, each checked by 4 lanes
-  Ctx C = {D, e, spec_for(D, D.task[e], RB::kGremlins), Slots(), D.task[e], global_objects(D, e)};
+  Ctx C = {D, e, spec_for(D, D.task[e], RB::kGremlins, RB::kCustom), Slots(), logic_task(D, D.task[e], RB::kCustom),
+           global_objects(D, e)};
   C.L = make_slots(C.sp);
   const ObjView G = C.O;
   const unsigned long long key = rng_key_value(rng_key(D));  // once per layout: the rejection sampler draws in a loop
@@ -2870,6 +2935,8 @@ __device__ __noinline__ void env_reset_coop(const Dev& D, int e, uint32_t episod
   double rxy[2] = {0.0, 0.0};
   bool ok = false;
   const double ext = C.sp.extent;
+  double rect[4] = {-ext, -ext, ext, ext};
+  if constexpr (RB::kCustom) custom_extents(D, D.task[e], rect);
   px[lane] = 0.0; py[lane] = 0.0;
   pk[lane] = lane < C.L.n ? slot_keepout(D, C.sp, slot_kind(C.sp, C.L, lane)) + D.placements_margin : 0.0;
   __syncwarp();
@@ -2880,10 +2947,14 @@ __device__ __noinline__ void env_reset_coop(const Dev& D, int e, uint32_t episod
       int kind = idx < 0 ? K_NONE : slot_kind(C.sp, C.L, idx);
       double keepout = idx < 0 ? D.robot_keepout : slot_keepout(D, C.sp, kind);
       double half = ext;
-      if (kind == K_GOAL) half = 1.5;
-      else if (kind == K_BUTTON) half = C.sp.button_rect;
-      else if ((kind == K_BOX || kind == K_ROD || kind == K_BALL) && C.sp.box_rect > 0.0) half = C.sp.box_rect;
-      const double xmin = -half + keepout, xmax = half - keepout;
+      bool free_xy = true;
+      if (kind == K_GOAL) { half = 1.5; free_xy = false; }
+      else if (kind == K_BUTTON) { half = C.sp.button_rect; free_xy = false; }
+      else if ((kind == K_BOX || kind == K_ROD || kind == K_BALL) && C.sp.box_rect > 0.0) { half = C.sp.box_rect; free_xy = false; }
+      double xmin = -half + keepout, xmax = half - keepout, ymin = xmin, ymax = xmax;
+      if constexpr (RB::kCustom) {
+        if (free_xy) { xmin = rect[0] + keepout; ymin = rect[1] + keepout; xmax = rect[2] - keepout; ymax = rect[3] - keepout; }
+      }
       bool placed = false;
       double x = 0.0, y = 0.0;
       int used = 0;  // draws spent on this object (limit 1000, world.py:209)
@@ -2894,7 +2965,7 @@ __device__ __noinline__ void env_reset_coop(const Dev& D, int e, uint32_t episod
         if ((long)window > draws_left) window = (int)draws_left;
         double u1, u2;
         rng.pair(0u, ctr + (uint32_t)cand, u1, u2);
-        const double cx = xmin + (xmax - xmin) * u1, cy = xmin + (xmax - xmin) * u2;
+        const double cx = xmin + (xmax - xmin) * u1, cy = ymin + (ymax - ymin) * u2;
         bool bad = false;
         if (idx >= 0) {
           if (grp == 0) { double dx = cx - rxy[0], dy = cy - rxy[1]; if (sqrt_less(dx * dx + dy * dy, rk + keepout)) bad = true; }

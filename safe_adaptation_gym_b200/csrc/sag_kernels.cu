@@ -68,7 +68,9 @@ struct Handle {
   void* field_ptr[SAG_NUM_FIELDS];
   size_t field_bytes[SAG_NUM_FIELDS];
   double *sret, *scost, *sn;  // per-env finished-episode statistics (under the env's current task)
-  double* stats_acc;          // [SAG_NUM_TASKS][3]: statistics folded away when environments changed task
+  double* stats_acc;          // [SAG_NUM_TASKS + SAG_MAX_CUSTOM_TASKS][3]: statistics folded away when environments changed task
+  CustomTable custom_h;       // host copy of the user-defined task table (sag_define_task; the kernels read the slab's)
+  CustomTable* custom_d;      // the slab's table
   int32_t* next_task;         // [stride] SAG_F_NEXT_TASK: task queued for the next reset (-1 = none); k_reset consumes it
   int* err_h;                 // mapped pinned int[4]: sticky error words written by the kernels (sag_error_flags)
   int32_t* ids_d;             // staging for sag_set_tasks_host
@@ -164,7 +166,8 @@ __global__ void __launch_bounds__(kBS, RB::kKind == 1 ? 2 : 4) k_step_free(Dev D
   bool run = false, pretest = false;
   if (e < D.n) {
     RB R;
-    load_robot(D, e, task_spec(D.task[e]), R);
+    if constexpr (RB::kCustom) load_robot(D, e, spec_for(D, D.task[e], false, true), R);
+    else load_robot(D, e, task_spec(D.task[e]), R);
     const unsigned char fl = D.flags[e];
     run = !(fl & F_PHYS_ERROR) && D.movmask[e] == 0 && D.num_gremlins == 0;  // (a welded gremlin is a constraint row in every pass)
     pretest = !env_is_quiet(D.clear[e], R);
@@ -358,7 +361,7 @@ __global__ void __launch_bounds__(32 * kResetWarps) k_reset(Dev D, const uint8_t
     int fresh = new_task != 0;
     if (lane == 0) {
       if ((fl & F_NEEDS_RESET) && D.nstep[e] > 0) { sret[e] += D.epret[e]; scost[e] += D.epcost[e]; sn[e] += 1.0; }
-      fresh = take_next_task(D, e, next_task, sret, scost, sn, acc, fresh != 0);
+      fresh = take_next_task(D, e, next_task, sret, scost, sn, acc, fresh != 0, num_task_ids(D, RB::kCustom));
     }
     fresh = __shfl_sync(0xffffffffu, fresh, 0);
     __syncwarp();  // lane 0's writes (a new D.task[e]) are seen by the whole warp
@@ -379,19 +382,31 @@ __global__ void __launch_bounds__(32 * kResetWarps) k_reset(Dev D, const uint8_t
 // env.set_task: statistics gathered under the old task are folded into the per-task accumulator first (so that they
 // are not re-labelled), including an episode that has finished but has not been reset yet; ids are validated; queued
 // next tasks are dropped.
+// nids: the handle's task ids (SAG_NUM_TASKS, or more in k_set_tasks_custom)
+__device__ __forceinline__ void set_task_of(const Dev& D, int e, const int32_t* __restrict__ ids, double* sret, double* scost,
+                                            double* sn, double* acc, int* next_task, int nids) {
+  const int old = D.task[e];
+  double r = sret[e], c = scost[e], k = sn[e];
+  if ((D.flags[e] & F_NEEDS_RESET) && D.nstep[e] > 0) { r += D.epret[e]; c += D.epcost[e]; k += 1.0; D.nstep[e] = 0; }
+  if (k != 0.0 && old >= 0 && old < nids) { atomicAdd(acc + 3 * old, r); atomicAdd(acc + 3 * old + 1, c); atomicAdd(acc + 3 * old + 2, k); }
+  sret[e] = 0.0; scost[e] = 0.0; sn[e] = 0.0;
+  int id = ids[e];
+  if (id < 0 || id >= nids) { id = SAG_T_GO_TO_GOAL; D.errflags[1] = 1; }
+  D.task[e] = id;
+  next_task[e] = -1;
+}
 __global__ void k_set_tasks(Dev D, const int32_t* __restrict__ ids, double* sret, double* scost, double* sn, double* acc,
                             int* next_task) {
   const int e = blockIdx.x * blockDim.x + threadIdx.x;
   if (e >= D.n) return;
-  const int old = D.task[e];
-  double r = sret[e], c = scost[e], k = sn[e];
-  if ((D.flags[e] & F_NEEDS_RESET) && D.nstep[e] > 0) { r += D.epret[e]; c += D.epcost[e]; k += 1.0; D.nstep[e] = 0; }
-  if (k != 0.0 && old >= 0 && old < SAG_NUM_TASKS) { atomicAdd(acc + 3 * old, r); atomicAdd(acc + 3 * old + 1, c); atomicAdd(acc + 3 * old + 2, k); }
-  sret[e] = 0.0; scost[e] = 0.0; sn[e] = 0.0;
-  int id = ids[e];
-  if (id < 0 || id >= SAG_NUM_TASKS) { id = SAG_T_GO_TO_GOAL; D.errflags[1] = 1; }
-  D.task[e] = id;
-  next_task[e] = -1;
+  set_task_of(D, e, ids, sret, scost, sn, acc, next_task, SAG_NUM_TASKS);
+}
+// handles with user-defined tasks: their ids are valid too
+__global__ void k_set_tasks_custom(Dev D, const int32_t* __restrict__ ids, double* sret, double* scost, double* sn,
+                                   double* acc, int* next_task) {
+  const int e = blockIdx.x * blockDim.x + threadIdx.x;
+  if (e >= D.n) return;
+  set_task_of(D, e, ids, sret, scost, sn, acc, next_task, num_task_ids(D, true));
 }
 
 // sag_copy_envs: environment states gathered column by column.  The fields are SoA and environment-minor, so the
@@ -431,6 +446,11 @@ __global__ void k_copy_envs_fold(Dev D, const int32_t* __restrict__ src_of_dst, 
   const int j = blockIdx.x * blockDim.x + threadIdx.x;
   if (j < D.n) copy_env_source(D, src_of_dst, j, n_src, same_handle != 0, true, sret, scost, sn, acc);
 }
+__global__ void k_copy_envs_fold_custom(Dev D, const int32_t* __restrict__ src_of_dst, int n_src, int same_handle,
+                                        double* sret, double* scost, double* sn, double* acc) {
+  const int j = blockIdx.x * blockDim.x + threadIdx.x;
+  if (j < D.n) copy_env_source(D, src_of_dst, j, n_src, same_handle != 0, true, sret, scost, sn, acc, num_task_ids(D, true));
+}
 
 __global__ void __launch_bounds__(kCopyThreads) k_copy_envs(Dev D, CopyFields F, const int32_t* __restrict__ src_of_dst,
                                                             int n_src, int src_stride, int same_handle) {
@@ -461,6 +481,21 @@ __global__ void k_task_stats(Dev D, const double* sret, const double* scost, con
   }
   __syncthreads();
   for (int i = threadIdx.x; i < SAG_NUM_TASKS * 3; i += blockDim.x)
+    if ((&acc[0][0])[i] != 0.0) atomicAdd(out + i, (&acc[0][0])[i]);
+}
+// the same with a row for every id a handle with user-defined tasks can have; out has sag_num_task_ids rows, and a row
+// beyond them is never non-zero (every environment's task id is below that count)
+__global__ void k_task_stats_custom(Dev D, const double* sret, const double* scost, const double* sn, double* out) {
+  constexpr int kRows = SAG_NUM_TASKS + SAG_MAX_CUSTOM_TASKS;
+  __shared__ double acc[kRows][3];
+  for (int i = threadIdx.x; i < kRows * 3; i += blockDim.x) (&acc[0][0])[i] = 0.0;
+  __syncthreads();
+  for (int e = blockIdx.x * blockDim.x + threadIdx.x; e < D.n; e += gridDim.x * blockDim.x) {
+    int t = D.task[e];
+    if (sn[e] != 0.0) { atomicAdd(&acc[t][0], sret[e]); atomicAdd(&acc[t][1], scost[e]); atomicAdd(&acc[t][2], sn[e]); }
+  }
+  __syncthreads();
+  for (int i = threadIdx.x; i < kRows * 3; i += blockDim.x)
     if ((&acc[0][0])[i] != 0.0) atomicAdd(out + i, (&acc[0][0])[i]);
 }
 
@@ -726,10 +761,14 @@ struct Ops {
   }
 };
 
-// one set of kernels per robot model; environments with gremlins (SagConfig.num_gremlins > 0) use the *G instantiations
-#define SAG_DISPATCH(H, call)                                                                                     \
-  ((H)->D.robot == SAG_ROBOT_CAR ? ((H)->D.num_gremlins > 0 ? Ops<CarRobotG>::call : Ops<CarRobot>::call)          \
-                                 : ((H)->D.num_gremlins > 0 ? Ops<PointRobotG>::call : Ops<PointRobot>::call))
+// one set of kernels per robot model; environments with gremlins (SagConfig.num_gremlins > 0) use the *G instantiations,
+// handles with user-defined tasks (sag_define_task) the *C ones
+#define SAG_DISPATCH(H, call)                                                                                       \
+  ((H)->custom_h.count > 0                                                                                          \
+       ? ((H)->D.robot == SAG_ROBOT_CAR ? ((H)->D.num_gremlins > 0 ? Ops<CarRobotGC>::call : Ops<CarRobotC>::call)    \
+                                        : ((H)->D.num_gremlins > 0 ? Ops<PointRobotGC>::call : Ops<PointRobotC>::call)) \
+       : ((H)->D.robot == SAG_ROBOT_CAR ? ((H)->D.num_gremlins > 0 ? Ops<CarRobotG>::call : Ops<CarRobot>::call)      \
+                                        : ((H)->D.num_gremlins > 0 ? Ops<PointRobotG>::call : Ops<PointRobot>::call)))
 
 }  // namespace
 
@@ -777,6 +816,8 @@ int sag_create(const SagConfig* cfg, int device, void** handle) {
   // episode counters start at 0xFFFFFFFF so that the first reset is episode 0
   ce = cudaMemset(D.episode, 0xFF, st * sizeof(unsigned));
   if (ce == cudaSuccess) ce = cudaMemcpy(D.key, &cfg->seed, sizeof(*D.key), cudaMemcpyHostToDevice);
+  H->custom_d = (CustomTable*)(base + LY.custom_off);  // (zeroed with the slab: no task defined)
+  if (ce == cudaSuccess) ce = cudaMemcpy(D.counts + kCustomTablePtr, &H->custom_d, sizeof(H->custom_d), cudaMemcpyHostToDevice);
   H->stats_acc = (double*)(base + LY.acc_off);
   H->ids_d = (int32_t*)(base + LY.ids_off); H->mask_d = (uint8_t*)(base + LY.mask_off);
   H->next_task = (int32_t*)H->field_ptr[SAG_F_NEXT_TASK];
@@ -824,27 +865,58 @@ size_t sag_field_bytes(void* handle, int field) {
   return ((Handle*)handle)->field_bytes[field];
 }
 
+static int launch_set_tasks(Handle* H, const int32_t* ids, cudaStream_t s) {
+  auto k = H->custom_h.count > 0 ? k_set_tasks_custom : k_set_tasks;
+  k<<<(H->D.n + 255) / 256, 256, 0, s>>>(H->D, ids, H->sret, H->scost, H->sn, H->stats_acc, H->next_task);
+  ++H->launches;
+  CK(cudaGetLastError());
+  return 0;
+}
+
 int sag_set_tasks(void* handle, const int32_t* ids, void* stream) {
   Handle* H = (Handle*)handle;
   if (!H || !ids) return fail("sag_set_tasks: null argument");
   DevGuard guard(H->device);
-  k_set_tasks<<<(H->D.n + 255) / 256, 256, 0, (cudaStream_t)stream>>>(H->D, ids, H->sret, H->scost, H->sn, H->stats_acc, H->next_task);
-  ++H->launches;
-  CK(cudaGetLastError());
+  return launch_set_tasks(H, ids, (cudaStream_t)stream);
+}
+
+int sag_num_task_ids(void* handle) { return handle ? SAG_NUM_TASKS + ((Handle*)handle)->custom_h.count : SAG_NUM_TASKS; }
+
+int sag_define_task(void* handle, const SagTaskDef* def, int32_t* task_id) {
+  Handle* H = (Handle*)handle;
+  if (!H || !def || !task_id) return fail("sag_define_task: null argument");
+  if (const char* what = task_def_error(*def, H->D.num_gremlins)) {
+    snprintf(g_err, sizeof(g_err), "sag_define_task: %s", what);
+    return 1;
+  }
+  if (H->custom_h.count >= SAG_MAX_CUSTOM_TASKS) return fail("sag_define_task: SAG_MAX_CUSTOM_TASKS tasks are defined already");
+  DevGuard guard(H->device);
+  CK(cudaDeviceSynchronize());  // ordered after everything issued earlier; the kernels read the table from the slab
+  if (H->custom_h.count == 0) {  // the first definition switches the handle to the *C kernel set
+    Handle T = *H;
+    T.custom_h.count = 1;
+    CK(SAG_DISPATCH(&T, setup(&T)));
+    H->busy_grid = T.busy_grid;
+  }
+  CustomTable next = H->custom_h;
+  next.t[next.count] = custom_task(*def);
+  ++next.count;
+  CK(cudaMemcpy(H->custom_d, &next, sizeof(next), cudaMemcpyHostToDevice));
+  H->custom_h = next;
+  *task_id = SAG_NUM_TASKS + next.count - 1;
   return 0;
 }
 
 int sag_set_tasks_host(void* handle, const int32_t* ids_host) {
   Handle* H = (Handle*)handle;
   if (!H || !ids_host) return fail("sag_set_tasks_host: null argument");
+  const int nids = sag_num_task_ids(H);
   for (int e = 0; e < H->D.n; ++e)
-    if (ids_host[e] < 0 || ids_host[e] >= SAG_NUM_TASKS) return fail("sag_set_tasks_host: task id out of range [0, SAG_NUM_TASKS)");
+    if (ids_host[e] < 0 || ids_host[e] >= nids) return fail("sag_set_tasks_host: task id out of range [0, sag_num_task_ids)");
   DevGuard guard(H->device);
   CK(cudaDeviceSynchronize());  // the host API is ordered after everything issued through the stream API
   CK(cudaMemcpyAsync(H->ids_d, ids_host, (size_t)H->D.n * sizeof(int32_t), cudaMemcpyHostToDevice, H->own_stream));
-  k_set_tasks<<<(H->D.n + 255) / 256, 256, 0, H->own_stream>>>(H->D, H->ids_d, H->sret, H->scost, H->sn, H->stats_acc, H->next_task);
-  ++H->launches;
-  CK(cudaGetLastError());
+  if (launch_set_tasks(H, H->ids_d, H->own_stream)) return 1;
   CK(cudaStreamSynchronize(H->own_stream));
   return 0;
 }
@@ -861,9 +933,10 @@ int sag_set_next_tasks(void* handle, const int32_t* ids, void* stream) {
 int sag_set_next_tasks_host(void* handle, const int32_t* ids_host) {
   Handle* H = (Handle*)handle;
   if (!H || !ids_host) return fail("sag_set_next_tasks_host: null argument");
+  const int nids = sag_num_task_ids(H);
   for (int e = 0; e < H->D.n; ++e)
-    if (ids_host[e] < -1 || ids_host[e] >= SAG_NUM_TASKS)
-      return fail("sag_set_next_tasks_host: task id out of range [-1, SAG_NUM_TASKS)");
+    if (ids_host[e] < -1 || ids_host[e] >= nids)
+      return fail("sag_set_next_tasks_host: task id out of range [-1, sag_num_task_ids)");
   DevGuard guard(H->device);
   CK(cudaDeviceSynchronize());  // the host API is ordered after everything issued through the stream API
   CK(cudaMemcpyAsync(H->next_task, ids_host, (size_t)H->D.n * sizeof(int32_t), cudaMemcpyHostToDevice, H->own_stream));
@@ -882,7 +955,7 @@ int sag_bound(void* handle, double* bound, void* stream) {
 static int copy_envs_check(const Handle* D, const Handle* S, const char* who) {
   if (!D || !S) { snprintf(g_err, sizeof(g_err), "%s: null handle", who); return 1; }
   if (D->device != S->device) { snprintf(g_err, sizeof(g_err), "%s: the handles are on different devices", who); return 1; }
-  if (const char* what = copy_incompatibility(D->D, S->D)) {
+  if (const char* what = copy_incompatibility(D->D, S->D, &D->custom_h, &S->custom_h)) {
     snprintf(g_err, sizeof(g_err), "%s: the handles differ in %s", who, what);
     return 1;
   }
@@ -896,7 +969,8 @@ static int launch_copy_envs(Handle* H, const Handle* S, const int32_t* src_of_ds
     F.rows[f] = kFieldShape[f].rows; F.elem[f] = kFieldShape[f].elem;
   }
   const int blocks = (H->D.n + kCopyThreads - 1) / kCopyThreads;
-  k_copy_envs_fold<<<blocks, kCopyThreads, 0, s>>>(H->D, src_of_dst, S->D.n, H == S, H->sret, H->scost, H->sn, H->stats_acc);
+  auto fold = H->custom_h.count > 0 ? k_copy_envs_fold_custom : k_copy_envs_fold;
+  fold<<<blocks, kCopyThreads, 0, s>>>(H->D, src_of_dst, S->D.n, H == S, H->sret, H->scost, H->sn, H->stats_acc);
   ++H->launches;
   CK(cudaGetLastError());
   k_copy_envs<<<dim3(blocks, copy_chunks()), kCopyThreads, 0, s>>>(H->D, F, src_of_dst, S->D.n, S->D.stride, H == S);
@@ -1238,13 +1312,15 @@ int sag_task_stats(void* handle, double* out, int reset, void* stream) {
   if (!H || !out) return fail("sag_task_stats: null argument");
   DevGuard guard(H->device);
   cudaStream_t s = (cudaStream_t)stream;
-  CK(cudaMemcpyAsync(out, H->stats_acc, SAG_NUM_TASKS * 3 * sizeof(double), cudaMemcpyDeviceToDevice, s));
-  k_task_stats<<<148, 256, 0, s>>>(H->D, H->sret, H->scost, H->sn, out);
+  const size_t rows = (size_t)sag_num_task_ids(H);
+  CK(cudaMemcpyAsync(out, H->stats_acc, rows * 3 * sizeof(double), cudaMemcpyDeviceToDevice, s));
+  if (H->custom_h.count > 0) k_task_stats_custom<<<148, 256, 0, s>>>(H->D, H->sret, H->scost, H->sn, out);
+  else k_task_stats<<<148, 256, 0, s>>>(H->D, H->sret, H->scost, H->sn, out);
   ++H->launches;
   CK(cudaGetLastError());
   if (reset) {
     CK(cudaMemsetAsync(H->sret, 0, 3 * (size_t)H->D.stride * sizeof(double), s));
-    CK(cudaMemsetAsync(H->stats_acc, 0, SAG_NUM_TASKS * 3 * sizeof(double), s));
+    CK(cudaMemsetAsync(H->stats_acc, 0, rows * 3 * sizeof(double), s));
   }
   return 0;
 }

@@ -23,7 +23,7 @@ inline size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
 
 struct SlabLayout {
   size_t off[SAG_NUM_FIELDS], bytes[SAG_NUM_FIELDS];
-  size_t stats_off, sched_off, act_off, obs_off, rew_off, cost_off, done_off, acc_off, ids_off, mask_off, total;
+  size_t stats_off, sched_off, act_off, obs_off, rew_off, cost_off, done_off, acc_off, ids_off, mask_off, custom_off, total;
 };
 
 // The per-environment shape of every state field: rows of `elem`-byte elements, each row `stride` elements long
@@ -54,9 +54,10 @@ inline SlabLayout slab_layout(int n, int stride, int obs_dim) {
   L.rew_off = total; total += align_up((size_t)n * sizeof(double), 256);
   L.cost_off = total; total += align_up((size_t)n, 256);
   L.done_off = total; total += align_up((size_t)n, 256);
-  L.acc_off = total; total += align_up(SAG_NUM_TASKS * 3 * sizeof(double), 256);
+  L.acc_off = total; total += align_up((SAG_NUM_TASKS + SAG_MAX_CUSTOM_TASKS) * 3 * sizeof(double), 256);
   L.ids_off = total; total += align_up((size_t)n * sizeof(int32_t), 256);
   L.mask_off = total; total += align_up((size_t)n, 256);
+  L.custom_off = total; total += align_up(sizeof(CustomTable), 256);
   L.total = total;
   return L;
 }
@@ -81,11 +82,15 @@ inline void slab_bind(Dev& D, const SlabLayout& L, char* base) {
   int32_t* sc = (int32_t*)(base + L.sched_off);
   // the block after the work list is 96 ints: two counter sets (16), 18 x u64 (36), the step epoch and the contact
   // kernel's finished-CTA counter (2), the Philox key (u64; 8-byte aligned: the block starts 256-aligned and 3 * st is a
-  // multiple of 96)
+  // multiple of 96), the address of the user-defined task table (custom_table; 8-byte aligned too)
   D.worklist = sc; D.counts = sc + 3 * st;
   D.dbg = (unsigned long long*)(sc + 3 * st + 16);
   D.epoch = (unsigned*)(sc + 3 * st + 52);
   D.key = (unsigned long long*)(sc + 3 * st + 54);
+#if !defined(__CUDACC__)
+  // a host build (the host emulation of the tests) stores the table's address here; the library copies it to the device
+  *reinterpret_cast<CustomTable**>(sc + 3 * st + kCustomTablePtr) = reinterpret_cast<CustomTable*>(base + L.custom_off);
+#endif
 }
 
 inline void dev_from_config(Dev& D, const SagConfig& c) {
@@ -105,10 +110,24 @@ inline void dev_from_config(Dev& D, const SagConfig& c) {
   D.num_gremlins = c.num_gremlins; D.gremlins_travel = c.gremlins_travel;
 }
 
+// sag_copy_envs: the two handles must have defined the same tasks in the same order (the ids are part of the state)
+inline bool custom_tables_differ(const CustomTable& a, const CustomTable& b) {
+  if (a.count != b.count) return true;
+  for (int i = 0; i < a.count; ++i) {
+    const CustomTask &x = a.t[i], &y = b.t[i];
+    if (x.base != y.base || x.sp.nh != y.sp.nh || x.sp.nv != y.sp.nv || x.sp.ng != y.sp.ng || x.sp.np != y.sp.np) return true;
+    for (int k = 0; k < 4; ++k) if (x.ext[k] != y.ext[k]) return true;
+  }
+  return false;
+}
+
 // sag_copy_envs: two handles whose environments can exchange states -- every configuration value that the layout
 // samplers or the step read from Dev, except the Philox key, the global ids and the per-handle budgets (n_envs,
 // max_episode_steps, max_layout_draws, action_noise).  Returns the first difference, or nullptr.
-inline const char* copy_incompatibility(const Dev& a, const Dev& b) {
+// ta / tb: host copies of the handles' user-defined task tables, which must be equal (the ids are part of the state).
+inline const char* copy_incompatibility(const Dev& a, const Dev& b, const CustomTable* ta = nullptr,
+                                        const CustomTable* tb = nullptr) {
+  if (ta && tb && custom_tables_differ(*ta, *tb)) return "user-defined tasks";
   if (a.robot != b.robot) return "robot";
   if (a.num_gremlins != b.num_gremlins) return "num_gremlins";
   if (a.hazards_size != b.hazards_size || a.vases_size != b.vases_size || a.pillars_size != b.pillars_size ||
@@ -123,6 +142,33 @@ inline const char* copy_incompatibility(const Dev& a, const Dev& b) {
   if (a.random_bound != b.random_bound) return "random_bound";
   if (a.max_bound != b.max_bound) return "max_bound";
   return nullptr;
+}
+
+static_assert(SAG_MAX_CUSTOM_TASKS == kMaxCustomTasks, "the ABI's and the kernels' custom-task capacity");
+
+// sag_define_task: the definition's errors, or nullptr.  `base` must be a registry id.
+inline const char* task_def_error(const SagTaskDef& d, int num_gremlins) {
+  if (d.base_task < 0 || d.base_task >= SAG_NUM_TASKS) return "base_task must be a registry task id [0, SAG_NUM_TASKS)";
+  for (int k = 0; k < 4; ++k) if (d.obstacles[k] < 0) return "obstacle counts must be >= 0";
+  if (d.obstacles[2] != num_gremlins) return "obstacles[2] (gremlins) must equal the handle's num_gremlins";
+  const TaskSpec b = task_spec(d.base_task);
+  const int task_objects = b.kind == 0 ? 1 : b.kind == 1 ? b.nbuttons : 2;
+  if ((long)d.obstacles[0] + d.obstacles[1] + d.obstacles[2] + d.obstacles[3] + task_objects > SAG_MAX_SLOTS)
+    return "hazards + vases + gremlins + pillars + the base task's objects exceed SAG_MAX_SLOTS";
+  const double* x = d.placement_extents;
+  if (!(x[0] < x[2]) || !(x[1] < x[3])) return "placement_extents need x_min < x_max and y_min < y_max";
+  return nullptr;
+}
+
+// the table entry of a valid definition: the base's descriptor with the definition's counts and extents
+inline CustomTask custom_task(const SagTaskDef& d) {
+  CustomTask c;
+  memset(&c, 0, sizeof(c));
+  c.sp = task_spec(d.base_task);
+  c.sp.nh = d.obstacles[0]; c.sp.nv = d.obstacles[1]; c.sp.ng = d.obstacles[2]; c.sp.np = d.obstacles[3];
+  c.base = d.base_task;
+  for (int k = 0; k < 4; ++k) c.ext[k] = d.placement_extents[k];
+  return c;
 }
 
 // sag_copy_envs_host: the checks the device path makes per pair (copy_env_source), for a whole host index array, so

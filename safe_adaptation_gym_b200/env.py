@@ -27,6 +27,11 @@ ctrl-range scale and bound draws).  With a device tensor of ids it may be record
 ``step``, so a graphed adaptation loop can walk through tasks; ``task_ids`` tells which task each environment runs now.
 ``set_task(task, mask)`` switches the masked environments at once (their running episodes are cut short and not counted).
 
+User-defined tasks: an instance of a subclass of a registry task that overrides ``obstacles`` and / or
+``placement_extents`` runs the base's logic with its own obstacle counts and extents, under a task id of its own (14,
+15, ... per batch; ``task_id_of``).  Everything that takes a task takes one.  Defining the first one switches the batch
+to another kernel set: a CUDA graph captured before it must be captured again.
+
 All per-step arithmetic (dynamics, reward / goal logic, cost, pseudo-lidar) runs in the CUDA library behind
 the C ABI of ``include/sag_b200.h``; this class only owns torch tensors and passes raw pointers.  There is
 no CPU fallback: without the built library and a CUDA device construction raises.
@@ -147,6 +152,7 @@ class BatchedSafeAdaptationGym:
         self._task_ids = None
         self._tasks = None
         self._any_unsupervised = False
+        self._custom = []          # user-defined tasks of this batch, in order of definition: id = NUM_TASKS + index
         self._next_armed = False   # set_next_task has been called: step refreshes a random bound after the auto-reset
         self._action_space = Box(-1, 1, (2,), dtype=np.float32)  # safe_adaptation_gym.py:49-50 (nu = 2)
         self._observation_space = None
@@ -343,10 +349,10 @@ class BatchedSafeAdaptationGym:
         ``Unsupervised`` (its reward is a pair, written to another buffer)."""
         self._forbid_capture('set_task')
         task_list = self._task_list(task, allow_none=False)
-        ids = torch.tensor([t.task_id for t in task_list], dtype=torch.int32)
+        ids = torch.tensor([self.task_id_of(t) for t in task_list], dtype=torch.int32)
         if mask is not None:
             m = torch.as_tensor(mask).to(device=self.device, dtype=torch.bool).reshape(self.num_envs)
-            unsup = ids == _tasks.Unsupervised.task_id
+            unsup = self._is_unsupervised(ids)
             self._any_unsupervised = self._any_unsupervised or bool(unsup[m.cpu()].any())
             # the masked environments get the task queued and are reset: the reset consumes the slot
             queued = torch.where(m, ids.to(self.device), self.get_field('next_task')[:self.num_envs]).contiguous()
@@ -356,7 +362,7 @@ class BatchedSafeAdaptationGym:
             return
         self._tasks = task_list
         self._task_ids = ids.to(self.device)
-        self._any_unsupervised = bool((ids == _tasks.Unsupervised.task_id).any())
+        self._any_unsupervised = bool(self._is_unsupervised(ids).any())
         self._lib.check(self._lib.L.sag_set_tasks(self._h, self._p(self._task_ids), self._stream()))
         self._observation_space = None
         self._reset_all(new_task=True)
@@ -372,7 +378,8 @@ class BatchedSafeAdaptationGym:
         the slot.  The other environments reset as before.  ``set_task`` without a mask clears every slot.
 
         May be recorded in a CUDA graph with a device tensor (a host sequence raises ``RuntimeError`` under capture).
-        Host input is validated; a device tensor is checked where it is consumed: an id outside [-1, 14) is not applied
+        Host input is validated; a device tensor is checked where it is consumed: an id outside [-1, 14 + the number of
+        user-defined tasks) is not applied
         and raises ``ValueError`` at the next call that checks errors (``step``, ``check_errors``).  Queuing
         ``Unsupervised`` into a batch whose reward is not the pair raises ``ValueError``: ``step`` would have to record
         another reward buffer, so use ``set_task`` for that.  With a device tensor this is the caller's rule.  With
@@ -389,17 +396,18 @@ class BatchedSafeAdaptationGym:
                 raise RuntimeError('under CUDA graph capture set_next_task needs an int32 tensor of task ids on the env\'s '
                                    f'device ({self.device}); a host sequence would record a copy from pageable memory')
             if torch.is_tensor(task) or isinstance(task, np.ndarray):
-                by_id = {cls.task_id: cls for cls in _tasks.TASK_CLASSES}
+                by_id = self._classes_by_id()
                 raw = [int(i) for i in np.asarray(task.cpu() if torch.is_tensor(task) else task).reshape(-1)]
                 bad = [i for i in raw if i != -1 and i not in by_id]
                 if bad:
-                    raise ValueError(f'task id {bad[0]} out of range [-1, {_abi.NUM_TASKS})')
+                    raise ValueError(f'task id {bad[0]} out of range [-1, {len(by_id)})')
                 task = [None if i == -1 else by_id[i]() for i in raw]
             task_list = self._task_list(task, allow_none=True)
             if not self._any_unsupervised and any(isinstance(t, _tasks.Unsupervised) for t in task_list):
                 raise ValueError("Unsupervised's reward is a pair, which this batch's step does not record: "
                                  'switch to it with set_task')
-            ids = torch.tensor([-1 if t is None else t.task_id for t in task_list], dtype=torch.int32).to(self.device)
+            ids = torch.tensor([-1 if t is None else self.task_id_of(t) for t in task_list],
+                               dtype=torch.int32).to(self.device)
         self._lib.check(self._lib.L.sag_set_next_tasks(self._h, self._p(ids), self._stream()))
         self._next_armed = True
 
@@ -414,6 +422,7 @@ class BatchedSafeAdaptationGym:
         for kind in ('hazards', 'vases', 'pillars', 'gremlins'):
             w[kind + '_size'] = float(c[kind + '_size'])
             w[kind + '_keepout (effective)'] = max(float(c[kind + '_keepout']), float(c[kind + '_size']))
+        w['user-defined tasks'] = self._definitions()
         return w
 
     def copy_envs(self, index, source=None):
@@ -481,8 +490,8 @@ class BatchedSafeAdaptationGym:
                     raise ValueError(f'environment {k} copies environment {int(raw[k])}, which the same call overwrites')
             if not self._any_unsupervised:
                 used = torch.as_tensor(raw[raw >= 0], device=src.device)
-                unsup = _tasks.Unsupervised.task_id
-                if bool((src.task_ids[used] == unsup).any() | (src.get_field('next_task')[used] == unsup).any()):
+                if bool(self._is_unsupervised(src.task_ids[used]).any()
+                        | self._is_unsupervised(src.get_field('next_task')[used]).any()):
                     raise ValueError("a copied environment runs or has queued Unsupervised, whose reward is a pair that "
                                      'this batch\'s step does not record: set_task it here first')
             idx = torch.as_tensor(raw, dtype=torch.int32).to(self.device)
@@ -513,9 +522,78 @@ class BatchedSafeAdaptationGym:
 
     def _tasks_from_ids(self, ids: torch.Tensor):
         """The host-side task list from the ids the device holds (int32 [N] on the host)."""
-        by_id = {cls.task_id: cls for cls in _tasks.TASK_CLASSES}
+        by_id = self._classes_by_id()
         self._tasks = [by_id[int(i)]() for i in ids.tolist()]
         self._task_ids = ids.to(self.device)
+
+    # ---- user-defined tasks -------------------------------------------------------------------
+    def task_id_of(self, task) -> int:
+        """The task id of `task` on this batch, for ``set_next_task`` with a device tensor and for reading
+        ``task_ids`` / ``task_stats``.  A registry task, or a subclass whose ``obstacles`` and ``placement_extents``
+        equal its base's, has the registry id.  Another subclass of a registry task (a user-defined task) gets an id of
+        its own, 14, 15, ... in order of first use on this batch, one per class; the first use defines it, which
+        synchronises (``RuntimeError`` under CUDA graph capture).  A definition restored by ``load_state_dict`` is
+        taken by the first class with the same base, obstacles and extents, so a resumed batch keeps its ids.  Raises ``NotImplementedError`` for a subclass that
+        overrides anything besides ``obstacles`` and ``placement_extents`` and ``ValueError`` for a definition the
+        device cannot run (see ``_check_definition``)."""
+        if type(task) in _tasks.TASK_CLASSES:
+            return type(task).task_id
+        base, obstacles, extents = _tasks.definition(task)
+        for k, c in enumerate(self._custom):
+            if c['cls'] is type(task):
+                return _abi.NUM_TASKS + k
+        if _tasks.is_registry_equivalent(task):
+            return base.task_id
+        for k, c in enumerate(self._custom):
+            if not c['claimed'] and (c['base'], c['obstacles'], c['extents']) == (base, obstacles, extents):
+                c['cls'], c['claimed'] = type(task), True
+                return _abi.NUM_TASKS + k
+        return self._define(type(task), base, obstacles, extents)
+
+    def _check_definition(self, name, base, obstacles, extents):
+        if any(v < 0 for v in obstacles):
+            raise ValueError(f'{name}: obstacle counts must be >= 0, got {obstacles}')
+        ng = int(self.base_config.get('num_gremlins', 0))
+        if obstacles[2] != ng:
+            raise ValueError(f'{name}: obstacles[2] = {obstacles[2]} gremlins, but this batch runs num_gremlins = {ng} '
+                             '(gremlins are a batch setting: make the batch with config={"num_gremlins": k})')
+        # the base's task objects: its buttons, goal + box, or goal
+        n_task = (base.NUM_BUTTONS if issubclass(base, _tasks.PressButtons) else 2 if issubclass(base, _tasks.PushBox)
+                  else 1)
+        if sum(obstacles) + n_task > _abi.MAX_SLOTS:
+            raise ValueError(f'{name}: {sum(obstacles)} obstacles + {n_task} task objects exceed {_abi.MAX_SLOTS} slots')
+        if not (extents[0] < extents[2] and extents[1] < extents[3]):
+            raise ValueError(f'{name}: placement_extents {tuple(extents)} need x_min < x_max and y_min < y_max')
+        if len(self._custom) >= _abi.MAX_CUSTOM_TASKS:
+            raise ValueError(f'{name}: a batch holds at most {_abi.MAX_CUSTOM_TASKS} user-defined tasks')
+
+    def _define(self, cls, base, obstacles, extents, claimed=True) -> int:
+        """claimed=False: a definition restored by load_state_dict, under a stand-in class until task_id_of meets the
+        user's class"""
+        if _capturing():
+            raise RuntimeError(f'defining the task {cls.__name__} synchronises: call task_id_of before the CUDA graph capture')
+        self._check_definition(cls.__name__, base, obstacles, extents)
+        d = _abi.SagTaskDef(base.task_id, (C.c_int32 * 4)(*obstacles), (C.c_double * 4)(*extents))
+        tid = C.c_int32()
+        self._lib.check(self._lib.L.sag_define_task(self._h, C.byref(d), C.byref(tid)))
+        self._custom.append({'cls': cls, 'base': base, 'obstacles': list(obstacles), 'extents': list(extents),
+                             'claimed': claimed})
+        return tid.value
+
+    def _definitions(self):
+        return tuple((c['base'].task_id, tuple(c['obstacles']), tuple(c['extents'])) for c in self._custom)
+
+    def _classes_by_id(self):
+        by_id = {cls.task_id: cls for cls in _tasks.TASK_CLASSES}
+        for k, c in enumerate(self._custom):
+            by_id[_abi.NUM_TASKS + k] = c['cls']
+        return by_id
+
+    def _is_unsupervised(self, ids: torch.Tensor) -> torch.Tensor:
+        """Which of `ids` run Unsupervised's logic (the registry task or a user-defined task based on it)."""
+        unsup = [_tasks.Unsupervised.task_id] + [_abi.NUM_TASKS + k for k, c in enumerate(self._custom)
+                                                 if c['base'] is _tasks.Unsupervised]
+        return torch.isin(ids, torch.tensor(unsup, dtype=ids.dtype, device=ids.device))
 
     def render(self, mode='human'):
         raise NotImplementedError('rendering is outside the B200 hot path (reference: safe_adaptation_gym.py:109-111)')
@@ -618,7 +696,7 @@ class BatchedSafeAdaptationGym:
         in-step draw counters, the task ids, the queued next tasks and the cached clearance), and the host-side step
         budget.  The finished-episode statistics of `task_stats` are not part of it."""
         self._forbid_capture('state_dict')
-        return {'seed': self._seed, 'num_envs': self.num_envs, 'robot': self.robot_name,
+        return {'seed': self._seed, 'num_envs': self.num_envs, 'robot': self.robot_name, 'custom_tasks': self._definitions(),
                 'config': dict(self.base_config), 'env_id_base': self.env_id_base, 'max_episode_steps': self.max_episode_steps,
                 'fields': {name: self.get_field(name).cpu() for name in self._FIELDS}}
 
@@ -630,6 +708,17 @@ class BatchedSafeAdaptationGym:
                           ('max_episode_steps', self.max_episode_steps)):
             if key in sd and sd[key] != mine:
                 raise ValueError(f'state_dict was saved with a different {key}: {sd[key]!r} != {mine!r} (the continuation would not be bit-exact)')
+        saved = tuple(sd.get('custom_tasks', ()))
+        mine = self._definitions()
+        if mine[:len(saved)] != saved[:len(mine)]:
+            raise ValueError(f'state_dict defines the user-defined tasks {saved!r}, which conflict with this batch\'s '
+                             f'{mine!r}')
+        for base_id, obstacles, extents in saved[len(mine):]:
+            base = {c.task_id: c for c in _tasks.TASK_CLASSES}[base_id]
+            cls = type(f'{base.__name__}Custom{len(self._custom)}', (base,), {
+                'obstacles': property(lambda self, o=list(obstacles): list(o)),
+                'placement_extents': property(lambda self, x=tuple(extents): x)})
+            self._define(cls, base, list(obstacles), list(extents), claimed=False)
         self.seed(sd['seed'])
         for name, value in sd['fields'].items():
             self.set_field(name, value)
@@ -639,7 +728,7 @@ class BatchedSafeAdaptationGym:
             self._next_armed = True
         ids = sd['fields']['task_i32'][0, :self.num_envs].to(torch.int32)
         self._tasks_from_ids(ids)
-        self._any_unsupervised = bool((ids == _tasks.Unsupervised.task_id).any())
+        self._any_unsupervised = bool(self._is_unsupervised(ids).any())
         self._observation_space = None
         if self.base_config['random_bound']:
             self._bound.copy_(self.get_field('task_f64')[14, :self.num_envs])  # in place: a CUDA graph may export it
@@ -653,7 +742,12 @@ class BatchedSafeAdaptationGym:
                 {'cost': self._cost.to(torch.float32), 'bound': self._out(self._bound)})
 
     def task_stats(self, reset: bool = False) -> torch.Tensor:
-        """[14, 3] float64: per-task (sum of finished-episode returns, sum of costs, #episodes) on this device."""
-        out = torch.zeros((_abi.NUM_TASKS, 3), dtype=torch.float64, device=self.device)
+        """[14 + user-defined tasks, 3] float64: per-task id (sum of finished-episode returns, sum of costs, #episodes)
+        on this device.  Row 14 + k is the k-th user-defined task of this batch (``task_id_of``): ranks that reduce
+        these rows together (``stats.reduce_task_stats``) must define the same tasks in the same order."""
+        # as many rows as the library writes (a task may also have been defined through the C ABI on this handle)
+        L = self._lib.L
+        rows = L.sag_num_task_ids(self._h) if hasattr(L, 'sag_num_task_ids') else _abi.NUM_TASKS
+        out = torch.zeros((rows, 3), dtype=torch.float64, device=self.device)
         self._lib.check(self._lib.L.sag_task_stats(self._h, self._p(out), 1 if reset else 0, self._stream()))
         return out

@@ -2,7 +2,9 @@
 
 Each rank reduces its own environments into a [14, 3] float64 buffer on the device (sag_task_stats:
 sum of finished-episode returns, sum of costs, number of episodes per task id); the buffers are summed
-with one all-reduce (NCCL over NVLink on GPUs, gloo in the CPU tests)."""
+with one all-reduce (NCCL over NVLink on GPUs, gloo in the CPU tests).  A batch with user-defined tasks has a row for
+each of them after the 14 registry rows (``env.task_id_of``): the sum is right when every rank defines the same tasks
+in the same order."""
 import torch
 import torch.distributed as dist
 

@@ -168,3 +168,48 @@ DEVICE_UNSUPPORTED = frozenset()
 
 # every concrete task class (task_id = index in the registry's alphabetical order, benchmark/__init__.py:16-20)
 TASK_CLASSES = tuple(sorted((globals()[n] for n in __all__), key=lambda c: c.task_id))
+
+# what a user-defined task may override: the two properties the device path takes from it, and what Python puts in
+# every class body
+_OVERRIDABLE = frozenset(("obstacles", "placement_extents"))
+_CLASS_BOOKKEEPING = frozenset(("__module__", "__qualname__", "__doc__", "__dict__", "__weakref__", "__annotations__",
+                                "__firstlineno__", "__static_attributes__", "__orig_bases__", "__parameters__"))
+
+
+def registry_base(task: Task) -> type:
+    """The registry class a task instance derives from (the first of TASK_CLASSES in its MRO)."""
+    for cls in type(task).__mro__:
+        if cls in TASK_CLASSES:
+            return cls
+    raise TypeError(f'{type(task).__name__} does not derive from a registry task ({", ".join(__all__)})')
+
+
+def definition(task: Task):
+    """A task as the device path sees it: (base class, obstacles [4 ints], placement_extents [4 floats]).
+
+    Only ``obstacles`` and ``placement_extents`` may differ from the base; a subclass that overrides anything else
+    (class constants such as ``GOAL_SIZE``, methods such as a reward, other attributes) raises NotImplementedError
+    naming it."""
+    base = registry_base(task)
+    for cls in type(task).__mro__:
+        if cls is base:
+            break
+        for name in cls.__dict__:
+            if name not in _OVERRIDABLE and name not in _CLASS_BOOKKEEPING:
+                raise NotImplementedError(f'{type(task).__name__} overrides {name!r}: the device path runs '
+                                          f'{base.__name__} with its own obstacles and placement_extents only')
+    for name in vars(task):
+        raise NotImplementedError(f'{type(task).__name__} sets the instance attribute {name!r}: the device path runs '
+                                  f'{base.__name__} with its own obstacles and placement_extents only')
+    obstacles = [int(v) for v in task.obstacles]
+    extents = [float(v) for v in task.placement_extents]
+    if len(obstacles) != 4 or len(extents) != 4:
+        raise ValueError(f'{type(task).__name__}: obstacles and placement_extents need 4 entries each')
+    return base, obstacles, extents
+
+
+def is_registry_equivalent(task: Task) -> bool:
+    """Whether a task runs exactly as its registry base (the same obstacles and extents, nothing else overridden)."""
+    base, obstacles, extents = definition(task)
+    b = base()
+    return obstacles == [int(v) for v in b.obstacles] and extents == [float(v) for v in b.placement_extents]
