@@ -85,9 +85,10 @@ enum {
   SAG_F_ROBOT = 0,    /* double [6][stride]: x, y, yaw, vx, vy, w */
   SAG_F_OBJECTS = 1,  /* double [6][SAG_MAX_SLOTS][stride]: x, y, yaw, vx, vy, w per object slot */
   SAG_F_TASK_F64 = 2, /* double [15][stride]: last0,last1,cg_cur,cg_next,cg_ox,cg_oy,time,clearance,ep_return,ep_cost,ctrl0,ctrl1,
-                         ctrl_scale0,ctrl_scale1 (world.py:72-73),bound (world.py:75-78) */
+                         ctrl_scale0,ctrl_scale1 (world.py:72-73),bound (world.py:75-78); clearance is derived (rebuilt by
+                         sag_write_field) */
   SAG_F_TASK_I32 = 3, /* int32 [10][stride]: task, goal_button, btn_state, btn_timer, active_mask, cg_timer, n_step, step_ctr, episode,
-                         moving_mask (derived; rebuilt by sag_observe after an injection) */
+                         moving_mask (derived; rebuilt by sag_write_field) */
   SAG_F_FLAGS = 4,    /* uint8 [stride] */
   SAG_F_ROBOT_EXT = 5,/* double [6][stride]: car only -- wheel rates (2), castor ball-joint quaternion w,x,y,z (4) */
   SAG_F_GREMLINS = 6, /* double [2 + 3 * SAG_MAX_GREMLINS][stride]: mocap position of the last kinematics pass (x, y), then the weld
@@ -202,8 +203,7 @@ int sag_reset_host(void* handle, const uint8_t* mask_host, int only_flagged, int
  * cost uint8[n] (world.py:155 binary); done uint8[n]. */
 int sag_step(void* handle, const float* act, float* obs, double* reward, double* reward2, uint8_t* cost, uint8_t* done,
              void* stream);
-/* env.observation (safe_adaptation_gym.py:120-131) at the current state; also refreshes internal caches
- * after sag_write_field. */
+/* env.observation (safe_adaptation_gym.py:120-131) at the current state. */
 int sag_observe(void* handle, float* obs, void* stream);
 /* same as sag_step with HOST buffers: H2D, kernels, D2H, sync; returns when the outputs are in the host buffers.
  * Page-locked buffers (sag_host_alloc, cudaHostRegister, torch pin_memory) take the overlapped path: the bulk copy runs
@@ -251,7 +251,10 @@ int sag_export_outputs(void* handle, const float* obs, const double* reward, int
  * NULL). */
 int sag_rollout(void* handle, int k_steps, float* obs, double* reward, uint8_t* cost, uint8_t* done, void* stream);
 
-/* state injection / extraction; buffers are DEVICE pointers of sag_field_bytes(field) bytes */
+/* state injection / extraction; buffers are DEVICE pointers of sag_field_bytes(field) bytes.  sag_write_field of any
+ * field but SAG_F_NEXT_TASK then rebuilds, on the same stream, the derived rows (clearance, moving mask) from the state
+ * as written, so the next sag_step sees a consistent state without a sag_observe; on a state the library left, the
+ * rebuild writes the values that were there. */
 int sag_read_field(void* handle, int field, void* dst_dev, void* stream);
 int sag_write_field(void* handle, int field, const void* src_dev, void* stream);
 /* User-defined tasks (a subclass of a registry task that overrides Task.obstacles and Task.placement_extents,

@@ -8,8 +8,10 @@
  * operations in a fixed order, so the CUDA kernels and the CPU oracle get identical bits from them.
  *
  * The algorithms are the classic fdlibm ones (Cody-Waite reduction by pi/2 + minimax kernels; argument
- * range splitting for atan; 2^k(1+f) decomposition for log).  Accuracy (< 1 ulp, checked against glibc in
- * tests/test_detmath.py) is the same as libm's, so neither side gains or loses fidelity to the reference,
+ * range splitting for atan; 2^k(1+f) decomposition for log).  Accuracy against a long-double reference
+ * (tests/test_detmath.py): sin / cos <= 1.5 ulp for |x| <= 20 and <= 3 ulp up to |x| = 7e4 away from their
+ * zeros, where only an absolute bound holds (<= 5e-22 next to multiples of pi/2); atan2 <= 1.5 ulp; log
+ * <= 0.9 ulp.  That is libm's class of accuracy, so neither side gains or loses fidelity to the reference,
  * which itself just calls numpy / MuJoCo's libm.
  *
  * Valid C99 and CUDA C++.  Used by oracle/sag_oracle.c and safe_adaptation_gym_b200/csrc/sag_core.cuh.

@@ -1304,6 +1304,10 @@ int sag_write_field(void* handle, int field, const void* src, void* stream) {
   if (!H || !src || field < 0 || field >= SAG_NUM_FIELDS) return fail("sag_write_field: bad argument");
   DevGuard guard(H->device);
   CK(cudaMemcpyAsync(H->field_ptr[field], src, H->field_bytes[field], cudaMemcpyDeviceToDevice, (cudaStream_t)stream));
+  // The step's shortcuts read the clearance and moving mask cached in TASK_F64 / TASK_I32: rebuild them from the state
+  // just written (k_observe, into the staging buffer no caller sees).  On a state the kernels left, this rewrites the
+  // same values.  The queued next task is read by the resets only.
+  if (field != SAG_F_NEXT_TASK) CK(SAG_DISPATCH(H, observe(H, H->obs_d, (cudaStream_t)stream)));
   return 0;
 }
 

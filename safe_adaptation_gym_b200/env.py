@@ -682,6 +682,9 @@ class BatchedSafeAdaptationGym:
         return t
 
     def set_field(self, name: str, value: torch.Tensor):
+        """Overwrite an internal SoA state field, shape (*lead, stride) (see include/sag_b200.h SAG_F_*).  The derived
+        rows (the clearance in task_f64 row 7 and the moving mask in task_i32 row 9) are rebuilt from the state as
+        written, so `step` may follow directly."""
         self._forbid_capture('set_field')
         fid, dt, lead = self._FIELDS[name]
         t = torch.as_tensor(value).to(device=self.device, dtype=dt).contiguous()

@@ -99,6 +99,14 @@ void do_observe(Handle* H, float* obs) {
     write_tile(tile, obs, e0, D.n, RB::kObsDim);
   }
 }
+// sag_write_field: the clearance and moving mask that the step's dispatch reads, rebuilt as k_observe rebuilds them; the
+// observation is dropped
+template <class RB>
+void do_refresh(Handle* H) {
+  static float tile[kObsMax * kTileStride];
+  static Scratch scratch;
+  for (int e = 0; e < H->D.n; ++e) env_observe<RB>(1u, &scratch, H->D, e, tile, kTileStride);
+}
 template <class RB>
 void do_rollout(Handle* H, int k_steps, float* obs, double* reward, uint8_t* cost, uint8_t* done) {
   Dev& D = H->D;
@@ -213,7 +221,12 @@ int sag_rollout(void* h, int k_steps, float* obs, double* reward, uint8_t* cost,
   return 0;
 }
 int sag_read_field(void* h, int f, void* dst, void* s) { (void)s; Handle* H = (Handle*)h; memcpy(dst, H->slab + H->LY.off[f], H->LY.bytes[f]); return 0; }
-int sag_write_field(void* h, int f, const void* src, void* s) { (void)s; Handle* H = (Handle*)h; memcpy(H->slab + H->LY.off[f], src, H->LY.bytes[f]); return 0; }
+int sag_write_field(void* h, int f, const void* src, void* s) {
+  (void)s; Handle* H = (Handle*)h;
+  memcpy(H->slab + H->LY.off[f], src, H->LY.bytes[f]);
+  if (f != SAG_F_NEXT_TASK) HOSTEMU_DISPATCH(H, do_refresh, (H));
+  return 0;
+}
 int sag_task_stats(void* h, double* out, int reset, void* s) {
   (void)s; Handle* H = (Handle*)h; Dev& D = H->D;
   memcpy(out, H->stats_acc, SAG_NUM_TASKS * 3 * sizeof(double));
